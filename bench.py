@@ -4,6 +4,7 @@
     python bench.py --gpus N --steps K --warmup W                      # this repo's sm_100a path, BASELINE config 2 (Mean-Teacher 8+24)
     python bench.py --config {mt_acdc,mt_cfg1,mt_isic,cps,uamt} ...    # the other BASELINE.json configurations
     python bench.py --impl reference --gpus N --steps K --warmup W     # the reference algorithm on the host CPU cores
+    python bench.py ... --dump-outputs DIR                             # also write what the last timed step computed, DIR/<name>.npy
 
 A "step" is one training iteration of the configured trainer over one synthetic batch of 224x224 slices:
   mt_*  2017_03_NIPS_Mean-Teacher_ACDC.py:89-113      student forward+backward, teacher forward, fused SSL loss, SGD, EMA
@@ -134,6 +135,35 @@ class ClockSampler(threading.Thread):
                 "reasons": reasons, "samples": len(self.samples)}
 
 
+DUMP_MAX_BYTES = 64 << 20
+DUMP_SAMPLE = 2 << 20                # elements kept of a larger output: the same seeded positions in every run
+
+
+def dump_outputs(out_dir, step):
+    """Write what the step driver handed back after its last call, one DIR/<name>.npy per array (float32, float64 kept): the
+    tensors of step.last (loss scalars, logits) and the flat parameters and BatchNorm running statistics of every network it
+    updates.  An array of more than DUMP_SAMPLE elements is reduced to DUMP_SAMPLE positions drawn by a fixed seed, so two
+    builds run with the same arguments can be compared output for output."""
+    import numpy as np
+    import torch
+    arrays = {k: v for k, v in step.last.items() if torch.is_tensor(v)}
+    for attr in ("model", "ema_model", "m1", "m2"):
+        m = getattr(step, attr, None)
+        if m is not None:
+            arrays[attr + ".flat_params"], arrays[attr + ".bn_running"] = m.flat_params, m.bn_running
+    os.makedirs(out_dir, exist_ok=True)
+    total = 0
+    for name, t in arrays.items():
+        t = t.detach().flatten().cpu()
+        t = t if t.dtype == torch.float64 else t.float()
+        if t.numel() > DUMP_SAMPLE:
+            t = t[torch.randperm(t.numel(), generator=torch.Generator().manual_seed(0))[:DUMP_SAMPLE].sort().values]
+        total += t.numel() * t.element_size()
+        assert total <= DUMP_MAX_BYTES, "outputs exceed %d bytes" % DUMP_MAX_BYTES
+        np.save(os.path.join(out_dir, name + ".npy"), t.numpy())
+    return sorted(arrays)
+
+
 def synthetic_batch(c, seed):
     import torch
     g = torch.Generator().manual_seed(seed)
@@ -231,16 +261,14 @@ def run_reference(args):
         return
     c = CONFIGS[args.config]
     # every step is the full configured batch (BatchNorm / Dice see the real batch): ~1.7 s of host work per Mean-Teacher step
-    # on 16 cores; K and W are honoured up to 100 steps in total
-    steps = min(args.steps, 100)
-    warmup = min(args.warmup, 100 - steps) if steps < 100 else 0
+    # on 16 cores
+    steps, warmup = args.steps, args.warmup
     ips, sec, kind = cpu_reference_steps(c, steps, warmup)
     cores = os.cpu_count()
     line = {"impl": "reference", "metric": METRICS[c["kind"]], "value": ips, "unit": "images/s", "n_gpus": args.gpus, "steps": steps,
             "warmup": warmup, "ms_per_step": sec * 1e3, "higher_is_better": True, "scaling": "weak", "vs_baseline": None,
             "dtype": "f32", "data": "synthetic", "config": config_block(c, args.gpus),
-            "note": "the reference's CPU path (config cuda: False) on the host cores of this box, one process, all threads; "
-                    "requested --steps %d --warmup %d bounded to %d + %d" % (args.steps, args.warmup, steps, warmup),
+            "note": "the reference's CPU path (config cuda: False) on the host cores of this box, one process, all threads",
             "cpu_baseline": {"value": ips, "unit": "images/s", "cores": cores, "kind": kind,
                              "sample": "the configured %d+%d images per step, %d timed steps after %d warm-up (%.2f s per step), torch fp32"
                                        % (c["n_l"], c["n_u"], steps, warmup, sec)},
@@ -411,6 +439,7 @@ def run_gpu(args):
     launches0 = lib.hpfg_launch_count() + step.replayed_kernels
     ms = timed(resident_step, args.steps)
     launches = lib.hpfg_launch_count() + step.replayed_kernels - launches0      # host launches + kernel nodes replayed
+    dumped = dump_outputs(args.dump_outputs, step) if args.dump_outputs and rank == 0 else None
     for _ in range(2):
         e2e_step()
     torch.cuda.synchronize()
@@ -541,6 +570,8 @@ def run_gpu(args):
                 traffic_source="ncu --set full, profiles/r02b_loss_mt_one_ncu.txt (dram read+write of the launch, L2 flushed before the call: the dlogits mostly stay in L2)")
         if dp_check is not None:
             line["dp_check"] = dp_check
+        if dumped is not None:
+            line["outputs_dumped"] = {"dir": args.dump_outputs, "names": dumped}
         if cpu is not None:
             line["cpu_baseline"] = {"value": cpu[0], "unit": "images/s", "cores": os.cpu_count(), "kind": cpu[2],
                                     "sample": "the configured %d+%d images per step, %d timed steps after 1 warm-up (%.2f s per step), torch fp32, all host threads"
@@ -566,7 +597,12 @@ def main():
     ap.add_argument("--no-incumbent", action="store_true", help="skip the torch-eager incumbent leg")
     ap.add_argument("--quick", action="store_true", help="skip the per-layer table and the incumbent leg")
     ap.add_argument("--eager", action="store_true", help="launch every kernel from the host each step instead of replaying a CUDA graph")
+    ap.add_argument("--dump-outputs", metavar="DIR", help="after the timed steps, write what the last one computed as DIR/<name>.npy")
     args = ap.parse_args()
+    if args.steps < 1 or args.warmup < 0:
+        ap.error("--steps must be at least 1 and --warmup at least 0")
+    if args.dump_outputs and args.impl == "reference":
+        ap.error("--dump-outputs writes the outputs of this repository's GPU path (--impl ours)")
     if args.impl == "reference":
         run_reference(args)
     else:

@@ -7,8 +7,9 @@ there only as the checker / the timed CPU baseline, never as the product path.
 The oracle is a plain PyTorch fp32 *restatement* of the reference algorithm (the reference itself is
 pure PyTorch; every function cites the reference file:line it follows).  It is pinned two ways:
 
-* ``tests/test_oracle_vs_reference.py`` runs it against the real reference modules loaded by file path
-  from ``/root/reference`` (only where that tree exists, i.e. in the build container);
+* ``tests/test_oracle_vs_reference.py`` runs it against values the real reference modules printed
+  (``tests/golden/reference_mt_acdc.json``), and against the modules themselves, loaded by file path from
+  a checkout named by ``$HPFG_REF``, where one is given;
 * ``tests/golden/*.pt`` hold input/output vectors produced by the real reference
   (``tests/golden/make_golden.py``), which travel to the GPU box.
 """

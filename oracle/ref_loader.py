@@ -1,6 +1,6 @@
 """Load the REAL reference hot-path modules by file path (never `import model` / `import utils`: those
-pull timm/easydict/medpy which are not installed).  Only available where the reference tree exists
-(the build container); the GPU box relies on tests/golden/ instead."""
+pull timm/easydict/medpy which are not installed).  Only available where a checkout of the reference is named by
+$HPFG_REF; everywhere else the tests rely on tests/golden/ instead."""
 import importlib.util
 import os
 import sys
@@ -8,10 +8,8 @@ import types
 
 
 def find_reference():
-    for p in (os.environ.get("HPFG_REF"), "/root/reference"):
-        if p and os.path.isfile(os.path.join(p, "model", "unet.py")):
-            return p
-    return None
+    p = os.environ.get("HPFG_REF")
+    return p if p and os.path.isfile(os.path.join(p, "model", "unet.py")) else None
 
 
 def _load(name, path):
@@ -26,7 +24,7 @@ def load_reference():
     get_current_consistency_weight, sigmoid_rampup, Medical_LR -- the reference's own objects."""
     root = find_reference()
     if root is None:
-        raise FileNotFoundError("reference tree not found (set HPFG_REF or run in the build container)")
+        raise FileNotFoundError("reference checkout not found (set HPFG_REF)")
     if "easydict" not in sys.modules:                       # utils/utils.py:3 imports it at module top
         stub = types.ModuleType("easydict")
 

@@ -206,5 +206,11 @@ def test_unet_plus_and_dense_loss():
     assert abs(loss.item() - g["loss"]) / g["loss"] < 1e-5
     grads = torch.autograd.grad(loss, [leaves[n] for n in names])
     for n, gr in zip(names, grads):
+        if n.endswith("conv_conv.0.bias") or n.endswith("conv_conv.4.bias"):
+            # conv biases ahead of train-mode BatchNorm have an analytically zero gradient: both sides hold rounding noise,
+            # which changes with the number of CPU threads, so it is bounded on an absolute scale
+            assert g["grads"][n]["abs_sum"] < 1e-5 * g["grads"][n]["numel"], n
+            assert gr.abs().max().item() < 1e-5, n
+            continue
         check_summary(gr, g["grads"][n], rtol=2e-4, atol=1e-6, what=n)
     check_summary(oracle.unet_forward(view, x, False), g["val_logits"], rtol=1e-5, atol=1e-6, what="val logits")
