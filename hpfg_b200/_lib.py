@@ -54,10 +54,8 @@ SIGNATURES = {
     "hpfg_ssl_loss_workspace_bytes": (c_i64, [c_int] * 6),
     "hpfg_ssl_loss": (c_int, [c_int, c_vp, c_vp, c_vp, c_int, c_vp, c_int, c_int, c_int, c_int, c_int, c_f, c_f,
                               ctypes.POINTER(c_f), c_f, c_f, c_vp, c_vp, c_vp, c_vp, c_vp, c_vp, c_vp]),
-    "hpfg_ssl_loss_dv": (c_int, [c_int, c_vp, c_vp, c_vp, c_int, c_vp, c_int, c_int, c_int, c_int, c_int, c_vp, c_f,
+    "hpfg_ssl_loss_dv": (c_int, [c_int, c_vp, c_vp, c_vp, c_int, c_vp, c_int, c_int, c_int, c_int, c_int, c_vp, c_f, c_vp,
                                  ctypes.POINTER(c_f), c_f, c_f, c_vp, c_vp, c_vp, c_vp, c_vp, c_vp, c_vp]),
-    "hpfg_ssl_loss_dv2": (c_int, [c_int, c_vp, c_vp, c_vp, c_int, c_vp, c_int, c_int, c_int, c_int, c_int, c_vp, c_vp,
-                                  ctypes.POINTER(c_f), c_f, c_f, c_vp, c_vp, c_vp, c_vp, c_vp, c_vp, c_vp]),
     "hpfg_ict_loss": (c_int, [c_vp, c_vp, c_vp, c_vp, c_int, c_int, c_int, c_int, c_int, c_f, c_vp, ctypes.POINTER(c_f),
                               c_f, c_f, c_vp, c_vp, c_vp, c_vp]),
     "hpfg_ict_mix": (c_int, [c_vp, c_vp, c_vp, c_int, c_i64, c_vp, c_vp]),

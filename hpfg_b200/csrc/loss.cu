@@ -932,26 +932,13 @@ extern "C" int hpfg_ssl_loss(int mode, const float *student, const float *other,
 extern "C" int hpfg_ssl_loss_dv(int mode, const float *student, const float *other, const float *mc_logits,
                                 int mc_passes, const int64_t *labels, int n_l, int n_u, int num_classes, int height,
                                 int width, const float *cons_weight_dev, float uamt_threshold,
-                                const float *class_weights_host, float ce_coef, float dice_coef, float *dstudent,
-                                float *dother, float *scalars_out, int64_t *pseudo1, int64_t *pseudo2, void *workspace,
-                                void *stream) {
+                                const float *uamt_threshold_dev, const float *class_weights_host, float ce_coef,
+                                float dice_coef, float *dstudent, float *dother, float *scalars_out, int64_t *pseudo1,
+                                int64_t *pseudo2, void *workspace, void *stream) {
     HPFG_REQUIRE(cons_weight_dev, "hpfg_ssl_loss_dv: cons_weight_dev is null");
     HPFG_REQUIRE(mode <= HPFG_LOSS_UAMT, "hpfg_ssl_loss_dv: use hpfg_ict_loss / hpfg_s4cv_loss for the ICT / S4CV modes");
     return ssl_loss_impl(mode, student, other, mc_logits, mc_passes, labels, n_l, n_u, num_classes, height, width, 0.f, cons_weight_dev,
                          uamt_threshold, class_weights_host, ce_coef, dice_coef, dstudent, dother, scalars_out, pseudo1, pseudo2,
-                         workspace, stream);
-}
-
-extern "C" int hpfg_ssl_loss_dv2(int mode, const float *student, const float *other, const float *mc_logits,
-                                 int mc_passes, const int64_t *labels, int n_l, int n_u, int num_classes, int height,
-                                 int width, const float *cons_weight_dev, const float *uamt_threshold_dev,
-                                 const float *class_weights_host, float ce_coef, float dice_coef, float *dstudent,
-                                 float *dother, float *scalars_out, int64_t *pseudo1, int64_t *pseudo2, void *workspace,
-                                 void *stream) {
-    HPFG_REQUIRE(cons_weight_dev && uamt_threshold_dev, "hpfg_ssl_loss_dv2: null device scalar");
-    HPFG_REQUIRE(mode <= HPFG_LOSS_UAMT, "hpfg_ssl_loss_dv2: use hpfg_ict_loss / hpfg_s4cv_loss for the ICT / S4CV modes");
-    return ssl_loss_impl(mode, student, other, mc_logits, mc_passes, labels, n_l, n_u, num_classes, height, width, 0.f, cons_weight_dev,
-                         0.f, class_weights_host, ce_coef, dice_coef, dstudent, dother, scalars_out, pseudo1, pseudo2,
                          workspace, stream, nullptr, 0.f, nullptr, uamt_threshold_dev);
 }
 

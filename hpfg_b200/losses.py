@@ -46,19 +46,12 @@ def ssl_loss_raw(mode, student, other, labels, n_l, *, cons_weight=0.0, mc_logit
     if want_pseudo and mode == L.LOSS_CPS:
         p1 = torch.empty((n_u, h, w), device=dev, dtype=torch.int64)
         p2 = torch.empty((n_u, h, w), device=dev, dtype=torch.int64)
-    if cons_weight_dev is not None and uamt_threshold_dev is not None:      # ... and so is the UAMT threshold
-        L.check(L.lib().hpfg_ssl_loss_dv2(mode, L.ptr(student), L.ptr(other), L.ptr(mc_logits), mc_passes, L.ptr(labels),
-                                          n_l, n_u, c, h, w, L.ptr(cons_weight_dev), L.ptr(uamt_threshold_dev),
-                                          _weights_arg(class_weights, c), float(ce_coef), float(dice_coef),
-                                          L.ptr(dstudent), L.ptr(dother), L.ptr(scalars), L.ptr(p1), L.ptr(p2), L.ptr(ws),
-                                          L.stream_ptr(dev)), "hpfg_ssl_loss_dv2")
-        return dict(scalars=scalars, dstudent=dstudent, dother=dother, pseudo1=p1, pseudo2=p2)
-    if cons_weight_dev is not None:      # CUDA-graph replays: the consistency weight is a device scalar
+    if cons_weight_dev is not None:      # CUDA-graph replays: the consistency weight (and UAMT threshold, if given) on the device
         L.check(L.lib().hpfg_ssl_loss_dv(mode, L.ptr(student), L.ptr(other), L.ptr(mc_logits), mc_passes, L.ptr(labels),
                                          n_l, n_u, c, h, w, L.ptr(cons_weight_dev), float(uamt_threshold),
-                                         _weights_arg(class_weights, c), float(ce_coef), float(dice_coef),
-                                         L.ptr(dstudent), L.ptr(dother), L.ptr(scalars), L.ptr(p1), L.ptr(p2), L.ptr(ws),
-                                         L.stream_ptr(dev)), "hpfg_ssl_loss_dv")
+                                         L.ptr(uamt_threshold_dev), _weights_arg(class_weights, c), float(ce_coef),
+                                         float(dice_coef), L.ptr(dstudent), L.ptr(dother), L.ptr(scalars), L.ptr(p1),
+                                         L.ptr(p2), L.ptr(ws), L.stream_ptr(dev)), "hpfg_ssl_loss_dv")
         return dict(scalars=scalars, dstudent=dstudent, dother=dother, pseudo1=p1, pseudo2=p2)
     L.check(L.lib().hpfg_ssl_loss(mode, L.ptr(student), L.ptr(other), L.ptr(mc_logits), mc_passes, L.ptr(labels), n_l,
                                   n_u, c, h, w, float(cons_weight), float(uamt_threshold),

@@ -13,6 +13,7 @@ all-reduce of the gradient buckets on a side stream, overlapped with the rest of
 SGD-momentum(+EMA) pass over the flat parameter buffers.  Nothing synchronises the host; the returned loss is
 a device scalar.  Host-side schedules (Medical_LR, consistency ramp-up, EMA alpha) are python floats exactly as
 in the reference (utils/scheduler/medical_lr.py:13-17, utils/utils.py:67-86)."""
+import contextlib
 import math
 
 import torch
@@ -41,7 +42,6 @@ def allreduce_flat_buckets(flat_grad, buckets, group=None, before_bucket=None, s
     """Sum-all-reduce ``flat_grad`` bucket by bucket (async), returning the work handles.  ``before_bucket(i)`` is
     called before bucket i is enqueued (the CUDA path makes the comm stream wait for that bucket's event there).
     Works for CPU tensors + gloo (host-logic tests) and CUDA tensors + NCCL alike."""
-    import contextlib
     import torch.distributed as dist
     works = []
     for i, (off, cnt) in enumerate(buckets):
@@ -77,7 +77,14 @@ def shard_batch(x_l, x_u, y, rank, world):
     return x_l[rank * a:(rank + 1) * a], x_u[rank * b:(rank + 1) * b], y[rank * a:(rank + 1) * a]
 
 
+def _input_noise(shape, like):
+    """Clamped Gaussian perturbation of a teacher's input (2019_07...:130,141; 2022_08...:111), ONE draw of ``shape``."""
+    return torch.clamp(torch.randn(shape, device=like.device, dtype=like.dtype) * 0.1, -0.2, 0.2)
+
+
 class _StepBase:
+    serialize = False             # profiling: every network on the calling stream, so per-category kernel times do not overlap
+
     def __init__(self, *, lr=0.01, momentum=0.9, weight_decay=1e-4, total_itrs=30000, consistency=0.1,
                  consistency_rampup=200.0, process_group=None, exact_global=False):
         self.base_lr, self.momentum, self.weight_decay = lr, momentum, weight_decay
@@ -98,6 +105,23 @@ class _StepBase:
         if self.exact_global:
             L.install_allreduce_hook(self.pg)
 
+    def _setup(self, trained, networks, train=None, grads=True):
+        """Construction shared by the drivers.  trained: the networks this driver optimises, in checkpoint order, each given a
+        flat momentum buffer and (unless autograd produces its gradients, grads=False) a flat gradient buffer; networks: every
+        network of the step, in the order of the checkpointed Philox offsets; train: the networks put in train() mode (default:
+        the trained ones).  Returns [(gradient buffer, momentum buffer)] in the order of ``trained``."""
+        self.in_channels, self.num_classes = trained[0].in_channels, trained[0].num_classes
+        for m in trained if train is None else train:
+            m.train()
+        for m in networks:
+            m.ensure_flat()
+        self._trained = [(m, torch.zeros_like(m.flat_params) if grads else None, torch.zeros_like(m.flat_params))
+                         for m in trained]
+        self._networks = list(networks)
+        self._check_buffers()
+        self._broadcast_from_rank0()
+        return [(g, b) for _, g, b in self._trained]
+
     # ------------------------------------------------------------------ CUDA-graph replay of the whole step
     _graph_enabled = False
     _graph_dp = False
@@ -109,49 +133,42 @@ class _StepBase:
         fused loss, backward with its side-stream weight gradients, fused SGD(+EMA)).  The scalars that change per
         iteration -- learning rate, EMA alpha, consistency weight, UAMT threshold, dropout Philox offsets -- live in a
         small device block that is refreshed before every replay (the `_dv` entry points read them at run time).
-        data_parallel=True also captures the bucketed NCCL all-reduces of a multi-process run (Mean-Teacher driver only,
-        measured on 2/4/8 B200; the other drivers stay eager when data parallel); by default a data-parallel step stays eager."""
+        data_parallel=True also captures the bucketed NCCL all-reduces of a multi-process run; by default a data-parallel
+        step stays eager, and so does the exact-global mode.  S4CVStep and HPFGStep always launch eagerly."""
         self._graph_enabled = bool(enabled)
         self._graph_dp = bool(data_parallel)      # also capture the NCCL bucket all-reduces (torch >= 2.x captures NCCL work)
         if not enabled:
             self._ggraph = None
             self._gsig = None
 
-    _graph_dp_capable = True      # the bucketed NCCL all-reduces are captured with the step (a refused capture falls back to eager launches)
-
     def _use_graph(self):
-        dp_ok = self.world == 1 or (self._graph_dp and self._graph_dp_capable)
-        return self._graph_enabled and self.cur_itrs >= 2 and dp_ok and not getattr(self, "exact_global", False)
+        dp_ok = self.world == 1 or self._graph_dp
+        return self._graph_enabled and self.cur_itrs >= 2 and dp_ok and not self.exact_global
 
-    class _GlobalSums:
-        """Loss sums over the batch of all ranks while a fused loss call is enqueued (hpfg_ssl_loss_set_global_sums)."""
-
-        def __init__(self, on):
-            self.on = on
-
-        def __enter__(self):
-            if self.on:
-                L.check(L.lib().hpfg_ssl_loss_set_global_sums(1), "hpfg_ssl_loss_set_global_sums")
-
-        def __exit__(self, *exc):
-            if self.on:
-                L.check(L.lib().hpfg_ssl_loss_set_global_sums(0), "hpfg_ssl_loss_set_global_sums")
-
+    @contextlib.contextmanager
     def _global_sums(self):
-        return self._GlobalSums(getattr(self, "exact_global", False))
+        """Loss sums over the batch of all ranks while a fused loss call is enqueued (exact-global mode; no-op otherwise)."""
+        if not self.exact_global:
+            yield
+            return
+        L.check(L.lib().hpfg_ssl_loss_set_global_sums(1), "hpfg_ssl_loss_set_global_sums")
+        try:
+            yield
+        finally:
+            L.check(L.lib().hpfg_ssl_loss_set_global_sums(0), "hpfg_ssl_loss_set_global_sums")
 
     def _global_consistency_value(self, scalars, w):
         """Mean-Teacher / ICT in exact-global mode: the kernel's consistency value is this rank's share of the global mean."""
-        if getattr(self, "exact_global", False):
+        if self.exact_global:
             torch.distributed.all_reduce(scalars[2:3], group=self.pg)
             scalars[0:1].copy_(scalars[1:2] + w * scalars[2:3])
 
     def _graph_replay(self, inputs, dyn_f, fwd_models, body):
         """Generic capture-once / replay driver (all step drivers).
         inputs: tensors copied into static buffers before each replay; dyn_f: python floats for the device block
-        (fp32); fwd_models: one entry per network forward in the eager call order -> one Philox-offset slot each (the
-        offsets advance exactly as the eager path advances them); body(static_inputs, dyn_f_dev, dyn_o_dev) enqueues the
-        step with the `_dv` entry points and returns its output dict (static tensors).
+        (fp32); fwd_models: the network of each forward in the order the body enqueues them -> one Philox-offset slot each
+        (the offsets advance exactly as eager launches advance them); body(static_inputs, dv) enqueues the step with
+        dv = (device block, Philox-offset slots) and returns its output dict (static tensors).
 
         The per-iteration scalars travel through a RING of pinned host slots: an async H2D copy reads pinned memory when
         the stream reaches it, not at enqueue time, so a slot is only rewritten after the event recorded behind its copy
@@ -167,7 +184,7 @@ class _StepBase:
         for m in models:
             m.ensure_flat(quick=True)
         ptrs = tuple((m.flat_params.data_ptr(), m.bn_running.data_ptr(), m.bn_counters.data_ptr(), id(m._plans)) for m in models)
-        ptrs += tuple(t.data_ptr() for t in self._state_tensors())
+        ptrs += tuple(t.data_ptr() for _, g, b in self._trained for t in (g, b) if t is not None)
         # (the dropout seed is a by-value launch argument: a re-seeded generator needs a new capture)
         ptrs += (torch.cuda.default_generators[dev.index if dev.index is not None else torch.cuda.current_device()].initial_seed(),)
         sig = tuple((tuple(t.shape), t.dtype) for t in inputs) + (len(dyn_f), len(fwd_models), ptrs)
@@ -203,13 +220,13 @@ class _StepBase:
             n0 = L.lib().hpfg_launch_count()
             try:
                 with torch.cuda.graph(g):
-                    self._gout = body(self._gin, self._gf, self._go)
+                    self._gout = self._body_on_device_block(body, fwd_models)
             except Exception as exc:        # capture not possible here (e.g. a collective that refuses capture): stay eager
                 import warnings
                 warnings.warn("hpfg_b200: CUDA-graph capture of the step failed (%s); falling back to eager launches" % exc)
                 self._graph_enabled, self._ggraph = False, None
                 torch.cuda.synchronize()
-                return body(self._gin, self._gf, self._go)
+                return self._body_on_device_block(body, fwd_models)
             self._ggraph = g
             self.kernels_per_replay = int(L.lib().hpfg_launch_count() - n0)   # kernel nodes of the captured step
         self._ggraph.replay()
@@ -218,23 +235,21 @@ class _StepBase:
 
     _RING = 8
 
-    def _state_tensors(self):
-        """Optimiser-side device buffers of this driver (gradient + momentum buffers), in a fixed order."""
-        return [getattr(self, n) for n in ("grads", "mom", "g1", "b1", "g2", "b2") if hasattr(self, n)]
-
-    def _models(self):
-        return [getattr(self, n) for n in ("model", "ema_model", "m1", "m2") if hasattr(self, n)]
+    def _body_on_device_block(self, body, fwd_models):
+        """Enqueue body with every per-iteration scalar read from the device block; _forward takes the Philox slots of
+        ``fwd_models`` in call order."""
+        self._slots, self._slot = fwd_models, 0
+        out = body(self._gin, (self._gf, self._go))
+        assert self._slot == len(fwd_models), "the step ran %d forwards for %d Philox slots" % (self._slot, len(fwd_models))
+        return out
 
     # ------------------------------------------------------------------ checkpoint / resume (2017_03...:126-133)
     def state_dict(self):
         """{cur_itrs, philox offsets, optimizer}: `optimizer` holds torch.optim.SGD-style per-parameter momentum buffers
         (state[i]['momentum_buffer'] in model.parameters() order) so that a reference checkpoint's optimizer state and
         this driver's flat momentum buffer interchange."""
-        out = {"cur_itrs": self.cur_itrs, "philox": [m._philox_offset for m in self._models()], "optimizers": []}
-        pairs = [(getattr(self, a, None), getattr(self, b, None)) for a, b in (("model", "mom"), ("m1", "b1"), ("m2", "b2"))]
-        for model, buf in pairs:
-            if model is None or buf is None:
-                continue
+        out = {"cur_itrs": self.cur_itrs, "philox": [m._philox_offset for m in self._networks], "optimizers": []}
+        for model, _, buf in self._trained:
             state = {i: {"momentum_buffer": buf[o:o + n].view(shape).clone()} for i, (o, n, shape) in enumerate(model._layout)}
             out["optimizers"].append({"state": state if self.cur_itrs > 0 else {},
                                       "param_groups": [{"lr": medical_lr(self.cur_itrs + 1, self.base_lr, self.total_itrs),
@@ -244,11 +259,9 @@ class _StepBase:
 
     def load_state_dict(self, sd):
         self.cur_itrs = int(sd["cur_itrs"])
-        for m, off in zip(self._models(), sd.get("philox", [])):
+        for m, off in zip(self._networks, sd.get("philox", [])):
             m._philox_offset = int(off)
-        pairs = [(getattr(self, a, None), getattr(self, b, None)) for a, b in (("model", "mom"), ("m1", "b1"), ("m2", "b2"))]
-        pairs = [(m, b) for m, b in pairs if m is not None and b is not None]
-        for (model, buf), opt in zip(pairs, sd.get("optimizers", [])):
+        for (model, _, buf), opt in zip(self._trained, sd.get("optimizers", [])):
             buf.zero_()
             for i, (o, n, shape) in enumerate(model._layout):
                 st = opt["state"].get(i)
@@ -257,16 +270,13 @@ class _StepBase:
 
     def _check_buffers(self):
         """The flat gradient / momentum buffers must match the (possibly re-flattened or moved) parameter buffer."""
-        for model, names in ((getattr(self, "model", None), ("grads", "mom")), (getattr(self, "m1", None), ("g1", "b1")),
-                             (getattr(self, "m2", None), ("g2", "b2"))):
-            if model is None:
-                continue
+        for model, *bufs in self._trained:
             flat = model.flat_params
-            for n in names:
-                buf = getattr(self, n)
-                if buf.device != flat.device or buf.numel() != flat.numel():
-                    raise L.HpfgError("step driver buffer '%s' (%s, %d) no longer matches the model's flat parameters (%s, %d): "
-                                      "build the step driver after moving the model" % (n, buf.device, buf.numel(), flat.device, flat.numel()))
+            for what, buf in zip(("gradient", "momentum"), bufs):
+                if buf is not None and (buf.device != flat.device or buf.numel() != flat.numel()):
+                    raise L.HpfgError("step driver %s buffer (%s, %d) no longer matches the model's flat parameters (%s, %d): "
+                                      "build the step driver after moving the model"
+                                      % (what, buf.device, buf.numel(), flat.device, flat.numel()))
             if flat.is_cuda and flat.device.index != torch.cuda.current_device():
                 raise L.HpfgError("the model lives on %s but the current CUDA device is %d: call torch.cuda.set_device first "
                                   "(the library launches on the current device)" % (flat.device, torch.cuda.current_device()))
@@ -276,7 +286,7 @@ class _StepBase:
         if self.world <= 1:
             return
         import torch.distributed as dist
-        for m in self._models():
+        for m in self._networks:
             m.ensure_flat()
             for t in (m.flat_params, m.bn_running, m.bn_counters):
                 dist.broadcast(t, src=dist.get_global_rank(self.pg, 0) if self.pg is not None else 0, group=self.pg)
@@ -288,7 +298,7 @@ class _StepBase:
     share_forward = True
 
     def _set_forward_share(self, plan, shared):
-        if getattr(self, "exact_global", False) and not getattr(plan, "sync_bn", False):
+        if self.exact_global and not getattr(plan, "sync_bn", False):
             L.check(L.lib().hpfg_unet_plan_set_sync_bn(plan.handle, 1), "hpfg_unet_plan_set_sync_bn")
             plan.sync_bn = True
         want = self.SHARED_FORWARD_CTAS if shared else 0
@@ -296,46 +306,49 @@ class _StepBase:
             L.check(L.lib().hpfg_unet_plan_set_forward_ctas(plan.handle, want), "hpfg_unet_plan_set_forward_ctas")
             plan.fwd_ctas = want
 
-    def _forward_dv(self, model, x, save, out, offset_dev):
-        plan = model._acquire_plan(x, need_grad=save)
-        self._set_forward_share(plan, self.share_forward)      # (graph replays always run the forwards on two streams)
-        return plan, model._run_forward(plan, x, save=save, out=out, offset_dev=offset_dev)
-
-    def _sgd_dv(self, model, grads, buf, dyn_f, ema_model=None):
-        """SGD(+EMA) with {lr, ema_alpha, 1-ema_alpha} read from the device block (first_step = 0: replays start at
-        iteration 2)."""
-        n = model.flat_params.numel()
-        st = L.stream_ptr(grads.device)
-        if ema_model is None:
-            L.check(L.lib().hpfg_sgd_momentum_dv(L.ptr(model.flat_params), L.ptr(grads), L.ptr(buf), n, self.momentum,
-                                                 self.weight_decay, 1.0 / self.world, 0, L.ptr(dyn_f), st),
-                    "hpfg_sgd_momentum_dv")
-        else:
-            L.check(L.lib().hpfg_sgd_momentum_ema_dv(L.ptr(model.flat_params), L.ptr(grads), L.ptr(buf),
-                                                     L.ptr(ema_model.flat_params), n, self.momentum, self.weight_decay,
-                                                     1.0 / self.world, 0, L.ptr(dyn_f), st), "hpfg_sgd_momentum_ema_dv")
+    def _lr(self):
+        return medical_lr(self.cur_itrs, self.base_lr, self.total_itrs)
 
     def _dyn_scalars(self, ema_decay=None):
-        """[lr, ema_alpha, 1 - ema_alpha (fp32 subtraction, as the by-value entry point), consistency weight]."""
-        lr = medical_lr(self.cur_itrs, self.base_lr, self.total_itrs)
+        """The device block: [lr, ema_alpha, 1 - ema_alpha (fp32 subtraction, as the by-value entry point), consistency
+        weight]; UAMT appends its threshold."""
         alpha = min(1 - 1 / (self.cur_itrs + 1), ema_decay) if ema_decay is not None else 0.0
-        w = self._consistency_weight()
-        return [lr, alpha, float(1.0 - torch.tensor(alpha, dtype=torch.float32)), w]
+        return [self._lr(), alpha, float(1.0 - torch.tensor(alpha, dtype=torch.float32)), self._consistency_weight()]
+
+    @staticmethod
+    def _dv_scalar(dv, i):
+        """Entry i of the device block during capture, None for eager launches."""
+        return None if dv is None else dv[0][i:i + 1]
 
     def _side_stream(self, device):
         if getattr(self, "_side", None) is None:
             self._side = torch.cuda.Stream(device=device)
         return self._side
 
+    def _fork(self, device):
+        """(main, side): the calling stream and the stream the other network(s) run on (the same one when ``serialize`` is
+        set), the side stream ordered after everything enqueued so far."""
+        main = torch.cuda.current_stream(device)
+        side = main if self.serialize else self._side_stream(device)
+        side.wait_stream(main)
+        return main, side
+
     def _consistency_weight(self):
         return self.consistency * sigmoid_rampup(self.cur_itrs // 150, self.consistency_rampup)
 
-    def _forward(self, model, x, save, out=None):
-        model.ensure_flat(quick=True)
+    def _forward(self, model, x, save, out, dv):
+        """One network forward into ``out`` (activations kept in the plan when ``save``).  Eager launches (dv None) use the
+        model's Philox offset; during capture the offset is read from the next slot of the device block."""
+        if dv is None:
+            model.ensure_flat(quick=True)          # (captures: _graph_replay has checked every network)
+            offset_dev = None
+        else:
+            assert self._slots[self._slot] is model, "forward %d does not run the network of its Philox slot" % self._slot
+            offset_dev = dv[1][self._slot:self._slot + 1]
+            self._slot += 1
         plan = model._acquire_plan(x, need_grad=save)
-        self._set_forward_share(plan, self.share_forward and not getattr(self, "serialize", False))
-        logits = model._run_forward(plan, x, save=save, out=out)
-        return plan, logits
+        self._set_forward_share(plan, self.share_forward and not self.serialize)
+        return plan, model._run_forward(plan, x, save=save, out=out, offset_dev=offset_dev)
 
     def _persistent(self, name, shape, device):
         """Step-persistent fp32 buffer (no per-step allocation: tensors that cross streams would otherwise need
@@ -367,94 +380,63 @@ class _StepBase:
         for w in works:
             w.wait()            # stream-level wait on the compute stream, not a host sync
 
-    def _sgd(self, model, grads, buf, ema_model=None, ema_alpha=0.0):
-        lr = medical_lr(self.cur_itrs, self.base_lr, self.total_itrs)
-        n = model.flat_params.numel()
-        st = L.stream_ptr(grads.device)
+    def _sgd(self, model, grads, buf, dv, ema_model=None):
+        """Fused SGD-momentum over the flat buffers, with the EMA of ``model`` into ``ema_model`` in the same pass if given.
+        Eager launches take this iteration's learning rate and EMA alpha by value; captures read {lr, alpha, 1 - alpha}
+        from the device block."""
+        lib, n, st = L.lib(), model.flat_params.numel(), L.stream_ptr(grads.device)
+        p, g, m = L.ptr(model.flat_params), L.ptr(grads), L.ptr(buf)
         first = int(self.cur_itrs == 1)
-        if ema_model is None:
-            L.check(L.lib().hpfg_sgd_momentum(L.ptr(model.flat_params), L.ptr(grads), L.ptr(buf), n, lr, self.momentum,
-                                              self.weight_decay, self._grad_scale, first, st), "hpfg_sgd_momentum")
+        if dv is not None:
+            if ema_model is None:
+                L.check(lib.hpfg_sgd_momentum_dv(p, g, m, n, self.momentum, self.weight_decay, self._grad_scale, first,
+                                                 L.ptr(dv[0]), st), "hpfg_sgd_momentum_dv")
+            else:
+                L.check(lib.hpfg_sgd_momentum_ema_dv(p, g, m, L.ptr(ema_model.flat_params), n, self.momentum, self.weight_decay,
+                                                     self._grad_scale, first, L.ptr(dv[0]), st), "hpfg_sgd_momentum_ema_dv")
+        elif ema_model is None:
+            L.check(lib.hpfg_sgd_momentum(p, g, m, n, self._lr(), self.momentum, self.weight_decay, self._grad_scale, first, st),
+                    "hpfg_sgd_momentum")
         else:
-            L.check(L.lib().hpfg_sgd_momentum_ema(L.ptr(model.flat_params), L.ptr(grads), L.ptr(buf),
-                                                  L.ptr(ema_model.flat_params), n, lr, self.momentum, self.weight_decay,
-                                                  self._grad_scale, first, ema_alpha, st), "hpfg_sgd_momentum_ema")
-        return lr
+            alpha = min(1 - 1 / (self.cur_itrs + 1), self.ema_decay)      # utils/utils.py:84
+            L.check(lib.hpfg_sgd_momentum_ema(p, g, m, L.ptr(ema_model.flat_params), n, self._lr(), self.momentum,
+                                              self.weight_decay, self._grad_scale, first, alpha, st), "hpfg_sgd_momentum_ema")
 
 
 class MeanTeacherStep(_StepBase):
-    _graph_dp_capable = True
-
     def __init__(self, model, ema_model, *, ema_decay=0.99, **kw):
         super().__init__(**kw)
         self.model, self.ema_model, self.ema_decay = model, ema_model, ema_decay
-        self.in_channels, self.num_classes = model.in_channels, model.num_classes
-        model.train()
-        ema_model.train()                               # the teacher runs in train() mode (2017_03...:70)
-        model.ensure_flat()
-        ema_model.ensure_flat()
-        self.grads = torch.zeros_like(model.flat_params)
-        self.mom = torch.zeros_like(model.flat_params)
-        self._check_buffers()
-        self._broadcast_from_rank0()
+        # the teacher runs in train() mode (2017_03...:70)
+        [(self.grads, self.mom)] = self._setup([model], [model, ema_model], train=[model, ema_model])
 
     def step(self, x, labels):
         """x: [n_l+n_u, C, H, W] fp32 CUDA (labeled slices first); labels: [n_l, H, W] int64 CUDA."""
         self.cur_itrs += 1
         self._check_buffers()
-        if self._use_graph():
-            return self._step_graph(x, labels)
-        n_l = labels.shape[0]
+        ins = [x, labels]
+        out = (self._graph_replay(ins, self._dyn_scalars(self.ema_decay), [self.ema_model, self.model], self._body)
+               if self._use_graph() else self._body(ins, None))
+        self.last = dict(out, lr=self._lr(), w=self._consistency_weight())
+        return out["scalars"][0]
+
+    def _body(self, ins, dv):
+        x, labels = ins
+        n_l, dev = labels.shape[0], x.device
+        shape = (x.shape[0], self.num_classes, x.shape[2], x.shape[3])
         # the teacher forward is independent of the student forward: it runs on a side stream so that each network's
         # small / dependent kernels fill the other's bubbles (the teacher sees the whole batch, 2017_03...:100)
-        main = torch.cuda.current_stream(x.device)
-        side = main if getattr(self, "serialize", False) else self._side_stream(x.device)   # serialize: profiling only
-        side.wait_stream(main)
-        shape = (x.shape[0], self.num_classes, x.shape[2], x.shape[3])
+        main, side = self._fork(dev)
         with torch.cuda.stream(side):
-            _, t_out = self._forward(self.ema_model, x, False, out=self._persistent("t_out", shape, x.device))
-        plan, out = self._forward(self.model, x, True, out=self._persistent("s_out", shape, x.device))
+            _, t_out = self._forward(self.ema_model, x, False, self._persistent("t_out", shape, dev), dv)
+        plan, out = self._forward(self.model, x, True, self._persistent("s_out", shape, dev), dv)
         main.wait_stream(side)
         w = self._consistency_weight()
         with self._global_sums():
-            r = ssl_loss_raw(L.LOSS_MT, out, t_out[n_l:], labels, n_l, cons_weight=w)
+            r = ssl_loss_raw(L.LOSS_MT, out, t_out[n_l:], labels, n_l, cons_weight=w, cons_weight_dev=self._dv_scalar(dv, 3))
         self._global_consistency_value(r["scalars"], w)
         self._backward(self.model, plan, r["dstudent"], self.grads)
-        alpha = min(1 - 1 / (self.cur_itrs + 1), self.ema_decay)      # utils/utils.py:84
-        lr = self._sgd(self.model, self.grads, self.mom, self.ema_model, alpha)
-        self.last = dict(scalars=r["scalars"], lr=lr, w=w, logits=out, teacher_logits=t_out)
-        return r["scalars"][0]
-
-    def _step_graph(self, x, labels):
-        dyn = self._dyn_scalars(self.ema_decay)
-        out = self._graph_replay([x, labels], dyn, [self.model, self.ema_model], self._step_body_dv)
-        self.last = dict(scalars=out["scalars"], lr=dyn[0], w=dyn[3], logits=out["logits"], teacher_logits=out["teacher_logits"])
-        return out["scalars"][0]
-
-    def _step_body_dv(self, ins, dyn_f, dyn_o):
-        """The step with every per-iteration scalar read from the device block (captured once, replayed)."""
-        x, labels = ins
-        n_l = labels.shape[0]
-        dev = x.device
-        main, side = torch.cuda.current_stream(dev), self._side_stream(dev)
-        shape = (x.shape[0], self.num_classes, x.shape[2], x.shape[3])
-        side.wait_stream(main)
-        with torch.cuda.stream(side):
-            tplan = self.ema_model._acquire_plan(x, need_grad=False)
-            self._set_forward_share(tplan, True)
-            t_out = self.ema_model._run_forward(tplan, x, save=False, out=self._persistent("t_out", shape, dev),
-                                                offset_dev=dyn_o[1:2])
-        plan = self.model._acquire_plan(x, need_grad=True)
-        self._set_forward_share(plan, True)
-        out = self.model._run_forward(plan, x, save=True, out=self._persistent("s_out", shape, dev), offset_dev=dyn_o[0:1])
-        main.wait_stream(side)
-        r = ssl_loss_raw(L.LOSS_MT, out, t_out[n_l:], labels, n_l, cons_weight_dev=dyn_f[3:4])
-        self._backward(self.model, plan, r["dstudent"], self.grads)
-        n = self.model.flat_params.numel()
-        L.check(L.lib().hpfg_sgd_momentum_ema_dv(L.ptr(self.model.flat_params), L.ptr(self.grads), L.ptr(self.mom),
-                                                 L.ptr(self.ema_model.flat_params), n, self.momentum, self.weight_decay,
-                                                 1.0 / self.world, 0, L.ptr(dyn_f), L.stream_ptr(dev)),
-                "hpfg_sgd_momentum_ema_dv")
+        self._sgd(self.model, self.grads, self.mom, dv, self.ema_model)
         return dict(scalars=r["scalars"], logits=out, teacher_logits=t_out)
 
 
@@ -462,65 +444,37 @@ class CPSStep(_StepBase):
     def __init__(self, model1, model2, **kw):
         super().__init__(**kw)
         self.m1, self.m2 = model1, model2
-        self.in_channels, self.num_classes = model1.in_channels, model1.num_classes
-        model1.train()
-        model2.train()
-        model1.ensure_flat()
-        model2.ensure_flat()
-        self.g1, self.g2 = torch.zeros_like(model1.flat_params), torch.zeros_like(model2.flat_params)
-        self.b1, self.b2 = torch.zeros_like(model1.flat_params), torch.zeros_like(model2.flat_params)
-        self._check_buffers()
-        self._broadcast_from_rank0()
+        (self.g1, self.b1), (self.g2, self.b2) = self._setup([model1, model2], [model1, model2])
 
     def step(self, x, labels):
         self.cur_itrs += 1
         self._check_buffers()
-        if self._use_graph():
-            dyn = self._dyn_scalars()
-            out = self._graph_replay([x, labels], dyn, [self.m1, self.m2], self._body_dv)
-            self.last = dict(scalars=out["scalars"], lr=dyn[0], w=dyn[3], logits1=out["logits1"], logits2=out["logits2"])
-            return out["scalars"][0]
-        n_l = labels.shape[0]
-        # the two networks are independent except for the loss: network 2 runs on a side stream (forward, then backward + SGD)
-        main = torch.cuda.current_stream(x.device)
-        side = main if getattr(self, "serialize", False) else self._side_stream(x.device)
+        ins = [x, labels]
+        out = (self._graph_replay(ins, self._dyn_scalars(), [self.m2, self.m1], self._body)
+               if self._use_graph() else self._body(ins, None))
+        self.last = dict(out, lr=self._lr(), w=self._consistency_weight())
+        return out["scalars"][0]
+
+    def _body(self, ins, dv):
+        x, labels = ins
+        n_l, dev = labels.shape[0], x.device
         shape = (x.shape[0], self.num_classes, x.shape[2], x.shape[3])
-        side.wait_stream(main)
+        # the two networks are independent except for the loss: network 2 runs on a side stream (forward, then backward + SGD)
+        main, side = self._fork(dev)
         with torch.cuda.stream(side):
-            p2, o2 = self._forward(self.m2, x, True, out=self._persistent("o2", shape, x.device))
-        p1, o1 = self._forward(self.m1, x, True, out=self._persistent("o1", shape, x.device))
+            p2, o2 = self._forward(self.m2, x, True, self._persistent("o2", shape, dev), dv)
+        p1, o1 = self._forward(self.m1, x, True, self._persistent("o1", shape, dev), dv)
         main.wait_stream(side)
         w = self._consistency_weight()
         with self._global_sums():
-            r = ssl_loss_raw(L.LOSS_CPS, o1, o2, labels, n_l, cons_weight=w, want_pseudo=False)
+            r = ssl_loss_raw(L.LOSS_CPS, o1, o2, labels, n_l, cons_weight=w, cons_weight_dev=self._dv_scalar(dv, 3),
+                             want_pseudo=False)
         side.wait_stream(main)
         with torch.cuda.stream(side):
             self._backward(self.m2, p2, r["dother"], self.g2)
-            self._sgd(self.m2, self.g2, self.b2)
+            self._sgd(self.m2, self.g2, self.b2, dv)
         self._backward(self.m1, p1, r["dstudent"], self.g1)
-        lr = self._sgd(self.m1, self.g1, self.b1)
-        main.wait_stream(side)
-        self.last = dict(scalars=r["scalars"], lr=lr, w=w, logits1=o1, logits2=o2)
-        return r["scalars"][0]
-
-
-    def _body_dv(self, ins, f, o):
-        x, labels = ins
-        n_l, dev = labels.shape[0], x.device
-        main, side = torch.cuda.current_stream(dev), self._side_stream(dev)
-        shape = (x.shape[0], self.num_classes, x.shape[2], x.shape[3])
-        side.wait_stream(main)
-        with torch.cuda.stream(side):
-            p2, o2 = self._forward_dv(self.m2, x, True, self._persistent("o2", shape, dev), o[1:2])
-        p1, o1 = self._forward_dv(self.m1, x, True, self._persistent("o1", shape, dev), o[0:1])
-        main.wait_stream(side)
-        r = ssl_loss_raw(L.LOSS_CPS, o1, o2, labels, n_l, cons_weight_dev=f[3:4], want_pseudo=False)
-        side.wait_stream(main)
-        with torch.cuda.stream(side):
-            self._backward(self.m2, p2, r["dother"], self.g2)
-            self._sgd_dv(self.m2, self.g2, self.b2, f)
-        self._backward(self.m1, p1, r["dstudent"], self.g1)
-        self._sgd_dv(self.m1, self.g1, self.b1, f)
+        self._sgd(self.m1, self.g1, self.b1, dv)
         main.wait_stream(side)
         return dict(scalars=r["scalars"], logits1=o1, logits2=o2)
 
@@ -531,84 +485,42 @@ class UAMTStep(_StepBase):
     def __init__(self, model, ema_model, *, ema_decay=0.99, T=8, **kw):
         super().__init__(**kw)
         self.model, self.ema_model, self.ema_decay, self.T = model, ema_model, ema_decay, T
-        self.in_channels, self.num_classes = model.in_channels, model.num_classes
-        model.train()
-        ema_model.train()
-        model.ensure_flat()
-        ema_model.ensure_flat()
-        self.grads = torch.zeros_like(model.flat_params)
-        self.mom = torch.zeros_like(model.flat_params)
-        self._check_buffers()
-        self._broadcast_from_rank0()
+        [(self.grads, self.mom)] = self._setup([model], [model, ema_model], train=[model, ema_model])
 
-    @staticmethod
-    def make_noise(like):
-        return torch.clamp(torch.randn_like(like) * 0.1, -0.2, 0.2)      # 2019_07...:130,141
+    def _threshold(self):
+        """Entropy threshold of the certainty mask (2019_07...:150)."""
+        return (0.75 + 0.25 * sigmoid_rampup(self.cur_itrs, self.total_itrs)) * math.log(2)
 
     def step(self, x, labels, noise=None, mc_noise=None, teacher_masks=None):
-        """noise [n_u,...] / mc_noise [T//2, 2*n_u, ...]: the clamped perturbations; drawn here if None.
-        teacher_masks (parity harness only, eager path): 1 + T//2 dropout keep-mask sets, one per teacher forward in call
+        """noise [n_u,...] / mc_noise [T//2, 2*n_u, ...]: the clamped perturbations; each drawn here (one draw) if None.
+        teacher_masks (parity harness only, eager launches): 1 + T//2 dropout keep-mask sets, one per teacher forward in call
         order (the consistency forward on n_u slices, then the T//2 Monte-Carlo forwards on 2*n_u slices) -- every
         stochastic teacher pass draws its own masks, as nn.Dropout does in the reference (2019_07...:134-143)."""
         self.cur_itrs += 1
         self._check_buffers()
-        n_l = labels.shape[0]
-        x_u = x[n_l:]
-        n_u = x_u.shape[0]
+        x_u = x[labels.shape[0]:]
         if noise is None:
-            noise = self.make_noise(x_u)
-        if self._use_graph() and teacher_masks is None:
-            if mc_noise is None:
-                mc_noise = torch.clamp(torch.randn((self.T // 2, 2 * n_u) + tuple(x_u.shape[1:]), device=x.device,
-                                                   dtype=x.dtype) * 0.1, -0.2, 0.2)
-            dyn = self._dyn_scalars(self.ema_decay)
-            thr = (0.75 + 0.25 * sigmoid_rampup(self.cur_itrs, self.total_itrs)) * math.log(2)
-            out = self._graph_replay([x, labels, noise, mc_noise.contiguous()], dyn + [thr],
-                                     [self.model] + [self.ema_model] * (1 + self.T // 2), self._body_dv)
-            self.last = dict(scalars=out["scalars"], lr=dyn[0], w=dyn[3], threshold=thr, logits=out["logits"],
-                             teacher_logits=out["teacher_logits"], mc_logits=out["mc_logits"])
-            return out["scalars"][0]
-        xr = x_u.repeat(2, 1, 1, 1)
-        noises = [mc_noise[i] if mc_noise is not None else self.make_noise(xr) for i in range(self.T // 2)]
-        x_t = (x_u + noise).contiguous()
-        x_mc = [(xr + nz).contiguous() for nz in noises]
-        ncls, hh, ww = self.num_classes, x.shape[2], x.shape[3]
-        mc = self._persistent("mc", (self.T * n_u, ncls, hh, ww), x.device)
-        # the five teacher forwards are independent of the student forward: side stream
-        main = torch.cuda.current_stream(x.device)
-        side = main if getattr(self, "serialize", False) else self._side_stream(x.device)
-        side.wait_stream(main)
+            noise = _input_noise(x_u.shape, x_u)
+        if mc_noise is None:
+            mc_noise = _input_noise((self.T // 2, 2 * x_u.shape[0]) + tuple(x_u.shape[1:]), x_u)
+        self._teacher_masks = None
         if teacher_masks is not None:
             assert len(teacher_masks) == 1 + self.T // 2, "one mask set per teacher forward"
-            dev_sets = []                  # uploaded on the main stream before the fork; kept alive until the next step
+            self._teacher_masks = []       # uploaded on the calling stream before the fork; kept alive until the next step
             for ms in teacher_masks:
                 self.ema_model.set_dropout_masks(ms)
-                dev_sets.append(self.ema_model._dropout_masks)
-            self._mask_keepalive = dev_sets
-            side.wait_stream(main)
-        with torch.cuda.stream(side):
-            if teacher_masks is not None:
-                self.ema_model._dropout_masks = dev_sets[0]
-            _, t_out = self._forward(self.ema_model, x_t, False, out=self._persistent("t_out", (n_u, ncls, hh, ww), x.device))
-            for i in range(self.T // 2):
-                if teacher_masks is not None:
-                    self.ema_model._dropout_masks = dev_sets[1 + i]
-                self._forward(self.ema_model, x_mc[i], False, out=mc[2 * n_u * i:2 * n_u * (i + 1)])
-        plan, out = self._forward(self.model, x, True, out=self._persistent("s_out", (x.shape[0], ncls, hh, ww), x.device))
-        main.wait_stream(side)
-        w = self._consistency_weight()
-        thr = (0.75 + 0.25 * sigmoid_rampup(self.cur_itrs, self.total_itrs)) * math.log(2)
-        with self._global_sums():
-            r = ssl_loss_raw(L.LOSS_UAMT, out, t_out, labels, n_l, cons_weight=w, mc_logits=mc, mc_passes=self.T,
-                             uamt_threshold=thr)
-        self._backward(self.model, plan, r["dstudent"], self.grads)
-        alpha = min(1 - 1 / (self.cur_itrs + 1), self.ema_decay)
-        lr = self._sgd(self.model, self.grads, self.mom, self.ema_model, alpha)
-        self.last = dict(scalars=r["scalars"], lr=lr, w=w, threshold=thr, logits=out, teacher_logits=t_out, mc_logits=mc)
-        return r["scalars"][0]
+                self._teacher_masks.append(self.ema_model._dropout_masks)
+        ins = [x, labels, noise, mc_noise.contiguous()]
+        thr = self._threshold()
+        if teacher_masks is None and self._use_graph():
+            out = self._graph_replay(ins, self._dyn_scalars(self.ema_decay) + [thr],
+                                     [self.ema_model] * (1 + self.T // 2) + [self.model], self._body)
+        else:
+            out = self._body(ins, None)
+        self.last = dict(out, lr=self._lr(), w=self._consistency_weight(), threshold=thr)
+        return out["scalars"][0]
 
-
-    def _body_dv(self, ins, f, o):
+    def _body(self, ins, dv):
         x, labels, noise, mc_noise = ins
         n_l, dev = labels.shape[0], x.device
         x_u = x[n_l:]
@@ -618,18 +530,24 @@ class UAMTStep(_StepBase):
         x_mc = [(xr + mc_noise[i]).contiguous() for i in range(self.T // 2)]
         ncls, hh, ww = self.num_classes, x.shape[2], x.shape[3]
         mc = self._persistent("mc", (self.T * n_u, ncls, hh, ww), dev)
-        main, side = torch.cuda.current_stream(dev), self._side_stream(dev)
-        side.wait_stream(main)
+        # the five teacher forwards are independent of the student forward: side stream
+        main, side = self._fork(dev)
         with torch.cuda.stream(side):
-            _, t_out = self._forward_dv(self.ema_model, x_t, False, self._persistent("t_out", (n_u, ncls, hh, ww), dev), o[1:2])
-            for i in range(self.T // 2):
-                self._forward_dv(self.ema_model, x_mc[i], False, mc[2 * n_u * i:2 * n_u * (i + 1)], o[2 + i:3 + i])
-        plan, out = self._forward_dv(self.model, x, True, self._persistent("s_out", (x.shape[0], ncls, hh, ww), dev), o[0:1])
+            t_out = self._persistent("t_out", (n_u, ncls, hh, ww), dev)
+            outs = [t_out] + [mc[2 * n_u * i:2 * n_u * (i + 1)] for i in range(self.T // 2)]
+            for i, (xi, oi) in enumerate(zip([x_t] + x_mc, outs)):
+                if self._teacher_masks is not None:
+                    self.ema_model._dropout_masks = self._teacher_masks[i]
+                self._forward(self.ema_model, xi, False, oi, dv)
+        plan, out = self._forward(self.model, x, True, self._persistent("s_out", (x.shape[0], ncls, hh, ww), dev), dv)
         main.wait_stream(side)
-        r = ssl_loss_raw(L.LOSS_UAMT, out, t_out, labels, n_l, mc_logits=mc, mc_passes=self.T, cons_weight_dev=f[3:4],
-                         uamt_threshold_dev=f[4:5])
+        w = self._consistency_weight()
+        with self._global_sums():
+            r = ssl_loss_raw(L.LOSS_UAMT, out, t_out, labels, n_l, cons_weight=w, mc_logits=mc, mc_passes=self.T,
+                             uamt_threshold=self._threshold(), cons_weight_dev=self._dv_scalar(dv, 3),
+                             uamt_threshold_dev=self._dv_scalar(dv, 4))
         self._backward(self.model, plan, r["dstudent"], self.grads)
-        self._sgd_dv(self.model, self.grads, self.mom, f, self.ema_model)
+        self._sgd(self.model, self.grads, self.mom, dv, self.ema_model)
         return dict(scalars=r["scalars"], logits=out, teacher_logits=t_out, mc_logits=mc)
 
 
@@ -642,14 +560,7 @@ class ICTStep(_StepBase):
     def __init__(self, model, ema_model, *, ema_decay=0.99, ict_alpha=0.2, **kw):
         super().__init__(**kw)
         self.model, self.ema_model, self.ema_decay, self.ict_alpha = model, ema_model, ema_decay, ict_alpha
-        self.in_channels, self.num_classes = model.in_channels, model.num_classes
-        model.train()
-        model.ensure_flat()
-        ema_model.ensure_flat()
-        self.grads = torch.zeros_like(model.flat_params)
-        self.mom = torch.zeros_like(model.flat_params)
-        self._check_buffers()
-        self._broadcast_from_rank0()
+        [(self.grads, self.mom)] = self._setup([model], [model, ema_model])
 
     def draw_mix_factors(self, n_mixed):
         """np.random.beta(alpha, alpha, size=(n_u//2,1,1,1)) (2022_02...:112-113): host RNG, as in the reference."""
@@ -660,66 +571,40 @@ class ICTStep(_StepBase):
         """x: [n_l+n_u, C, H, W] (labeled first, n_u even); mix_factors: [n_u//2] floats (drawn here if None)."""
         self.cur_itrs += 1
         self._check_buffers()
-        n_l = labels.shape[0]
-        n_u = x.shape[0] - n_l
+        n_u = x.shape[0] - labels.shape[0]
         assert n_u % 2 == 0, "ICT needs an even unlabeled batch"
-        n_m = n_u // 2
-        dev = x.device
         if mix_factors is None:
-            mix_factors = self.draw_mix_factors(n_m)
-        lam = mix_factors.reshape(-1).to(device=dev, dtype=torch.float32, non_blocking=True).contiguous()
-        if self._use_graph():
-            dyn = self._dyn_scalars(self.ema_decay)
-            out = self._graph_replay([x, labels, lam], dyn, [self.model, self.ema_model, self.ema_model], self._body_dv)
-            self.last = dict(scalars=out["scalars"], lr=dyn[0], w=dyn[3], logits=out["logits"],
-                             teacher_logits=out["teacher_logits"], mix_factors=lam)
-            return out["scalars"][0]
-        ux0, ux1 = x[n_l:n_l + n_m], x[n_l + n_m:]
-        ncls, hh, ww = self.num_classes, x.shape[2], x.shape[3]
-        main = torch.cuda.current_stream(dev)
-        side = main if getattr(self, "serialize", False) else self._side_stream(dev)
-        side.wait_stream(main)
-        t_out = self._persistent("t_out", (n_u, ncls, hh, ww), dev)
-        with torch.cuda.stream(side):            # the two teacher forwards are independent of the student forward
-            self._forward(self.ema_model, ux0, False, out=t_out[:n_m])
-            self._forward(self.ema_model, ux1, False, out=t_out[n_m:])
-        x_in = self._persistent("x_in", (n_l + n_m,) + tuple(x.shape[1:]), dev)
-        x_in[:n_l].copy_(x[:n_l])
-        L.check(L.lib().hpfg_ict_mix(L.ptr(ux0), L.ptr(ux1), L.ptr(lam), n_m, ux0[0].numel(), L.ptr(x_in[n_l:]),
-                                     L.stream_ptr(dev)), "hpfg_ict_mix")
-        plan, out = self._forward(self.model, x_in, True, out=self._persistent("s_out", (n_l + n_m, ncls, hh, ww), dev))
-        main.wait_stream(side)
-        w = self._consistency_weight()
-        with self._global_sums():
-            r = ict_loss_raw(out, t_out, lam, labels, n_l, cons_weight=w)
-        self._global_consistency_value(r["scalars"], w)
-        self._backward(self.model, plan, r["dstudent"], self.grads)
-        alpha = min(1 - 1 / (self.cur_itrs + 1), self.ema_decay)
-        lr = self._sgd(self.model, self.grads, self.mom, self.ema_model, alpha)
-        self.last = dict(scalars=r["scalars"], lr=lr, w=w, logits=out, teacher_logits=t_out, mix_factors=lam)
-        return r["scalars"][0]
+            mix_factors = self.draw_mix_factors(n_u // 2)
+        lam = mix_factors.reshape(-1).to(device=x.device, dtype=torch.float32, non_blocking=True).contiguous()
+        ins = [x, labels, lam]
+        out = (self._graph_replay(ins, self._dyn_scalars(self.ema_decay), [self.ema_model, self.ema_model, self.model], self._body)
+               if self._use_graph() else self._body(ins, None))
+        self.last = dict(out, lr=self._lr(), w=self._consistency_weight(), mix_factors=lam)
+        return out["scalars"][0]
 
-    def _body_dv(self, ins, f, o):
+    def _body(self, ins, dv):
         x, labels, lam = ins
         n_l, dev = labels.shape[0], x.device
         n_m = (x.shape[0] - n_l) // 2
         ux0, ux1 = x[n_l:n_l + n_m], x[n_l + n_m:]
         ncls, hh, ww = self.num_classes, x.shape[2], x.shape[3]
-        main, side = torch.cuda.current_stream(dev), self._side_stream(dev)
-        side.wait_stream(main)
+        main, side = self._fork(dev)
         t_out = self._persistent("t_out", (2 * n_m, ncls, hh, ww), dev)
-        with torch.cuda.stream(side):
-            self._forward_dv(self.ema_model, ux0, False, t_out[:n_m], o[1:2])
-            self._forward_dv(self.ema_model, ux1, False, t_out[n_m:], o[2:3])
+        with torch.cuda.stream(side):            # the two teacher forwards are independent of the student forward
+            self._forward(self.ema_model, ux0, False, t_out[:n_m], dv)
+            self._forward(self.ema_model, ux1, False, t_out[n_m:], dv)
         x_in = self._persistent("x_in", (n_l + n_m,) + tuple(x.shape[1:]), dev)
         x_in[:n_l].copy_(x[:n_l])
         L.check(L.lib().hpfg_ict_mix(L.ptr(ux0), L.ptr(ux1), L.ptr(lam), n_m, ux0[0].numel(), L.ptr(x_in[n_l:]),
                                      L.stream_ptr(dev)), "hpfg_ict_mix")
-        plan, out = self._forward_dv(self.model, x_in, True, self._persistent("s_out", (n_l + n_m, ncls, hh, ww), dev), o[0:1])
+        plan, out = self._forward(self.model, x_in, True, self._persistent("s_out", (n_l + n_m, ncls, hh, ww), dev), dv)
         main.wait_stream(side)
-        r = ict_loss_raw(out, t_out, lam, labels, n_l, cons_weight_dev=f[3:4])
+        w = self._consistency_weight()
+        with self._global_sums():
+            r = ict_loss_raw(out, t_out, lam, labels, n_l, cons_weight=w, cons_weight_dev=self._dv_scalar(dv, 3))
+        self._global_consistency_value(r["scalars"], w)
         self._backward(self.model, plan, r["dstudent"], self.grads)
-        self._sgd_dv(self.model, self.grads, self.mom, f, self.ema_model)
+        self._sgd(self.model, self.grads, self.mom, dv, self.ema_model)
         return dict(scalars=r["scalars"], logits=out, teacher_logits=t_out)
 
 
@@ -727,31 +612,19 @@ class S4CVStep(_StepBase):
     """S4CVNet (2022_08_CVPR_S4CVNet_ACDC.py:108-167): two student networks trained with cross pseudo supervision (Dice only,
     weight 7w) plus, from iteration ``mt_start`` on, Mean-Teacher MSE of both students against the EMA teacher of student 2,
     which sees the noise-perturbed unlabeled slices.  w = consistency * linear_rampup(cur_itrs // 150, rampup) (:148-149).
-    One fused loss call (``hpfg_s4cv_loss``) produces the value and both logit gradients."""
+    One fused loss call (``hpfg_s4cv_loss``) produces the value and both logit gradients.  Eager launches only."""
     share_forward = False
 
     def __init__(self, model1, model2, ema_model, *, ema_decay=0.99, mt_start=1000, **kw):
         super().__init__(**kw)
         self.m1, self.m2, self.ema_model, self.ema_decay, self.mt_start = model1, model2, ema_model, ema_decay, mt_start
-        self.in_channels, self.num_classes = model1.in_channels, model1.num_classes
-        model1.train()
-        model2.train()
-        for m in (model1, model2, ema_model):
-            m.ensure_flat()
-        self.g1, self.g2 = torch.zeros_like(model1.flat_params), torch.zeros_like(model2.flat_params)
-        self.b1, self.b2 = torch.zeros_like(model1.flat_params), torch.zeros_like(model2.flat_params)
-        self._check_buffers()
-        self._broadcast_from_rank0()
+        (self.g1, self.b1), (self.g2, self.b2) = self._setup([model1, model2], [model1, model2, ema_model])
 
-    def _models(self):
-        return [self.m1, self.m2, self.ema_model]
+    def _use_graph(self):
+        return False
 
     def _consistency_weight(self):
         return self.consistency * linear_rampup(self.cur_itrs // 150, self.consistency_rampup)
-
-    @staticmethod
-    def make_noise(like):
-        return torch.clamp(torch.randn_like(like) * 0.1, -0.2, 0.2)      # 2022_08...:111
 
     def step(self, x, labels, noise=None):
         """x: [n_l+n_u, C, H, W] (labeled first); labels: [n_l, H, W]; noise [n_u, ...]: drawn here if None."""
@@ -760,31 +633,28 @@ class S4CVStep(_StepBase):
         n_l, dev = labels.shape[0], x.device
         x_u = x[n_l:]
         if noise is None:
-            noise = self.make_noise(x_u)
+            noise = _input_noise(x_u.shape, x_u)
         x_t = (x_u + noise).contiguous()
         ncls, hh, ww = self.num_classes, x.shape[2], x.shape[3]
-        main = torch.cuda.current_stream(dev)
-        side = main if getattr(self, "serialize", False) else self._side_stream(dev)
         shape = (x.shape[0], ncls, hh, ww)
-        side.wait_stream(main)
+        main, side = self._fork(dev)
         with torch.cuda.stream(side):               # student 2 and its teacher on the side stream, student 1 on the main stream
-            p2, o2 = self._forward(self.m2, x, True, out=self._persistent("o2", shape, dev))
-            _, t_out = self._forward(self.ema_model, x_t, False, out=self._persistent("t_out", (x_u.shape[0], ncls, hh, ww), dev))
-        p1, o1 = self._forward(self.m1, x, True, out=self._persistent("o1", shape, dev))
+            p2, o2 = self._forward(self.m2, x, True, self._persistent("o2", shape, dev), None)
+            _, t_out = self._forward(self.ema_model, x_t, False, self._persistent("t_out", (x_u.shape[0], ncls, hh, ww), dev), None)
+        p1, o1 = self._forward(self.m1, x, True, self._persistent("o1", shape, dev), None)
         main.wait_stream(side)
         w = self._consistency_weight()
         mt_on = self.cur_itrs >= self.mt_start
         with self._global_sums():
             r = s4cv_loss_raw(o1, o2, t_out if mt_on else None, labels, n_l, cps_weight=7.0 * w, mt_weight=w)
         side.wait_stream(main)
-        alpha = min(1 - 1 / (self.cur_itrs + 1), self.ema_decay)
         with torch.cuda.stream(side):
             self._backward(self.m2, p2, r["dother"], self.g2)
-            self._sgd(self.m2, self.g2, self.b2, self.ema_model, alpha)      # SGD of student 2 + EMA into its teacher, one pass
+            self._sgd(self.m2, self.g2, self.b2, None, self.ema_model)      # SGD of student 2 + EMA into its teacher, one pass
         self._backward(self.m1, p1, r["dstudent"], self.g1)
-        lr = self._sgd(self.m1, self.g1, self.b1)
+        self._sgd(self.m1, self.g1, self.b1, None)
         main.wait_stream(side)
-        self.last = dict(scalars=r["scalars"], lr=lr, w=w, logits1=o1, logits2=o2, teacher_logits=t_out)
+        self.last = dict(scalars=r["scalars"], lr=self._lr(), w=w, logits1=o1, logits2=o2, teacher_logits=t_out)
         return r["scalars"][0]
 
 
@@ -805,31 +675,14 @@ class HPFGStep(_StepBase):
         super().__init__(**kw)
         from .losses import Dense_Loss
         self.m1, self.m2, self.ema_model, self.ema_decay, self.mt_start = model1, model2, ema_model, ema_decay, mt_start
-        self.in_channels, self.num_classes = model1.in_channels, model1.num_classes
-        model1.train()
-        model2.train()
-        for m in (model1, model2, ema_model):
-            m.ensure_flat()
+        self._neck_mom = {}                         # id(parameter) -> momentum buffer of the neck tensors (outside the flat buffer)
+        # the gradients come from autograd (model.last_flat_grad): momentum buffers only
+        (_, self.b1), (_, self.b2) = self._setup([model1, model2], [model1, model2, ema_model], grads=False)
         for p in ema_model.parameters():
             p.requires_grad = False
         self.temperature = temperature
         self._dense = None
         self._DenseLoss = Dense_Loss
-        self.b1, self.b2 = torch.zeros_like(model1.flat_params), torch.zeros_like(model2.flat_params)
-        self._neck_mom = {}                         # id(parameter) -> momentum buffer of the neck tensors (outside the flat buffer)
-        self._check_buffers()
-        self._broadcast_from_rank0()
-
-    def _models(self):
-        return [self.m1, self.m2, self.ema_model]
-
-    def _state_tensors(self):
-        return [self.b1, self.b2]
-
-    def _check_buffers(self):
-        for model, buf in ((self.m1, self.b1), (self.m2, self.b2)):
-            if buf.device != model.flat_params.device or buf.numel() != model.flat_params.numel():
-                raise L.HpfgError("HPFGStep: momentum buffer no longer matches the model's flat parameters")
 
     def _consistency_weight(self):
         return self.consistency * linear_rampup(self.cur_itrs // 150, self.consistency_rampup)
@@ -841,7 +694,7 @@ class HPFGStep(_StepBase):
             return
         import torch.distributed as dist
         src = dist.get_global_rank(self.pg, 0) if self.pg is not None else 0
-        for m in self._models():
+        for m in self._networks:
             for p in self._neck_params(m):
                 dist.broadcast(p.data, src=src, group=self.pg)
 
@@ -856,7 +709,7 @@ class HPFGStep(_StepBase):
         ``model.parameters()``); tensors that never received a gradient (model1's necks: main.py:148 drops their outputs) have
         no state, as in torch."""
         out = super().state_dict()
-        for model, opt in zip((self.m1, self.m2), out["optimizers"]):
+        for model, opt in zip((m for m, _, _ in self._trained), out["optimizers"]):
             base = len(model._layout)
             necks = self._neck_params(model)
             opt["param_groups"][0]["params"] = list(range(base + len(necks)))
@@ -869,7 +722,7 @@ class HPFGStep(_StepBase):
     def load_state_dict(self, sd):
         super().load_state_dict(sd)
         self._neck_mom = {}
-        for model, opt in zip((self.m1, self.m2), sd.get("optimizers", [])):
+        for model, opt in zip((m for m, _, _ in self._trained), sd.get("optimizers", [])):
             base = len(model._layout)
             for j, p in enumerate(self._neck_params(model)):
                 st = opt["state"].get(base + j)

@@ -204,11 +204,14 @@ int hpfg_ssl_loss(int mode, const float *student, const float *other, const floa
                   float dice_coef, float *dstudent, float *dother, float *scalars_out, int64_t *pseudo1,
                   int64_t *pseudo2, void *workspace, void *stream);
 
+/* hpfg_ssl_loss with the consistency weight read from device memory (cons_weight_dev, required) and, when
+ * uamt_threshold_dev is not NULL, the UAMT threshold too (2019_07...:150, it ramps with the iteration count); with
+ * uamt_threshold_dev NULL the by-value uamt_threshold is used. */
 int hpfg_ssl_loss_dv(int mode, const float *student, const float *other, const float *mc_logits, int mc_passes,
                      const int64_t *labels, int n_l, int n_u, int num_classes, int height, int width,
-                     const float *cons_weight_dev, float uamt_threshold, const float *class_weights, float ce_coef,
-                     float dice_coef, float *dstudent, float *dother, float *scalars_out, int64_t *pseudo1,
-                     int64_t *pseudo2, void *workspace, void *stream);
+                     const float *cons_weight_dev, float uamt_threshold, const float *uamt_threshold_dev,
+                     const float *class_weights, float ce_coef, float dice_coef, float *dstudent, float *dother,
+                     float *scalars_out, int64_t *pseudo1, int64_t *pseudo2, void *workspace, void *stream);
 
 /* ---- "next" rows of SURVEY 8f.4: the ICT-MedSeg and S4CVNet step losses on the same two kernels ------------------
  * ICT (2022_02_ISBI_ICT-MedSeg_ACDC.py:111-137): student = logits of cat([labeled, mixed unlabeled]) [n_l+n_mixed,C,H,W];
@@ -248,13 +251,6 @@ int hpfg_argmax_labels(const float *logits, int n, int num_classes, int height, 
  * where it is the no_grad teacher output: 2019_07...:134-143,148). */
 int hpfg_softmax_mse(const float *input_logits, const float *target_logits, const float *grad_out, int n, int num_classes,
                      int height, int width, int sigmoid, float *out, void *stream);
-
-/* hpfg_ssl_loss_dv with the UAMT threshold (2019_07...:150, it ramps with the iteration count) read from device memory too. */
-int hpfg_ssl_loss_dv2(int mode, const float *student, const float *other, const float *mc_logits, int mc_passes,
-                      const int64_t *labels, int n_l, int n_u, int num_classes, int height, int width,
-                      const float *cons_weight_dev, const float *uamt_threshold_dev, const float *class_weights,
-                      float ce_coef, float dice_coef, float *dstudent, float *dother, float *scalars_out,
-                      int64_t *pseudo1, int64_t *pseudo2, void *workspace, void *stream);
 
 /* DiceLoss.forward (utils/loss/diceloss.py:178-191) alone: inputs are probabilities (softmax == 0) or
  * logits (softmax != 0); target int64 [n,H,W]; dinputs optional. scalars_out: float[1+C] = {loss, dice_c..}. */

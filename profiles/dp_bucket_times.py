@@ -37,8 +37,8 @@ for _ in range(reps):
     e_start.record(main)
     side.wait_stream(main)
     with torch.cuda.stream(side):
-        _, t_out = step._forward(teacher, x, False, out=step._persistent("t_out", shape, dev))
-    plan, out = step._forward(student, x, True, out=step._persistent("s_out", shape, dev))
+        _, t_out = step._forward(teacher, x, False, step._persistent("t_out", shape, dev), None)
+    plan, out = step._forward(student, x, True, step._persistent("s_out", shape, dev), None)
     main.wait_stream(side)
     r = ssl_loss_raw(L.LOSS_MT, out, t_out[8:], y, 8, cons_weight=0.001)
     e_bwd0.record(main)
@@ -58,7 +58,7 @@ for _ in range(reps):
             evs.append((a, z))
     main.wait_stream(comm)
     e_sgd0.record(main)
-    step._sgd(student, step.grads, step.mom, teacher, 0.99)
+    step._sgd(student, step.grads, step.mom, None, teacher)
     e_sgd1.record(main)
     torch.cuda.synchronize()
     vals = {"forward+loss": e_start.elapsed_time(e_bwd0), "backward (main stream)": e_bwd0.elapsed_time(e_bwd1),

@@ -26,14 +26,14 @@ for _ in range(reps):
     main, side = torch.cuda.current_stream(), step._side_stream(dev)
     e = [ev() for _ in range(8)]
     e[0].record()
-    plan, out = step._forward(student, x, True, out=step._persistent("s_out", shape, dev))
+    plan, out = step._forward(student, x, True, step._persistent("s_out", shape, dev), None)
     e[1].record()
-    _, t_out = step._forward(teacher, x, False, out=step._persistent("t_out", shape, dev))
+    _, t_out = step._forward(teacher, x, False, step._persistent("t_out", shape, dev), None)
     e[2].record()
     side.wait_stream(main)
     with torch.cuda.stream(side):
-        _, t_out = step._forward(teacher, x, False, out=step._persistent("t_out", shape, dev))
-    plan, out = step._forward(student, x, True, out=step._persistent("s_out", shape, dev))
+        _, t_out = step._forward(teacher, x, False, step._persistent("t_out", shape, dev), None)
+    plan, out = step._forward(student, x, True, step._persistent("s_out", shape, dev), None)
     main.wait_stream(side)
     if os.environ.get("PHASE_SYNC"):
         torch.cuda.synchronize()
@@ -45,7 +45,7 @@ for _ in range(reps):
     step._backward(student, plan, r["dstudent"], step.grads)
     e[5].record()
     step.cur_itrs += 1
-    step._sgd(student, step.grads, step.mom, teacher, 0.99)
+    step._sgd(student, step.grads, step.mom, None, teacher)
     e[6].record()
     torch.cuda.synchronize()
     for i in range(6):

@@ -119,7 +119,8 @@ def test_graph_replay_policy_host_logic():
     to capture the NCCL bucket all-reduces with the step (a refused capture falls back to eager launches at run time)."""
     a, b = hb.UNet(1, 4), hb.UNet(1, 4)
     mt, cps, ict = hb.MeanTeacherStep(a, copy.deepcopy(a)), hb.CPSStep(a, b), hb.ICTStep(a, b)
-    for st in (mt, cps, ict):
+    uamt = hb.UAMTStep(a, copy.deepcopy(a))
+    for st in (mt, cps, uamt, ict):
         assert not st._use_graph()
         st.enable_graph(True)
         st.cur_itrs = 1
@@ -129,10 +130,73 @@ def test_graph_replay_policy_host_logic():
         st.world = 2
         assert not st._use_graph()                       # data parallel stays eager unless asked
         st.enable_graph(True, data_parallel=True)
-    assert mt._use_graph() and cps._use_graph() and ict._use_graph()
+    assert mt._use_graph() and cps._use_graph() and uamt._use_graph() and ict._use_graph()
     mt.enable_graph(False)
     assert not mt._use_graph()
     assert mt._dyn_scalars(0.99)[0] == pytest.approx(hb.medical_lr(2, 0.01, 30000))
+    s4cv = hb.S4CVStep(a, b, copy.deepcopy(b))           # eager launches only
+    s4cv.enable_graph(True, data_parallel=True)
+    for it in (1, 2, 3):
+        s4cv.cur_itrs = it
+        assert not s4cv._use_graph()
+
+
+def _step_driver(kind):
+    torch.manual_seed(5)
+    if kind == "hpfg":
+        m1, m2 = hb.UNet_Plus(1, 4), hb.UNet_Plus(1, 4)
+        nets = (m1, m2, copy.deepcopy(m2))
+    else:
+        a, b = hb.UNet(1, 4), hb.UNet(1, 4)
+        nets = (a, b, copy.deepcopy(b)) if kind == "s4cv" else (a, b) if kind == "cps" else (a, copy.deepcopy(a))
+    cls = dict(mt=hb.MeanTeacherStep, cps=hb.CPSStep, uamt=hb.UAMTStep, ict=hb.ICTStep, s4cv=hb.S4CVStep, hpfg=hb.HPFGStep)[kind]
+    return cls(*nets), nets
+
+
+# Checkpoint layout of each driver: the networks whose Philox offsets it saves (constructor positions, in order) and, per
+# optimizer entry, the momentum buffer attribute and the number of parameters of its network.
+CHECKPOINT_LAYOUT = {
+    "mt": ([0, 1], [("mom", 82)]),
+    "cps": ([0, 1], [("b1", 82), ("b2", 82)]),
+    "uamt": ([0, 1], [("mom", 82)]),
+    "ict": ([0, 1], [("mom", 82)]),
+    "s4cv": ([0, 1, 2], [("b1", 82), ("b2", 82)]),
+    "hpfg": ([0, 1, 2], [("b1", 98), ("b2", 98)]),
+}
+
+
+@pytest.mark.parametrize("kind", sorted(CHECKPOINT_LAYOUT))
+def test_step_driver_checkpoint_layout_and_roundtrip(kind):
+    """state_dict() of every step driver: Philox offsets of its networks in a fixed order, one torch.optim.SGD-style entry per
+    trained network (lr of the next iteration, per-parameter momentum in parameters() order), and it round-trips."""
+    philox_of, opts = CHECKPOINT_LAYOUT[kind]
+    st, nets = _step_driver(kind)
+    assert all(opt["state"] == {} for opt in st.state_dict()["optimizers"])       # no momentum before the first step
+    for i, m in enumerate(nets):
+        m._philox_offset = 8 * (i + 1)
+    st.cur_itrs = 7
+    for name, _ in opts:
+        getattr(st, name).uniform_(-1, 1)
+    if kind == "hpfg":
+        for p in st._neck_params(nets[1]):
+            st._neck_mom[id(p)] = torch.randn_like(p)
+    sd = st.state_dict()
+    assert sd["cur_itrs"] == 7 and sd["philox"] == [8 * (i + 1) for i in philox_of]
+    assert len(sd["optimizers"]) == len(opts)
+    for opt, (name, n_params) in zip(sd["optimizers"], opts):
+        assert opt["param_groups"] == [{"lr": 0.00999819998199868, "momentum": 0.9, "weight_decay": 1e-4,
+                                        "params": list(range(n_params))}]
+        assert sorted(opt["state"]) == list(range(98 if kind == "hpfg" and name == "b2" else 82))
+        flat = torch.cat([opt["state"][i]["momentum_buffer"].reshape(-1) for i in range(82)])
+        assert torch.equal(flat, getattr(st, name))
+    st2, nets2 = _step_driver(kind)
+    st2.load_state_dict(sd)
+    assert [m._philox_offset for m in nets2] == [8 * (i + 1) if i in philox_of else 0 for i in range(len(nets2))]
+    sd2 = st2.state_dict()
+    assert sd2["cur_itrs"] == 7 and sd2["philox"] == sd["philox"]
+    for o, o2 in zip(sd["optimizers"], sd2["optimizers"]):
+        assert o2["param_groups"] == o["param_groups"] and sorted(o2["state"]) == sorted(o["state"])
+        assert all(torch.equal(o2["state"][i]["momentum_buffer"], o["state"][i]["momentum_buffer"]) for i in o["state"])
 
 
 def test_necks_and_dense_loss_have_no_cpu_path():
