@@ -75,6 +75,8 @@ SIGNATURES = {
     "hpfg_sgd_momentum_ema": (c_int, [c_vp, c_vp, c_vp, c_vp, c_i64, c_f, c_f, c_f, c_f, c_int, c_f, c_vp]),
     "hpfg_sgd_momentum_ema_dv": (c_int, [c_vp, c_vp, c_vp, c_vp, c_i64, c_f, c_f, c_f, c_int, c_vp, c_vp]),
     "hpfg_sgd_momentum_dv": (c_int, [c_vp, c_vp, c_vp, c_i64, c_f, c_f, c_f, c_int, c_vp, c_vp]),
+    "hpfg_adam": (c_int, [c_vp] * 5 + [c_i64] + [c_f] * 5 + [c_int] + [c_f] * 5 + [c_vp]),
+    "hpfg_adam_dv": (c_int, [c_vp] * 5 + [c_i64] + [c_f] * 5 + [c_int, c_f, c_vp, c_vp]),
 }
 
 PREC_FP32, PREC_BF16 = 0, 1

@@ -10,7 +10,7 @@
 Each ``step()`` enqueues: student forward (activations kept in the plan), teacher/peer forward(s), ONE fused
 loss launch pair (value + dlogits), backward into a persistent flat gradient buffer, (data parallel: NCCL
 all-reduce of the gradient buckets on a side stream, overlapped with the rest of backward), and ONE fused
-SGD-momentum(+EMA) pass over the flat parameter buffers.  Nothing synchronises the host; the returned loss is
+SGD-momentum or Adam / AdamW (+EMA) pass over the flat parameter buffers.  Nothing synchronises the host; the returned loss is
 a device scalar.  Host-side schedules (Medical_LR, consistency ramp-up, EMA alpha) are python floats exactly as
 in the reference (utils/scheduler/medical_lr.py:13-17, utils/utils.py:67-86)."""
 import contextlib
@@ -85,9 +85,25 @@ def _input_noise(shape, like):
 class _StepBase:
     serialize = False             # profiling: every network on the calling stream, so per-category kernel times do not overlap
 
+    OPTIMIZERS = ("sgd", "adam", "adamw")
+
     def __init__(self, *, lr=0.01, momentum=0.9, weight_decay=1e-4, total_itrs=30000, consistency=0.1,
-                 consistency_rampup=200.0, process_group=None, exact_global=False):
+                 consistency_rampup=200.0, process_group=None, exact_global=False, optimizer="sgd", betas=(0.9, 0.999),
+                 eps=1e-8):
+        """optimizer: "sgd" (torch.optim.SGD with ``momentum``), "adam" (torch.optim.Adam: L2 weight decay) or "adamw"
+        (torch.optim.AdamW: decoupled weight decay) with ``betas`` / ``eps``, as the reference's optimiser factory builds
+        them (utils/__init__.py:13-49); ``weight_decay`` applies to all three."""
+        if optimizer not in self.OPTIMIZERS:
+            raise ValueError("optimizer must be one of %s, got %r" % (", ".join(self.OPTIMIZERS), optimizer))
         self.base_lr, self.momentum, self.weight_decay = lr, momentum, weight_decay
+        self.optimizer = optimizer
+        if optimizer != "sgd":
+            self.betas, self.eps = (float(betas[0]), float(betas[1])), float(eps)
+            cls = torch.optim.AdamW if optimizer == "adamw" else torch.optim.Adam
+            # the param_group keys and values the installed torch emits for these hyperparameters (checkpoint layout)
+            group = cls([torch.zeros(1, requires_grad=True)], lr=lr, betas=self.betas, eps=self.eps,
+                        weight_decay=weight_decay).state_dict()["param_groups"][0]
+            self._adam_group = {k: v for k, v in group.items() if k != "params"}
         self.total_itrs, self.consistency, self.consistency_rampup = total_itrs, consistency, consistency_rampup
         self.cur_itrs = 0
         self.pg = process_group
@@ -107,16 +123,23 @@ class _StepBase:
 
     def _setup(self, trained, networks, train=None, grads=True):
         """Construction shared by the drivers.  trained: the networks this driver optimises, in checkpoint order, each given a
-        flat momentum buffer and (unless autograd produces its gradients, grads=False) a flat gradient buffer; networks: every
+        flat optimiser state and (unless autograd produces its gradients, grads=False) a flat gradient buffer; networks: every
         network of the step, in the order of the checkpointed Philox offsets; train: the networks put in train() mode (default:
-        the trained ones).  Returns [(gradient buffer, momentum buffer)] in the order of ``trained``."""
+        the trained ones).  Returns [(gradient buffer, optimiser state)] in the order of ``trained``: the state is the
+        momentum buffer (SGD) or the pair (exp_avg, exp_avg_sq) (Adam / AdamW, with one step count per network in
+        ``_adam_steps``)."""
         self.in_channels, self.num_classes = trained[0].in_channels, trained[0].num_classes
         for m in trained if train is None else train:
             m.train()
         for m in networks:
             m.ensure_flat()
-        self._trained = [(m, torch.zeros_like(m.flat_params) if grads else None, torch.zeros_like(m.flat_params))
-                         for m in trained]
+
+        def state(m):
+            if self.optimizer == "sgd":
+                return torch.zeros_like(m.flat_params)
+            return torch.zeros_like(m.flat_params), torch.zeros_like(m.flat_params)
+        self._trained = [(m, torch.zeros_like(m.flat_params) if grads else None, state(m)) for m in trained]
+        self._adam_steps = [0] * len(trained)
         self._networks = list(networks)
         self._check_buffers()
         self._broadcast_from_rank0()
@@ -140,6 +163,17 @@ class _StepBase:
         if not enabled:
             self._ggraph = None
             self._gsig = None
+
+    def _next_iteration(self):
+        """Start of every step(): the iteration counter, the Adam step counts (every U-Net tensor gets a gradient every
+        iteration), and the buffer check."""
+        self.cur_itrs += 1
+        self._adam_steps = [t + 1 for t in self._adam_steps]
+        self._check_buffers()
+
+    @staticmethod
+    def _state_tensors(state):
+        return state if isinstance(state, tuple) else (state,)
 
     def _use_graph(self):
         dp_ok = self.world == 1 or self._graph_dp
@@ -184,7 +218,7 @@ class _StepBase:
         for m in models:
             m.ensure_flat(quick=True)
         ptrs = tuple((m.flat_params.data_ptr(), m.bn_running.data_ptr(), m.bn_counters.data_ptr(), id(m._plans)) for m in models)
-        ptrs += tuple(t.data_ptr() for _, g, b in self._trained for t in (g, b) if t is not None)
+        ptrs += tuple(t.data_ptr() for _, g, b in self._trained for t in (g,) + self._state_tensors(b) if t is not None)
         # (the dropout seed is a by-value launch argument: a re-seeded generator needs a new capture)
         ptrs += (torch.cuda.default_generators[dev.index if dev.index is not None else torch.cuda.current_device()].initial_seed(),)
         sig = tuple((tuple(t.shape), t.dtype) for t in inputs) + (len(dyn_f), len(fwd_models), ptrs)
@@ -247,8 +281,17 @@ class _StepBase:
     def state_dict(self):
         """{cur_itrs, philox offsets, optimizer}: `optimizer` holds torch.optim.SGD-style per-parameter momentum buffers
         (state[i]['momentum_buffer'] in model.parameters() order) so that a reference checkpoint's optimizer state and
-        this driver's flat momentum buffer interchange."""
+        this driver's flat momentum buffer interchange.  Adam / AdamW drivers use the torch.optim.Adam / AdamW layout
+        instead: state[i] = {step, exp_avg, exp_avg_sq}."""
         out = {"cur_itrs": self.cur_itrs, "philox": [m._philox_offset for m in self._networks], "optimizers": []}
+        if self.optimizer != "sgd":
+            for (model, _, (m, v)), t in zip(self._trained, self._adam_steps):
+                state = {i: self._adam_entry(t, m[o:o + n].view(shape), v[o:o + n].view(shape))
+                         for i, (o, n, shape) in enumerate(model._layout)} if t > 0 else {}
+                out["optimizers"].append({"state": state, "param_groups": [dict(
+                    self._adam_group, lr=medical_lr(self.cur_itrs + 1, self.base_lr, self.total_itrs),
+                    params=list(range(len(model._layout))))]})
+            return out
         for model, _, buf in self._trained:
             state = {i: {"momentum_buffer": buf[o:o + n].view(shape).clone()} for i, (o, n, shape) in enumerate(model._layout)}
             out["optimizers"].append({"state": state if self.cur_itrs > 0 else {},
@@ -257,10 +300,48 @@ class _StepBase:
                                                         "params": list(range(len(model._layout)))}]})
         return out
 
+    @staticmethod
+    def _adam_entry(t, m, v):
+        return {"step": torch.tensor(float(t), dtype=torch.float32), "exp_avg": m.clone(), "exp_avg_sq": v.clone()}
+
+    def _check_optimizer_kind(self, opt):
+        """A checkpoint of the other optimiser kind (SGD momentum vs Adam moments) cannot be resumed by this driver."""
+        adam = any("betas" in g for g in opt.get("param_groups", [])) or \
+            any("exp_avg" in st for st in opt.get("state", {}).values())
+        sgd = any("momentum_buffer" in st for st in opt.get("state", {}).values()) or \
+            any("momentum" in g and "betas" not in g for g in opt.get("param_groups", []))
+        if (adam and self.optimizer == "sgd") or (sgd and self.optimizer != "sgd"):
+            raise ValueError("the checkpoint holds %s optimiser state but this step driver uses optimizer=%r"
+                             % ("Adam" if adam else "SGD", self.optimizer))
+
+    @staticmethod
+    def _adam_checkpoint_step(k, model, opt):
+        """The one step count of the U-Net tensors of optimizer entry k (0: no state yet)."""
+        entries = [opt["state"].get(i) for i in range(len(model._layout))]
+        steps = {float(st["step"]) for st in entries if st is not None}
+        if len(steps) > 1 or (steps and any(st is None for st in entries)):
+            raise ValueError("the %d U-Net tensors of optimizer entry %d carry different Adam step counts (%s): one flat "
+                             "buffer keeps one step count" % (len(entries), k, sorted(steps)))
+        return int(steps.pop()) if steps else 0
+
     def load_state_dict(self, sd):
+        for opt in sd.get("optimizers", []):
+            self._check_optimizer_kind(opt)
+        if self.optimizer != "sgd":
+            steps = [self._adam_checkpoint_step(k, model, opt)
+                     for k, ((model, _, _), opt) in enumerate(zip(self._trained, sd.get("optimizers", [])))]
         self.cur_itrs = int(sd["cur_itrs"])
         for m, off in zip(self._networks, sd.get("philox", [])):
             m._philox_offset = int(off)
+        if self.optimizer != "sgd":
+            for k, ((model, _, (m, v)), opt, t) in enumerate(zip(self._trained, sd.get("optimizers", []), steps)):
+                m.zero_()
+                v.zero_()
+                self._adam_steps[k] = t
+                for i, (o, n, _) in enumerate(model._layout if t > 0 else ()):
+                    m[o:o + n].copy_(opt["state"][i]["exp_avg"].reshape(-1))
+                    v[o:o + n].copy_(opt["state"][i]["exp_avg_sq"].reshape(-1))
+            return
         for (model, _, buf), opt in zip(self._trained, sd.get("optimizers", [])):
             buf.zero_()
             for i, (o, n, shape) in enumerate(model._layout):
@@ -270,9 +351,10 @@ class _StepBase:
 
     def _check_buffers(self):
         """The flat gradient / momentum buffers must match the (possibly re-flattened or moved) parameter buffer."""
-        for model, *bufs in self._trained:
+        names = ("gradient", "momentum") if self.optimizer == "sgd" else ("gradient", "exp_avg", "exp_avg_sq")
+        for model, g, state in self._trained:
             flat = model.flat_params
-            for what, buf in zip(("gradient", "momentum"), bufs):
+            for what, buf in zip(names, (g,) + self._state_tensors(state)):
                 if buf is not None and (buf.device != flat.device or buf.numel() != flat.numel()):
                     raise L.HpfgError("step driver %s buffer (%s, %d) no longer matches the model's flat parameters (%s, %d): "
                                       "build the step driver after moving the model"
@@ -309,11 +391,37 @@ class _StepBase:
     def _lr(self):
         return medical_lr(self.cur_itrs, self.base_lr, self.total_itrs)
 
-    def _dyn_scalars(self, ema_decay=None):
+    def _dyn_scalars(self, ema_decay=None, *extra):
         """The device block: [lr, ema_alpha, 1 - ema_alpha (fp32 subtraction, as the by-value entry point), consistency
-        weight]; UAMT appends its threshold."""
+        weight, *extra (UAMT: its threshold)]; Adam / AdamW drivers end it with one group of ``_adam_scalars`` per trained
+        network, in the order of ``_trained``."""
         alpha = min(1 - 1 / (self.cur_itrs + 1), ema_decay) if ema_decay is not None else 0.0
-        return [self._lr(), alpha, float(1.0 - torch.tensor(alpha, dtype=torch.float32)), self._consistency_weight()]
+        one_minus = float(1.0 - torch.tensor(alpha, dtype=torch.float32))
+        out = [self._lr(), alpha, one_minus, self._consistency_weight(), *extra]
+        if self.optimizer != "sgd":
+            for t in self._adam_steps:
+                out += self._adam_scalars(t, self._lr()) + [alpha, one_minus]
+        return out
+
+    def _adam_scalars(self, t, lr):
+        """[step_size, bc2_sqrt, decay_factor] of Adam step t, in double as torch.optim.adam._multi_tensor_adam computes them
+        (bias corrections from the float step count) before they are cast to fp32."""
+        beta1, beta2 = self.betas
+        bias_correction1 = 1 - beta1 ** float(t)
+        bias_correction2 = 1 - beta2 ** float(t)
+        decay = 1 - lr * self.weight_decay if self.optimizer == "adamw" else 1.0
+        return [(lr / bias_correction1) * -1, bias_correction2 ** 0.5, decay]
+
+    def _adam(self, p, g, m, v, ema, n, scalars, dyn, st):
+        """One hpfg_adam(_dv) call: ``scalars`` = [step_size, bc2_sqrt, decay_factor, ema_alpha] by value, or ``dyn`` = the
+        device slice of the same five entries (with 1 - ema_alpha)."""
+        beta1, beta2 = self.betas
+        common = (p, g, m, v, ema, n, 1 - beta1, beta2, 1 - beta2, self.eps, self.weight_decay, int(self.optimizer == "adamw"),
+                  self._grad_scale)
+        if dyn is not None:
+            L.check(L.lib().hpfg_adam_dv(*common, L.ptr(dyn), st), "hpfg_adam_dv")
+        else:
+            L.check(L.lib().hpfg_adam(*common, *scalars, st), "hpfg_adam")
 
     @staticmethod
     def _dv_scalar(dv, i):
@@ -381,10 +489,18 @@ class _StepBase:
             w.wait()            # stream-level wait on the compute stream, not a host sync
 
     def _sgd(self, model, grads, buf, dv, ema_model=None):
-        """Fused SGD-momentum over the flat buffers, with the EMA of ``model`` into ``ema_model`` in the same pass if given.
-        Eager launches take this iteration's learning rate and EMA alpha by value; captures read {lr, alpha, 1 - alpha}
-        from the device block."""
+        """The optimiser step of ``model`` over the flat buffers (fused SGD-momentum, or Adam / AdamW with ``buf`` =
+        (exp_avg, exp_avg_sq)), with the EMA of ``model`` into ``ema_model`` in the same pass if given.  Eager launches take
+        this iteration's scalars by value; captures read them from the device block."""
         lib, n, st = L.lib(), model.flat_params.numel(), L.stream_ptr(grads.device)
+        if self.optimizer != "sgd":
+            k = next(i for i, (m, _, _) in enumerate(self._trained) if m is model)
+            alpha = min(1 - 1 / (self.cur_itrs + 1), self.ema_decay) if ema_model is not None else 0.0
+            dyn = None if dv is None else dv[0][dv[0].numel() - 5 * (len(self._trained) - k):][:5]
+            self._adam(L.ptr(model.flat_params), L.ptr(grads), L.ptr(buf[0]), L.ptr(buf[1]),
+                       None if ema_model is None else L.ptr(ema_model.flat_params), n,
+                       self._adam_scalars(self._adam_steps[k], self._lr()) + [alpha], dyn, st)
+            return
         p, g, m = L.ptr(model.flat_params), L.ptr(grads), L.ptr(buf)
         first = int(self.cur_itrs == 1)
         if dv is not None:
@@ -412,8 +528,7 @@ class MeanTeacherStep(_StepBase):
 
     def step(self, x, labels):
         """x: [n_l+n_u, C, H, W] fp32 CUDA (labeled slices first); labels: [n_l, H, W] int64 CUDA."""
-        self.cur_itrs += 1
-        self._check_buffers()
+        self._next_iteration()
         ins = [x, labels]
         out = (self._graph_replay(ins, self._dyn_scalars(self.ema_decay), [self.ema_model, self.model], self._body)
                if self._use_graph() else self._body(ins, None))
@@ -447,8 +562,7 @@ class CPSStep(_StepBase):
         (self.g1, self.b1), (self.g2, self.b2) = self._setup([model1, model2], [model1, model2])
 
     def step(self, x, labels):
-        self.cur_itrs += 1
-        self._check_buffers()
+        self._next_iteration()
         ins = [x, labels]
         out = (self._graph_replay(ins, self._dyn_scalars(), [self.m2, self.m1], self._body)
                if self._use_graph() else self._body(ins, None))
@@ -496,8 +610,7 @@ class UAMTStep(_StepBase):
         teacher_masks (parity harness only, eager launches): 1 + T//2 dropout keep-mask sets, one per teacher forward in call
         order (the consistency forward on n_u slices, then the T//2 Monte-Carlo forwards on 2*n_u slices) -- every
         stochastic teacher pass draws its own masks, as nn.Dropout does in the reference (2019_07...:134-143)."""
-        self.cur_itrs += 1
-        self._check_buffers()
+        self._next_iteration()
         x_u = x[labels.shape[0]:]
         if noise is None:
             noise = _input_noise(x_u.shape, x_u)
@@ -513,7 +626,7 @@ class UAMTStep(_StepBase):
         ins = [x, labels, noise, mc_noise.contiguous()]
         thr = self._threshold()
         if teacher_masks is None and self._use_graph():
-            out = self._graph_replay(ins, self._dyn_scalars(self.ema_decay) + [thr],
+            out = self._graph_replay(ins, self._dyn_scalars(self.ema_decay, thr),
                                      [self.ema_model] * (1 + self.T // 2) + [self.model], self._body)
         else:
             out = self._body(ins, None)
@@ -569,8 +682,7 @@ class ICTStep(_StepBase):
 
     def step(self, x, labels, mix_factors=None):
         """x: [n_l+n_u, C, H, W] (labeled first, n_u even); mix_factors: [n_u//2] floats (drawn here if None)."""
-        self.cur_itrs += 1
-        self._check_buffers()
+        self._next_iteration()
         n_u = x.shape[0] - labels.shape[0]
         assert n_u % 2 == 0, "ICT needs an even unlabeled batch"
         if mix_factors is None:
@@ -628,8 +740,7 @@ class S4CVStep(_StepBase):
 
     def step(self, x, labels, noise=None):
         """x: [n_l+n_u, C, H, W] (labeled first); labels: [n_l, H, W]; noise [n_u, ...]: drawn here if None."""
-        self.cur_itrs += 1
-        self._check_buffers()
+        self._next_iteration()
         n_l, dev = labels.shape[0], x.device
         x_u = x[n_l:]
         if noise is None:
@@ -676,6 +787,7 @@ class HPFGStep(_StepBase):
         from .losses import Dense_Loss
         self.m1, self.m2, self.ema_model, self.ema_decay, self.mt_start = model1, model2, ema_model, ema_decay, mt_start
         self._neck_mom = {}                         # id(parameter) -> momentum buffer of the neck tensors (outside the flat buffer)
+        self._neck_adam = {}                        # Adam / AdamW: id(parameter) -> [step count, exp_avg, exp_avg_sq]
         # the gradients come from autograd (model.last_flat_grad): momentum buffers only
         (_, self.b1), (_, self.b2) = self._setup([model1, model2], [model1, model2, ema_model], grads=False)
         for p in ema_model.parameters():
@@ -713,6 +825,12 @@ class HPFGStep(_StepBase):
             base = len(model._layout)
             necks = self._neck_params(model)
             opt["param_groups"][0]["params"] = list(range(base + len(necks)))
+            if self.optimizer != "sgd":
+                for j, p in enumerate(necks):
+                    st = self._neck_adam.get(id(p))
+                    if st is not None:
+                        opt["state"][base + j] = self._adam_entry(*st)
+                continue
             for j, p in enumerate(necks):
                 mom = self._neck_mom.get(id(p))
                 if mom is not None and self.cur_itrs > 0:
@@ -721,19 +839,39 @@ class HPFGStep(_StepBase):
 
     def load_state_dict(self, sd):
         super().load_state_dict(sd)
-        self._neck_mom = {}
+        self._neck_mom, self._neck_adam = {}, {}
         for model, opt in zip((m for m, _, _ in self._trained), sd.get("optimizers", [])):
             base = len(model._layout)
             for j, p in enumerate(self._neck_params(model)):
                 st = opt["state"].get(base + j)
+                if self.optimizer != "sgd":
+                    if st is not None:
+                        self._neck_adam[id(p)] = [int(float(st["step"]))] + [
+                            st[k].to(device=p.device, dtype=p.dtype).reshape(p.shape).clone() for k in ("exp_avg", "exp_avg_sq")]
+                    continue
                 if st is not None and st.get("momentum_buffer") is not None:
                     self._neck_mom[id(p)] = st["momentum_buffer"].to(device=p.device, dtype=p.dtype).reshape(p.shape).clone()
 
     def _sgd_model(self, model, buf, lr, first):
-        """torch.optim.SGD semantics over all parameters of a UNet_Plus: the flat U-Net buffer in one pass + the neck tensors."""
+        """torch.optim.SGD (or Adam / AdamW) semantics over all parameters of a UNet_Plus: the flat U-Net buffer in one pass +
+        the neck tensors."""
         st = L.stream_ptr(model.flat_params.device)
         lib = L.lib()
         g = model.last_flat_grad
+        if self.optimizer != "sgd":
+            k = next(i for i, (m, _, _) in enumerate(self._trained) if m is model)
+            self._adam(L.ptr(model.flat_params), L.ptr(g), L.ptr(buf[0]), L.ptr(buf[1]), None, model.flat_params.numel(),
+                       self._adam_scalars(self._adam_steps[k], lr) + [0.0], None, st)
+            for p in self._neck_params(model):
+                if p.grad is None:
+                    continue
+                # torch.optim.Adam: state (zero moments, step 0) is created the first time a tensor has a gradient, and
+                # each tensor counts its own steps
+                state = self._neck_adam.setdefault(id(p), [0, torch.zeros_like(p.data), torch.zeros_like(p.data)])
+                state[0] += 1
+                self._adam(L.ptr(p.data), L.ptr(p.grad.contiguous()), L.ptr(state[1]), L.ptr(state[2]), None, p.numel(),
+                           self._adam_scalars(state[0], lr) + [0.0], None, st)
+            return
         L.check(lib.hpfg_sgd_momentum(L.ptr(model.flat_params), L.ptr(g), L.ptr(buf), model.flat_params.numel(), lr, self.momentum,
                                       self.weight_decay, self._grad_scale, first, st), "hpfg_sgd_momentum")
         for p in self._neck_params(model):
@@ -752,8 +890,7 @@ class HPFGStep(_StepBase):
         cutmix_mask: the 0/1 box masks of BoxMaskGenerator (main.py:141-143)."""
         from .utils import update_ema_variables, ema_update_flat
         from .losses import ssl_loss_raw, dice_loss_raw, argmax_labels
-        self.cur_itrs += 1
-        self._check_buffers()
+        self._next_iteration()
         m1, m2, ema = self.m1, self.m2, self.ema_model
         label_bs, unlabel_bs = label_img.shape[0], img_unlabel.shape[0]
         rep = int(unlabel_bs // label_bs)

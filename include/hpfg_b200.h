@@ -8,6 +8,7 @@
  *   the inline consistency / pseudo-label terms of the MT / CPS / UAMT trainers    (hpfg_ssl_loss_*)
  *   utils/utils.py:82-86 update_ema_variables                                      (hpfg_ema_update)
  *   torch.optim.SGD as built by utils/__init__.py:14-16                            (hpfg_sgd_momentum*)
+ *   torch.optim.Adam / AdamW as built by utils/__init__.py:13-49 (+ update_ema_variables) (hpfg_adam*)
  *
  * Conventions: plain pointers and sizes only.  Every pointer is a DEVICE pointer unless its name ends in
  * _host.  All work is enqueued on the caller's stream (passed as void* == cudaStream_t); no call
@@ -113,8 +114,8 @@ int hpfg_unet_forward(hpfg_unet_plan_t plan, const float *params, float *bn_runn
 /* CUDA-graph friendly variants ("_dv": device values).  Scalars that change every iteration are read from device memory
  * at execution time instead of being baked into the launch, so a captured step can be replayed after updating a small
  * device block: the Philox offset of the dropout masks (hpfg_unet_forward_dv), the consistency weight
- * (hpfg_ssl_loss_dv: utils/utils.py:67-79 ramp-up), and {lr, ema_alpha, 1-ema_alpha} (hpfg_sgd_momentum_ema_dv:
- * utils/scheduler/medical_lr.py:13-17, utils/utils.py:84). */
+ * (hpfg_ssl_loss_dv: utils/utils.py:67-79 ramp-up), {lr, ema_alpha, 1-ema_alpha} (hpfg_sgd_momentum_ema_dv:
+ * utils/scheduler/medical_lr.py:13-17, utils/utils.py:84) and the per-step Adam scalars (hpfg_adam_dv). */
 int hpfg_unet_forward_dv(hpfg_unet_plan_t plan, const float *params, float *bn_running, int64_t *bn_counters,
                          const float *x, float *logits, int training, int no_dropout, int save_for_backward,
                          uint64_t dropout_seed, const uint64_t *dropout_offset_dev,
@@ -302,6 +303,22 @@ int hpfg_sgd_momentum_ema_dv(float *param, const float *grad, float *momentum_bu
 /* lr_dev: device float[1] = {lr} (the CPS networks have no EMA teacher). */
 int hpfg_sgd_momentum_dv(float *param, const float *grad, float *momentum_buf, int64_t n, float momentum,
                          float weight_decay, float grad_scale, int first_step, const float *lr_dev, void *stream);
+
+/* torch.optim.Adam (decoupled == 0: L2 weight decay added to the gradient) or torch.optim.AdamW (decoupled != 0:
+ * param *= decay_factor) step, foreach implementation, no amsgrad / maximize; with ema != NULL, followed in the same
+ * pass by update_ema_variables (utils/utils.py:82-86) of the updated parameters into ema.  The scalars are what torch
+ * computes in Python (double) and casts to fp32: one_minus_beta1 = 1 - beta1, one_minus_beta2 = 1 - beta2 (not
+ * recomputed from the fp32 betas), and per step t: step_size = -lr / (1 - beta1^t), bc2_sqrt = sqrt(1 - beta2^t),
+ * decay_factor = 1 - lr*weight_decay.  grad_scale multiplies the gradient first (1/world for DP).  The caller keeps
+ * the step count. */
+int hpfg_adam(float *param, const float *grad, float *exp_avg, float *exp_avg_sq, float *ema, int64_t n,
+              float one_minus_beta1, float beta2, float one_minus_beta2, float eps, float weight_decay, int decoupled,
+              float grad_scale, float step_size, float bc2_sqrt, float decay_factor, float ema_alpha, void *stream);
+
+/* dyn: device float[5] = {step_size, bc2_sqrt, decay_factor, ema_alpha, 1 - ema_alpha}. */
+int hpfg_adam_dv(float *param, const float *grad, float *exp_avg, float *exp_avg_sq, float *ema, int64_t n,
+                 float one_minus_beta1, float beta2, float one_minus_beta2, float eps, float weight_decay, int decoupled,
+                 float grad_scale, const float *dyn, void *stream);
 
 #ifdef __cplusplus
 }
