@@ -180,60 +180,50 @@ extern "C" int hpfg_ema_update(float *ema, const float *param, int64_t n, float 
     return HPFG_OK;
 }
 
+static int sgd_launch(const char *what, float *param, const float *grad, float *momentum_buf, float *ema, int64_t n,
+                      const SgdArgs &a, void *stream) {
+    HPFG_REQUIRE(param && grad && momentum_buf && n >= 0, std::string(what) + ": null buffer");
+    HPFG_REQUIRE(aligned16(param) && aligned16(grad) && aligned16(momentum_buf) && (!ema || aligned16(ema)),
+                 std::string(what) + ": buffers must be 16-byte aligned");
+    if (n == 0) return HPFG_OK;
+    ProfScope _prof(PROF_OPTIM, (cudaStream_t)stream);
+    if (ema)
+        HPFG_CUDA_CHECK(launch_pdl(sgd_kernel<true>, flat_grid(n), 256, 0, (cudaStream_t)stream, param, grad, momentum_buf, ema, n, a));
+    else
+        HPFG_CUDA_CHECK(launch_pdl(sgd_kernel<false>, flat_grid(n), 256, 0, (cudaStream_t)stream, param, grad, momentum_buf, (float *)nullptr, n, a));
+    HPFG_LAUNCH_CHECK();
+    return HPFG_OK;
+}
+
 extern "C" int hpfg_sgd_momentum(float *param, const float *grad, float *momentum_buf, int64_t n, float lr,
                                  float momentum, float weight_decay, float grad_scale, int first_step,
                                  void *stream) {
-    HPFG_REQUIRE(param && grad && momentum_buf && n >= 0, "hpfg_sgd_momentum: null buffer");
-    HPFG_REQUIRE(aligned16(param) && aligned16(grad) && aligned16(momentum_buf),
-                 "hpfg_sgd_momentum: buffers must be 16-byte aligned");
-    if (n == 0) return HPFG_OK;
-    ProfScope _prof(PROF_OPTIM, (cudaStream_t)stream);
     SgdArgs a{lr, momentum, weight_decay, grad_scale, 0.f, 0.f, first_step, nullptr};
-    HPFG_CUDA_CHECK(launch_pdl(sgd_kernel<false>, flat_grid(n), 256, 0, (cudaStream_t)stream, param, grad, momentum_buf, nullptr, n, a));
-    HPFG_LAUNCH_CHECK();
-    return HPFG_OK;
+    return sgd_launch("hpfg_sgd_momentum", param, grad, momentum_buf, nullptr, n, a, stream);
 }
 
 extern "C" int hpfg_sgd_momentum_ema(float *param, const float *grad, float *momentum_buf, float *ema, int64_t n,
                                      float lr, float momentum, float weight_decay, float grad_scale,
                                      int first_step, float ema_alpha, void *stream) {
-    HPFG_REQUIRE(param && grad && momentum_buf && ema && n >= 0, "hpfg_sgd_momentum_ema: null buffer");
-    HPFG_REQUIRE(aligned16(param) && aligned16(grad) && aligned16(momentum_buf) && aligned16(ema),
-                 "hpfg_sgd_momentum_ema: buffers must be 16-byte aligned");
-    if (n == 0) return HPFG_OK;
-    ProfScope _prof(PROF_OPTIM, (cudaStream_t)stream);
+    HPFG_REQUIRE(ema, "hpfg_sgd_momentum_ema: null buffer");
     SgdArgs a{lr, momentum, weight_decay, grad_scale, ema_alpha, 1.0f - ema_alpha, first_step, nullptr};
-    HPFG_CUDA_CHECK(launch_pdl(sgd_kernel<true>, flat_grid(n), 256, 0, (cudaStream_t)stream, param, grad, momentum_buf, ema, n, a));
-    HPFG_LAUNCH_CHECK();
-    return HPFG_OK;
+    return sgd_launch("hpfg_sgd_momentum_ema", param, grad, momentum_buf, ema, n, a, stream);
 }
 
 extern "C" int hpfg_sgd_momentum_ema_dv(float *param, const float *grad, float *momentum_buf, float *ema, int64_t n,
                                         float momentum, float weight_decay, float grad_scale, int first_step,
                                         const float *lr_alpha_dev, void *stream) {
-    HPFG_REQUIRE(param && grad && momentum_buf && ema && lr_alpha_dev && n >= 0, "hpfg_sgd_momentum_ema_dv: null buffer");
-    HPFG_REQUIRE(aligned16(param) && aligned16(grad) && aligned16(momentum_buf) && aligned16(ema),
-                 "hpfg_sgd_momentum_ema_dv: buffers must be 16-byte aligned");
-    if (n == 0) return HPFG_OK;
-    ProfScope _prof(PROF_OPTIM, (cudaStream_t)stream);
+    HPFG_REQUIRE(ema && lr_alpha_dev, "hpfg_sgd_momentum_ema_dv: null buffer");
     SgdArgs a{0.f, momentum, weight_decay, grad_scale, 0.f, 0.f, first_step, lr_alpha_dev};
-    HPFG_CUDA_CHECK(launch_pdl(sgd_kernel<true>, flat_grid(n), 256, 0, (cudaStream_t)stream, param, grad, momentum_buf, ema, n, a));
-    HPFG_LAUNCH_CHECK();
-    return HPFG_OK;
+    return sgd_launch("hpfg_sgd_momentum_ema_dv", param, grad, momentum_buf, ema, n, a, stream);
 }
 
 extern "C" int hpfg_sgd_momentum_dv(float *param, const float *grad, float *momentum_buf, int64_t n, float momentum,
                                     float weight_decay, float grad_scale, int first_step, const float *lr_dev,
                                     void *stream) {
-    HPFG_REQUIRE(param && grad && momentum_buf && lr_dev && n >= 0, "hpfg_sgd_momentum_dv: null buffer");
-    HPFG_REQUIRE(aligned16(param) && aligned16(grad) && aligned16(momentum_buf),
-                 "hpfg_sgd_momentum_dv: buffers must be 16-byte aligned");
-    if (n == 0) return HPFG_OK;
-    ProfScope _prof(PROF_OPTIM, (cudaStream_t)stream);
+    HPFG_REQUIRE(lr_dev, "hpfg_sgd_momentum_dv: null buffer");
     SgdArgs a{0.f, momentum, weight_decay, grad_scale, 0.f, 0.f, first_step, lr_dev};
-    HPFG_CUDA_CHECK(launch_pdl(sgd_kernel<false>, flat_grid(n), 256, 0, (cudaStream_t)stream, param, grad, momentum_buf, nullptr, n, a));
-    HPFG_LAUNCH_CHECK();
-    return HPFG_OK;
+    return sgd_launch("hpfg_sgd_momentum_dv", param, grad, momentum_buf, nullptr, n, a, stream);
 }
 
 static int adam_launch(const char *what, float *param, const float *grad, float *exp_avg, float *exp_avg_sq, float *ema,

@@ -19,6 +19,7 @@ import math
 import torch
 
 from . import _lib as L
+from .optim import SGD, Adam
 from .losses import ssl_loss_raw, ict_loss_raw, ict_mix_inputs, s4cv_loss_raw
 from .utils import sigmoid_rampup, linear_rampup
 
@@ -85,7 +86,7 @@ def _input_noise(shape, like):
 class _StepBase:
     serialize = False             # profiling: every network on the calling stream, so per-category kernel times do not overlap
 
-    OPTIMIZERS = ("sgd", "adam", "adamw")
+    OPTIMIZERS = {"sgd": SGD, "adam": Adam, "adamw": Adam}
 
     def __init__(self, *, lr=0.01, momentum=0.9, weight_decay=1e-4, total_itrs=30000, consistency=0.1,
                  consistency_rampup=200.0, process_group=None, exact_global=False, optimizer="sgd", betas=(0.9, 0.999),
@@ -97,13 +98,6 @@ class _StepBase:
             raise ValueError("optimizer must be one of %s, got %r" % (", ".join(self.OPTIMIZERS), optimizer))
         self.base_lr, self.momentum, self.weight_decay = lr, momentum, weight_decay
         self.optimizer = optimizer
-        if optimizer != "sgd":
-            self.betas, self.eps = (float(betas[0]), float(betas[1])), float(eps)
-            cls = torch.optim.AdamW if optimizer == "adamw" else torch.optim.Adam
-            # the param_group keys and values the installed torch emits for these hyperparameters (checkpoint layout)
-            group = cls([torch.zeros(1, requires_grad=True)], lr=lr, betas=self.betas, eps=self.eps,
-                        weight_decay=weight_decay).state_dict()["param_groups"][0]
-            self._adam_group = {k: v for k, v in group.items() if k != "params"}
         self.total_itrs, self.consistency, self.consistency_rampup = total_itrs, consistency, consistency_rampup
         self.cur_itrs = 0
         self.pg = process_group
@@ -120,30 +114,26 @@ class _StepBase:
         self._grad_scale = 1.0 if self.exact_global else 1.0 / self.world
         if self.exact_global:
             L.install_allreduce_hook(self.pg)
+        self._opt = self.OPTIMIZERS[optimizer](optimizer, lr, momentum, weight_decay, betas, eps, self._grad_scale)
+        self._neck_states = {}      # id(parameter) -> OptState of the parameters outside the flat buffers (_neck_params)
 
     def _setup(self, trained, networks, train=None, grads=True):
         """Construction shared by the drivers.  trained: the networks this driver optimises, in checkpoint order, each given a
         flat optimiser state and (unless autograd produces its gradients, grads=False) a flat gradient buffer; networks: every
         network of the step, in the order of the checkpointed Philox offsets; train: the networks put in train() mode (default:
-        the trained ones).  Returns [(gradient buffer, optimiser state)] in the order of ``trained``: the state is the
-        momentum buffer (SGD) or the pair (exp_avg, exp_avg_sq) (Adam / AdamW, with one step count per network in
-        ``_adam_steps``)."""
+        the trained ones).  Returns [(gradient buffer, optimiser buffers)] in the order of ``trained``: the momentum buffer
+        (SGD) or the pair (exp_avg, exp_avg_sq) (Adam / AdamW)."""
         self.in_channels, self.num_classes = trained[0].in_channels, trained[0].num_classes
         for m in trained if train is None else train:
             m.train()
         for m in networks:
             m.ensure_flat()
-
-        def state(m):
-            if self.optimizer == "sgd":
-                return torch.zeros_like(m.flat_params)
-            return torch.zeros_like(m.flat_params), torch.zeros_like(m.flat_params)
-        self._trained = [(m, torch.zeros_like(m.flat_params) if grads else None, state(m)) for m in trained]
-        self._adam_steps = [0] * len(trained)
+        self._trained = [(m, torch.zeros_like(m.flat_params) if grads else None, self._opt.new_state(m.flat_params))
+                         for m in trained]
         self._networks = list(networks)
         self._check_buffers()
         self._broadcast_from_rank0()
-        return [(g, b) for _, g, b in self._trained]
+        return [(g, s.bufs[0] if len(s.bufs) == 1 else s.bufs) for _, g, s in self._trained]
 
     # ------------------------------------------------------------------ CUDA-graph replay of the whole step
     _graph_enabled = False
@@ -165,15 +155,12 @@ class _StepBase:
             self._gsig = None
 
     def _next_iteration(self):
-        """Start of every step(): the iteration counter, the Adam step counts (every U-Net tensor gets a gradient every
-        iteration), and the buffer check."""
+        """Start of every step(): the iteration counter, the step counts of the flat optimiser states (every U-Net tensor
+        gets a gradient every iteration; advanced on the host, so that graph replays see them move), and the buffer check."""
         self.cur_itrs += 1
-        self._adam_steps = [t + 1 for t in self._adam_steps]
+        for _, _, state in self._trained:
+            state.step += 1
         self._check_buffers()
-
-    @staticmethod
-    def _state_tensors(state):
-        return state if isinstance(state, tuple) else (state,)
 
     def _use_graph(self):
         dp_ok = self.world == 1 or self._graph_dp
@@ -218,7 +205,7 @@ class _StepBase:
         for m in models:
             m.ensure_flat(quick=True)
         ptrs = tuple((m.flat_params.data_ptr(), m.bn_running.data_ptr(), m.bn_counters.data_ptr(), id(m._plans)) for m in models)
-        ptrs += tuple(t.data_ptr() for _, g, b in self._trained for t in (g,) + self._state_tensors(b) if t is not None)
+        ptrs += tuple(t.data_ptr() for _, g, s in self._trained for t in (g,) + s.bufs if t is not None)
         # (the dropout seed is a by-value launch argument: a re-seeded generator needs a new capture)
         ptrs += (torch.cuda.default_generators[dev.index if dev.index is not None else torch.cuda.current_device()].initial_seed(),)
         sig = tuple((tuple(t.shape), t.dtype) for t in inputs) + (len(dyn_f), len(fwd_models), ptrs)
@@ -279,84 +266,57 @@ class _StepBase:
 
     # ------------------------------------------------------------------ checkpoint / resume (2017_03...:126-133)
     def state_dict(self):
-        """{cur_itrs, philox offsets, optimizer}: `optimizer` holds torch.optim.SGD-style per-parameter momentum buffers
-        (state[i]['momentum_buffer'] in model.parameters() order) so that a reference checkpoint's optimizer state and
-        this driver's flat momentum buffer interchange.  Adam / AdamW drivers use the torch.optim.Adam / AdamW layout
-        instead: state[i] = {step, exp_avg, exp_avg_sq}."""
+        """{cur_itrs, philox offsets, optimizer}: `optimizer` holds one torch.optim state dict per trained network, its
+        per-parameter state in model.parameters() order (the flat buffer's tensors, then the ones outside it) so that a
+        reference checkpoint's optimizer state and this driver's flat buffers interchange: state[i] = {momentum_buffer}
+        (torch.optim.SGD) or {step, exp_avg, exp_avg_sq} (torch.optim.Adam / AdamW).  SGD state appears from the first
+        iteration on, Adam state once it has taken a step; tensors that never received a gradient have none, as in torch."""
         out = {"cur_itrs": self.cur_itrs, "philox": [m._philox_offset for m in self._networks], "optimizers": []}
-        if self.optimizer != "sgd":
-            for (model, _, (m, v)), t in zip(self._trained, self._adam_steps):
-                state = {i: self._adam_entry(t, m[o:o + n].view(shape), v[o:o + n].view(shape))
-                         for i, (o, n, shape) in enumerate(model._layout)} if t > 0 else {}
-                out["optimizers"].append({"state": state, "param_groups": [dict(
-                    self._adam_group, lr=medical_lr(self.cur_itrs + 1, self.base_lr, self.total_itrs),
-                    params=list(range(len(model._layout))))]})
-            return out
-        for model, _, buf in self._trained:
-            state = {i: {"momentum_buffer": buf[o:o + n].view(shape).clone()} for i, (o, n, shape) in enumerate(model._layout)}
-            out["optimizers"].append({"state": state if self.cur_itrs > 0 else {},
-                                      "param_groups": [{"lr": medical_lr(self.cur_itrs + 1, self.base_lr, self.total_itrs),
-                                                        "momentum": self.momentum, "weight_decay": self.weight_decay,
-                                                        "params": list(range(len(model._layout)))}]})
+        lr = medical_lr(self.cur_itrs + 1, self.base_lr, self.total_itrs)
+        for model, _, state in self._trained:
+            entries = {i: self._opt.entry(state.step, [b[o:o + n].view(shape) for b in state.bufs])
+                       for i, (o, n, shape) in enumerate(model._layout)} if self._opt.has_state(state, self.cur_itrs) else {}
+            necks = self._neck_params(model)
+            for j, p in enumerate(necks):
+                s = self._neck_states.get(id(p))
+                if s is not None and self._opt.has_state(s, self.cur_itrs):
+                    entries[len(model._layout) + j] = self._opt.entry(s.step, s.bufs)
+            out["optimizers"].append({"state": entries,
+                                      "param_groups": [self._opt.param_group(lr, len(model._layout) + len(necks))]})
         return out
 
-    @staticmethod
-    def _adam_entry(t, m, v):
-        return {"step": torch.tensor(float(t), dtype=torch.float32), "exp_avg": m.clone(), "exp_avg_sq": v.clone()}
-
-    def _check_optimizer_kind(self, opt):
-        """A checkpoint of the other optimiser kind (SGD momentum vs Adam moments) cannot be resumed by this driver."""
-        adam = any("betas" in g for g in opt.get("param_groups", [])) or \
-            any("exp_avg" in st for st in opt.get("state", {}).values())
-        sgd = any("momentum_buffer" in st for st in opt.get("state", {}).values()) or \
-            any("momentum" in g and "betas" not in g for g in opt.get("param_groups", []))
-        if (adam and self.optimizer == "sgd") or (sgd and self.optimizer != "sgd"):
-            raise ValueError("the checkpoint holds %s optimiser state but this step driver uses optimizer=%r"
-                             % ("Adam" if adam else "SGD", self.optimizer))
-
-    @staticmethod
-    def _adam_checkpoint_step(k, model, opt):
-        """The one step count of the U-Net tensors of optimizer entry k (0: no state yet)."""
-        entries = [opt["state"].get(i) for i in range(len(model._layout))]
-        steps = {float(st["step"]) for st in entries if st is not None}
-        if len(steps) > 1 or (steps and any(st is None for st in entries)):
-            raise ValueError("the %d U-Net tensors of optimizer entry %d carry different Adam step counts (%s): one flat "
-                             "buffer keeps one step count" % (len(entries), k, sorted(steps)))
-        return int(steps.pop()) if steps else 0
-
     def load_state_dict(self, sd):
-        for opt in sd.get("optimizers", []):
-            self._check_optimizer_kind(opt)
-        if self.optimizer != "sgd":
-            steps = [self._adam_checkpoint_step(k, model, opt)
-                     for k, ((model, _, _), opt) in enumerate(zip(self._trained, sd.get("optimizers", [])))]
-        self.cur_itrs = int(sd["cur_itrs"])
+        """Everything is checked before anything changes: a checkpoint of the other optimiser kind, or one whose U-Net tensors
+        carry different Adam step counts, raises and leaves the driver as it was."""
+        cur_itrs, opts = int(sd["cur_itrs"]), sd.get("optimizers", [])
+        for opt in opts:
+            self._opt.check_kind(opt)
+        steps = [self._opt.checkpoint_step([opt["state"].get(i) for i in range(len(model._layout))], k, cur_itrs)
+                 for k, ((model, _, _), opt) in enumerate(zip(self._trained, opts))]
+        self.cur_itrs = cur_itrs
         for m, off in zip(self._networks, sd.get("philox", [])):
             m._philox_offset = int(off)
-        if self.optimizer != "sgd":
-            for k, ((model, _, (m, v)), opt, t) in enumerate(zip(self._trained, sd.get("optimizers", []), steps)):
-                m.zero_()
-                v.zero_()
-                self._adam_steps[k] = t
-                for i, (o, n, _) in enumerate(model._layout if t > 0 else ()):
-                    m[o:o + n].copy_(opt["state"][i]["exp_avg"].reshape(-1))
-                    v[o:o + n].copy_(opt["state"][i]["exp_avg_sq"].reshape(-1))
-            return
-        for (model, _, buf), opt in zip(self._trained, sd.get("optimizers", [])):
-            buf.zero_()
-            for i, (o, n, shape) in enumerate(model._layout):
-                st = opt["state"].get(i)
-                if st is not None and st.get("momentum_buffer") is not None:
-                    buf[o:o + n].copy_(st["momentum_buffer"].reshape(-1))
+        self._neck_states = {}
+        for k, ((model, _, state), opt, step) in enumerate(zip(self._trained, opts, steps)):
+            state.step = step
+            for b in state.bufs:
+                b.zero_()
+            for i, (o, n, _) in enumerate(model._layout):
+                self._opt.load_entry(opt["state"].get(i), [b[o:o + n] for b in state.bufs])
+            for j, p in enumerate(self._neck_params(model)):
+                st = opt["state"].get(len(model._layout) + j)
+                if st is not None and all(st.get(key) is not None for key in self._opt.KEYS):
+                    s = self._neck_states[id(p)] = self._opt.new_state(p.data)
+                    s.step = self._opt.checkpoint_step([st], k, cur_itrs)
+                    self._opt.load_entry(st, s.bufs)
 
     def _check_buffers(self):
-        """The flat gradient / momentum buffers must match the (possibly re-flattened or moved) parameter buffer."""
-        names = ("gradient", "momentum") if self.optimizer == "sgd" else ("gradient", "exp_avg", "exp_avg_sq")
+        """The flat gradient / optimiser buffers must match the (possibly re-flattened or moved) parameter buffer."""
         for model, g, state in self._trained:
             flat = model.flat_params
-            for what, buf in zip(names, (g,) + self._state_tensors(state)):
+            for what, buf in zip(("gradient",) + self._opt.KEYS, (g,) + state.bufs):
                 if buf is not None and (buf.device != flat.device or buf.numel() != flat.numel()):
-                    raise L.HpfgError("step driver %s buffer (%s, %d) no longer matches the model's flat parameters (%s, %d): "
+                    raise L.HpfgError("step driver buffer %s (%s, %d) no longer matches the model's flat parameters (%s, %d): "
                                       "build the step driver after moving the model"
                                       % (what, buf.device, buf.numel(), flat.device, flat.numel()))
             if flat.is_cuda and flat.device.index != torch.cuda.current_device():
@@ -364,14 +324,22 @@ class _StepBase:
                                   "(the library launches on the current device)" % (flat.device, torch.cuda.current_device()))
 
     def _broadcast_from_rank0(self):
-        """Data parallel: every rank starts from rank 0's parameters / BN buffers (what DDP does at construction)."""
+        """Data parallel: every rank starts from rank 0's parameters / BN buffers (what DDP does at construction), the
+        tensors outside the flat buffers included."""
         if self.world <= 1:
             return
         import torch.distributed as dist
         for m in self._networks:
             m.ensure_flat()
-            for t in (m.flat_params, m.bn_running, m.bn_counters):
+            for t in (m.flat_params, m.bn_running, m.bn_counters, *(p.data for p in self._neck_params(m))):
                 dist.broadcast(t, src=dist.get_global_rank(self.pg, 0) if self.pg is not None else 0, group=self.pg)
+
+    @staticmethod
+    def _neck_params(model):
+        """The parameters of ``model`` outside its flat buffer, in parameters() order (a UNet_Plus: its 16 projection-neck
+        tensors after the 82 U-Net tensors; a UNet: none).  Each gets an optimiser state when it first has a gradient."""
+        core = {id(q) for q in model._flat_params_list}
+        return [p for p in model.parameters() if id(p) not in core]
 
     # Two forwards enqueued on two streams share the machine: half of the SMs each (hpfg_unet_plan_set_forward_ctas).  Only the
     # drivers whose two streams carry about the same forward work do this (Mean-Teacher, CPS, ICT); with unbalanced streams
@@ -393,35 +361,17 @@ class _StepBase:
 
     def _dyn_scalars(self, ema_decay=None, *extra):
         """The device block: [lr, ema_alpha, 1 - ema_alpha (fp32 subtraction, as the by-value entry point), consistency
-        weight, *extra (UAMT: its threshold)]; Adam / AdamW drivers end it with one group of ``_adam_scalars`` per trained
-        network, in the order of ``_trained``."""
+        weight, *extra (UAMT: its threshold)], then the optimiser's group of each trained network in the order of ``_trained``
+        (SGD: none; Adam / AdamW: [step_size, bc2_sqrt, decay_factor, ema_alpha, 1 - ema_alpha]), whose offset its state
+        records."""
         alpha = min(1 - 1 / (self.cur_itrs + 1), ema_decay) if ema_decay is not None else 0.0
         one_minus = float(1.0 - torch.tensor(alpha, dtype=torch.float32))
-        out = [self._lr(), alpha, one_minus, self._consistency_weight(), *extra]
-        if self.optimizer != "sgd":
-            for t in self._adam_steps:
-                out += self._adam_scalars(t, self._lr()) + [alpha, one_minus]
+        lr = self._lr()
+        out = [lr, alpha, one_minus, self._consistency_weight(), *extra]
+        for _, _, state in self._trained:
+            state.dv_offset = len(out)
+            out += self._opt.device_group(state.step, lr, alpha, one_minus)
         return out
-
-    def _adam_scalars(self, t, lr):
-        """[step_size, bc2_sqrt, decay_factor] of Adam step t, in double as torch.optim.adam._multi_tensor_adam computes them
-        (bias corrections from the float step count) before they are cast to fp32."""
-        beta1, beta2 = self.betas
-        bias_correction1 = 1 - beta1 ** float(t)
-        bias_correction2 = 1 - beta2 ** float(t)
-        decay = 1 - lr * self.weight_decay if self.optimizer == "adamw" else 1.0
-        return [(lr / bias_correction1) * -1, bias_correction2 ** 0.5, decay]
-
-    def _adam(self, p, g, m, v, ema, n, scalars, dyn, st):
-        """One hpfg_adam(_dv) call: ``scalars`` = [step_size, bc2_sqrt, decay_factor, ema_alpha] by value, or ``dyn`` = the
-        device slice of the same five entries (with 1 - ema_alpha)."""
-        beta1, beta2 = self.betas
-        common = (p, g, m, v, ema, n, 1 - beta1, beta2, 1 - beta2, self.eps, self.weight_decay, int(self.optimizer == "adamw"),
-                  self._grad_scale)
-        if dyn is not None:
-            L.check(L.lib().hpfg_adam_dv(*common, L.ptr(dyn), st), "hpfg_adam_dv")
-        else:
-            L.check(L.lib().hpfg_adam(*common, *scalars, st), "hpfg_adam")
 
     @staticmethod
     def _dv_scalar(dv, i):
@@ -488,35 +438,14 @@ class _StepBase:
         for w in works:
             w.wait()            # stream-level wait on the compute stream, not a host sync
 
-    def _sgd(self, model, grads, buf, dv, ema_model=None):
-        """The optimiser step of ``model`` over the flat buffers (fused SGD-momentum, or Adam / AdamW with ``buf`` =
-        (exp_avg, exp_avg_sq)), with the EMA of ``model`` into ``ema_model`` in the same pass if given.  Eager launches take
-        this iteration's scalars by value; captures read them from the device block."""
-        lib, n, st = L.lib(), model.flat_params.numel(), L.stream_ptr(grads.device)
-        if self.optimizer != "sgd":
-            k = next(i for i, (m, _, _) in enumerate(self._trained) if m is model)
-            alpha = min(1 - 1 / (self.cur_itrs + 1), self.ema_decay) if ema_model is not None else 0.0
-            dyn = None if dv is None else dv[0][dv[0].numel() - 5 * (len(self._trained) - k):][:5]
-            self._adam(L.ptr(model.flat_params), L.ptr(grads), L.ptr(buf[0]), L.ptr(buf[1]),
-                       None if ema_model is None else L.ptr(ema_model.flat_params), n,
-                       self._adam_scalars(self._adam_steps[k], self._lr()) + [alpha], dyn, st)
-            return
-        p, g, m = L.ptr(model.flat_params), L.ptr(grads), L.ptr(buf)
-        first = int(self.cur_itrs == 1)
-        if dv is not None:
-            if ema_model is None:
-                L.check(lib.hpfg_sgd_momentum_dv(p, g, m, n, self.momentum, self.weight_decay, self._grad_scale, first,
-                                                 L.ptr(dv[0]), st), "hpfg_sgd_momentum_dv")
-            else:
-                L.check(lib.hpfg_sgd_momentum_ema_dv(p, g, m, L.ptr(ema_model.flat_params), n, self.momentum, self.weight_decay,
-                                                     self._grad_scale, first, L.ptr(dv[0]), st), "hpfg_sgd_momentum_ema_dv")
-        elif ema_model is None:
-            L.check(lib.hpfg_sgd_momentum(p, g, m, n, self._lr(), self.momentum, self.weight_decay, self._grad_scale, first, st),
-                    "hpfg_sgd_momentum")
-        else:
-            alpha = min(1 - 1 / (self.cur_itrs + 1), self.ema_decay)      # utils/utils.py:84
-            L.check(lib.hpfg_sgd_momentum_ema(p, g, m, L.ptr(ema_model.flat_params), n, self._lr(), self.momentum,
-                                              self.weight_decay, self._grad_scale, first, alpha, st), "hpfg_sgd_momentum_ema")
+    def _opt_step(self, trained, dv, ema_model=None):
+        """The optimiser step of one ``_trained`` entry (network, gradient buffer, optimiser state) over its flat buffers, with
+        the EMA of the network into ``ema_model`` in the same pass if given.  Eager launches take this iteration's scalars by
+        value; captures read them from the device block."""
+        model, grads, state = trained
+        alpha = min(1 - 1 / (self.cur_itrs + 1), self.ema_decay) if ema_model is not None else 0.0      # utils/utils.py:84
+        self._opt.launch(model.flat_params, grads, state, None if ema_model is None else ema_model.flat_params, self._lr(),
+                         alpha, None if dv is None else dv[0], L.stream_ptr(grads.device))
 
 
 class MeanTeacherStep(_StepBase):
@@ -551,7 +480,7 @@ class MeanTeacherStep(_StepBase):
             r = ssl_loss_raw(L.LOSS_MT, out, t_out[n_l:], labels, n_l, cons_weight=w, cons_weight_dev=self._dv_scalar(dv, 3))
         self._global_consistency_value(r["scalars"], w)
         self._backward(self.model, plan, r["dstudent"], self.grads)
-        self._sgd(self.model, self.grads, self.mom, dv, self.ema_model)
+        self._opt_step(self._trained[0], dv, self.ema_model)
         return dict(scalars=r["scalars"], logits=out, teacher_logits=t_out)
 
 
@@ -586,9 +515,9 @@ class CPSStep(_StepBase):
         side.wait_stream(main)
         with torch.cuda.stream(side):
             self._backward(self.m2, p2, r["dother"], self.g2)
-            self._sgd(self.m2, self.g2, self.b2, dv)
+            self._opt_step(self._trained[1], dv)
         self._backward(self.m1, p1, r["dstudent"], self.g1)
-        self._sgd(self.m1, self.g1, self.b1, dv)
+        self._opt_step(self._trained[0], dv)
         main.wait_stream(side)
         return dict(scalars=r["scalars"], logits1=o1, logits2=o2)
 
@@ -660,7 +589,7 @@ class UAMTStep(_StepBase):
                              uamt_threshold=self._threshold(), cons_weight_dev=self._dv_scalar(dv, 3),
                              uamt_threshold_dev=self._dv_scalar(dv, 4))
         self._backward(self.model, plan, r["dstudent"], self.grads)
-        self._sgd(self.model, self.grads, self.mom, dv, self.ema_model)
+        self._opt_step(self._trained[0], dv, self.ema_model)
         return dict(scalars=r["scalars"], logits=out, teacher_logits=t_out, mc_logits=mc)
 
 
@@ -716,7 +645,7 @@ class ICTStep(_StepBase):
             r = ict_loss_raw(out, t_out, lam, labels, n_l, cons_weight=w, cons_weight_dev=self._dv_scalar(dv, 3))
         self._global_consistency_value(r["scalars"], w)
         self._backward(self.model, plan, r["dstudent"], self.grads)
-        self._sgd(self.model, self.grads, self.mom, dv, self.ema_model)
+        self._opt_step(self._trained[0], dv, self.ema_model)
         return dict(scalars=r["scalars"], logits=out, teacher_logits=t_out)
 
 
@@ -761,9 +690,9 @@ class S4CVStep(_StepBase):
         side.wait_stream(main)
         with torch.cuda.stream(side):
             self._backward(self.m2, p2, r["dother"], self.g2)
-            self._sgd(self.m2, self.g2, self.b2, None, self.ema_model)      # SGD of student 2 + EMA into its teacher, one pass
+            self._opt_step(self._trained[1], None, self.ema_model)      # student 2 + EMA into its teacher, one pass
         self._backward(self.m1, p1, r["dstudent"], self.g1)
-        self._sgd(self.m1, self.g1, self.b1, None)
+        self._opt_step(self._trained[0], None)
         main.wait_stream(side)
         self.last = dict(scalars=r["scalars"], lr=self._lr(), w=w, logits1=o1, logits2=o2, teacher_logits=t_out)
         return r["scalars"][0]
@@ -786,9 +715,7 @@ class HPFGStep(_StepBase):
         super().__init__(**kw)
         from .losses import Dense_Loss
         self.m1, self.m2, self.ema_model, self.ema_decay, self.mt_start = model1, model2, ema_model, ema_decay, mt_start
-        self._neck_mom = {}                         # id(parameter) -> momentum buffer of the neck tensors (outside the flat buffer)
-        self._neck_adam = {}                        # Adam / AdamW: id(parameter) -> [step count, exp_avg, exp_avg_sq]
-        # the gradients come from autograd (model.last_flat_grad): momentum buffers only
+        # the gradients come from autograd (model.last_flat_grad): optimiser state only
         (_, self.b1), (_, self.b2) = self._setup([model1, model2], [model1, model2, ema_model], grads=False)
         for p in ema_model.parameters():
             p.requires_grad = False
@@ -799,91 +726,21 @@ class HPFGStep(_StepBase):
     def _consistency_weight(self):
         return self.consistency * linear_rampup(self.cur_itrs // 150, self.consistency_rampup)
 
-    def _broadcast_from_rank0(self):
-        """The flat buffers as in ``_StepBase``, plus the neck tensors (they live outside the flat buffer)."""
-        super()._broadcast_from_rank0()
-        if self.world <= 1:
-            return
-        import torch.distributed as dist
-        src = dist.get_global_rank(self.pg, 0) if self.pg is not None else 0
-        for m in self._networks:
-            for p in self._neck_params(m):
-                dist.broadcast(p.data, src=src, group=self.pg)
-
-    @staticmethod
-    def _neck_params(model):
-        """The 16 projection-neck tensors of a UNet_Plus: parameters() order after the 82 U-Net tensors of the flat buffer."""
-        core = {id(q) for q in model._flat_params_list}
-        return [p for p in model.parameters() if id(p) not in core]
-
-    def state_dict(self):
-        """As ``_StepBase.state_dict``, with the neck tensors' momentum buffers at their torch.optim.SGD indices (82..97 of
-        ``model.parameters()``); tensors that never received a gradient (model1's necks: main.py:148 drops their outputs) have
-        no state, as in torch."""
-        out = super().state_dict()
-        for model, opt in zip((m for m, _, _ in self._trained), out["optimizers"]):
-            base = len(model._layout)
-            necks = self._neck_params(model)
-            opt["param_groups"][0]["params"] = list(range(base + len(necks)))
-            if self.optimizer != "sgd":
-                for j, p in enumerate(necks):
-                    st = self._neck_adam.get(id(p))
-                    if st is not None:
-                        opt["state"][base + j] = self._adam_entry(*st)
-                continue
-            for j, p in enumerate(necks):
-                mom = self._neck_mom.get(id(p))
-                if mom is not None and self.cur_itrs > 0:
-                    opt["state"][base + j] = {"momentum_buffer": mom.clone()}
-        return out
-
-    def load_state_dict(self, sd):
-        super().load_state_dict(sd)
-        self._neck_mom, self._neck_adam = {}, {}
-        for model, opt in zip((m for m, _, _ in self._trained), sd.get("optimizers", [])):
-            base = len(model._layout)
-            for j, p in enumerate(self._neck_params(model)):
-                st = opt["state"].get(base + j)
-                if self.optimizer != "sgd":
-                    if st is not None:
-                        self._neck_adam[id(p)] = [int(float(st["step"]))] + [
-                            st[k].to(device=p.device, dtype=p.dtype).reshape(p.shape).clone() for k in ("exp_avg", "exp_avg_sq")]
-                    continue
-                if st is not None and st.get("momentum_buffer") is not None:
-                    self._neck_mom[id(p)] = st["momentum_buffer"].to(device=p.device, dtype=p.dtype).reshape(p.shape).clone()
-
-    def _sgd_model(self, model, buf, lr, first):
+    def _sgd_model(self, trained, lr):
         """torch.optim.SGD (or Adam / AdamW) semantics over all parameters of a UNet_Plus: the flat U-Net buffer in one pass +
-        the neck tensors."""
+        one launch per neck tensor that has a gradient (model1's necks never have one: main.py:148 drops their outputs)."""
+        model, _, state = trained
         st = L.stream_ptr(model.flat_params.device)
-        lib = L.lib()
-        g = model.last_flat_grad
-        if self.optimizer != "sgd":
-            k = next(i for i, (m, _, _) in enumerate(self._trained) if m is model)
-            self._adam(L.ptr(model.flat_params), L.ptr(g), L.ptr(buf[0]), L.ptr(buf[1]), None, model.flat_params.numel(),
-                       self._adam_scalars(self._adam_steps[k], lr) + [0.0], None, st)
-            for p in self._neck_params(model):
-                if p.grad is None:
-                    continue
-                # torch.optim.Adam: state (zero moments, step 0) is created the first time a tensor has a gradient, and
-                # each tensor counts its own steps
-                state = self._neck_adam.setdefault(id(p), [0, torch.zeros_like(p.data), torch.zeros_like(p.data)])
-                state[0] += 1
-                self._adam(L.ptr(p.data), L.ptr(p.grad.contiguous()), L.ptr(state[1]), L.ptr(state[2]), None, p.numel(),
-                           self._adam_scalars(state[0], lr) + [0.0], None, st)
-            return
-        L.check(lib.hpfg_sgd_momentum(L.ptr(model.flat_params), L.ptr(g), L.ptr(buf), model.flat_params.numel(), lr, self.momentum,
-                                      self.weight_decay, self._grad_scale, first, st), "hpfg_sgd_momentum")
+        self._opt.launch(model.flat_params, model.last_flat_grad, state, None, lr, 0.0, None, st)
         for p in self._neck_params(model):
             if p.grad is None:
                 continue
-            mom = self._neck_mom.get(id(p))
-            fresh = mom is None                       # torch.optim.SGD: the first gradient a tensor sees initialises its buffer
-            if fresh:
-                mom = self._neck_mom[id(p)] = torch.zeros_like(p.data)
-            L.check(lib.hpfg_sgd_momentum(L.ptr(p.data), L.ptr(p.grad.contiguous()), L.ptr(mom), p.numel(), lr, self.momentum,
-                                          self.weight_decay, self._grad_scale, int(fresh), st),
-                    "hpfg_sgd_momentum")
+            # torch.optim: a tensor's state is created the first time it has a gradient, and each tensor counts its own steps
+            neck = self._neck_states.get(id(p))
+            if neck is None:
+                neck = self._neck_states[id(p)] = self._opt.new_state(p.data)
+            neck.step += 1
+            self._opt.launch(p.data, p.grad.contiguous(), neck, None, lr, 0.0, None, st)
 
     def step(self, label_img, target_label, label_img1, target_label1, img_unlabel, cutmix_mask, lr=None):
         """lr: override of the Medical_LR value of this iteration (resuming with a fresh scheduler; parity harness).
@@ -933,9 +790,8 @@ class HPFGStep(_StepBase):
                 dist.all_reduce(m.last_flat_grad, group=self.pg)
                 allreduce_tensor_list([p.grad for p in self._neck_params(m)], group=self.pg)
         lr = medical_lr(self.cur_itrs, self.base_lr, self.total_itrs) if lr is None else lr
-        first = int(self.cur_itrs == 1)
-        self._sgd_model(m1, self.b1, lr, first)
-        self._sgd_model(m2, self.b2, lr, first)
+        self._sgd_model(self._trained[0], lr)
+        self._sgd_model(self._trained[1], lr)
         alpha = min(1 - 1 / (self.cur_itrs + 1), self.ema_decay)
         ema_update_flat(m2.ensure_flat(), m1.ensure_flat(), alpha)          # update_ema_variables_backbone: encoder + decoder = the flat buffer
         update_ema_variables(m2, ema, self.ema_decay, self.cur_itrs)

@@ -29,7 +29,7 @@ acc = {}
 lib = L.lib()
 buckets = hb.gradient_buckets(1, 4)
 for _ in range(reps):
-    step.cur_itrs += 1
+    step._next_iteration()
     main = torch.cuda.current_stream(dev)
     side = step._side_stream(dev)
     shape = (32, 4, 224, 224)
@@ -58,7 +58,7 @@ for _ in range(reps):
             evs.append((a, z))
     main.wait_stream(comm)
     e_sgd0.record(main)
-    step._sgd(student, step.grads, step.mom, None, teacher)
+    step._opt_step(step._trained[0], None, teacher)
     e_sgd1.record(main)
     torch.cuda.synchronize()
     vals = {"forward+loss": e_start.elapsed_time(e_bwd0), "backward (main stream)": e_bwd0.elapsed_time(e_bwd1),

@@ -44,8 +44,8 @@ for _ in range(reps):
     e[4].record()
     step._backward(student, plan, r["dstudent"], step.grads)
     e[5].record()
-    step.cur_itrs += 1
-    step._sgd(student, step.grads, step.mom, None, teacher)
+    step._next_iteration()
+    step._opt_step(step._trained[0], None, teacher)
     e[6].record()
     torch.cuda.synchronize()
     for i in range(6):

@@ -6,6 +6,7 @@ import pytest
 import torch
 
 import hpfg_b200 as hb
+from hpfg_b200.optim import OptState
 
 KINDS = ("mt", "cps", "uamt", "ict", "s4cv", "hpfg")
 # per driver kind: the attribute holding each trained network's (exp_avg, exp_avg_sq) and its number of parameters
@@ -41,43 +42,45 @@ def test_every_driver_accepts_adam_and_rejects_unknown_optimizers(kind):
 
 
 @pytest.mark.parametrize("name", ["adam", "adamw"])
-def test_dyn_scalars_match_torch_python_formulas(name):
+def test_device_block_adam_groups_match_torch_python_formulas(name):
     """The Adam group of the device block is torch's double-precision scalars (adam.py, non-capturable foreach branch)
     rounded once to fp32; graph replays and eager launches read the same values."""
     lr0, wd, betas = 0.01, 1e-2, (0.9, 0.999)
     st, _ = _driver("cps", optimizer=name, lr=lr0, weight_decay=wd, betas=betas)
     for t in (1, 2, 3, 10, 150, 4000, 29999):
         st.cur_itrs = t
-        st._adam_steps = [t, t]
+        for _, _, s in st._trained:
+            s.step = t
         lr = hb.medical_lr(t, lr0, 30000)
         bc1, bc2 = 1 - betas[0] ** t, 1 - betas[1] ** t
         want = [(lr / bc1) * -1, bc2 ** 0.5, 1 - lr * wd if name == "adamw" else 1.0]
-        assert st._adam_scalars(t, lr) == want
+        assert st._opt.scalars(t, lr) == want
         block = torch.tensor(st._dyn_scalars(), dtype=torch.float32)
         assert block.numel() == 4 + 2 * 5
         for k in range(2):
             assert torch.equal(block[4 + 5 * k:4 + 5 * k + 3], torch.tensor(want, dtype=torch.float32))
     uamt, _ = _driver("uamt", optimizer=name)
-    uamt.cur_itrs, uamt._adam_steps = 3, [3]
+    uamt.cur_itrs, uamt._trained[0][2].step = 3, 3
     block = uamt._dyn_scalars(0.99, 0.5)
     assert len(block) == 10 and block[4] == 0.5 and block[-2:] == block[1:3]       # [..., thr | step_size, bc2, decay, alpha, 1-alpha]
 
 
 def _fill_state(st, kind):
     st.cur_itrs = 7
-    st._adam_steps = [7] * len(st._adam_steps)
+    for _, _, s in st._trained:
+        s.step = 7
     for attr, _ in OPTS[kind]:
         m, v = getattr(st, attr)
         m.uniform_(-1, 1)
         v.uniform_(0, 1)
     if kind == "hpfg":
         for j, p in enumerate(st._neck_params(st.m2)):
-            st._neck_adam[id(p)] = [3 + j, torch.randn_like(p), torch.rand_like(p)]
+            st._neck_states[id(p)] = OptState([torch.randn_like(p), torch.rand_like(p)], 3 + j)
 
 
 @pytest.mark.parametrize("name", ["adam", "adamw"])
 @pytest.mark.parametrize("kind", KINDS)
-def test_adam_checkpoint_layout_and_roundtrip(kind, name):
+def test_adam_state_checkpoint_layout_and_roundtrip(kind, name):
     wd = 1e-4
     st, nets = _driver(kind, optimizer=name, weight_decay=wd)
     assert all(opt["state"] == {} for opt in st.state_dict()["optimizers"])       # no state before the first step
@@ -113,19 +116,19 @@ def test_adam_checkpoint_layout_and_roundtrip(kind, name):
             assert float(sd["optimizers"][1]["state"][82 + j]["step"]) == 3 + j          # per-tensor step counts
     st2, nets2 = _driver(kind, optimizer=name, weight_decay=wd)
     st2.load_state_dict(sd)
-    assert st2.cur_itrs == 7 and st2._adam_steps == [7] * len(OPTS[kind])
+    assert st2.cur_itrs == 7 and [s.step for _, _, s in st2._trained] == [7] * len(OPTS[kind])
     sd2 = st2.state_dict()
     for o, o2 in zip(sd["optimizers"], sd2["optimizers"]):
         assert o2["param_groups"] == o["param_groups"] and sorted(o2["state"]) == sorted(o["state"])
         for i in o["state"]:
             assert all(torch.equal(o2["state"][i][key], o["state"][i][key]) for key in o["state"][i])
     if kind == "hpfg":
-        assert not any(id(q) in st2._neck_adam for q in st2._neck_params(nets2[0]))
-        assert [st2._neck_adam[id(q)][0] for q in st2._neck_params(nets2[1])] == [3 + j for j in range(16)]
+        assert not any(id(q) in st2._neck_states for q in st2._neck_params(nets2[0]))
+        assert [st2._neck_states[id(q)].step for q in st2._neck_params(nets2[1])] == [3 + j for j in range(16)]
 
 
 @pytest.mark.parametrize("kind", ["mt", "hpfg"])
-def test_adam_checkpoint_mismatches_raise(kind):
+def test_adam_state_checkpoint_mismatches_raise(kind):
     st, _ = _driver(kind, optimizer="adamw")
     _fill_state(st, kind)
     sd = st.state_dict()
@@ -144,3 +147,49 @@ def test_adam_checkpoint_mismatches_raise(kind):
     for fresh in (sgd.state_dict(), _driver(kind)[0].state_dict()):         # with and without momentum state
         with pytest.raises(ValueError, match="SGD"):
             _driver(kind, optimizer="adam")[0].load_state_dict(fresh)
+
+
+def _fill_any(st, kind, step):
+    """State as after ``step`` iterations, for either optimiser kind: random buffers, step counts, Philox offsets."""
+    st.cur_itrs = step
+    for i, m in enumerate(st._networks):
+        m._philox_offset = 8 * (step + i)
+    for _, _, s in st._trained:
+        s.step = step
+        for b in s.bufs:
+            b.uniform_(0, 1)
+    if kind == "hpfg":
+        for p in st._neck_params(st.m2):
+            st._neck_states[id(p)] = OptState([torch.rand_like(p) for _ in st._opt.KEYS], step)
+
+
+def _snapshot(st):
+    states = [s for _, _, s in st._trained] + list(st._neck_states.values())
+    return ((st.cur_itrs, [m._philox_offset for m in st._networks], sorted(st._neck_states), [s.step for s in states]),
+            [b.clone() for s in states for b in s.bufs])
+
+
+@pytest.mark.parametrize("name", ["sgd", "adamw"])
+@pytest.mark.parametrize("kind", ["mt", "hpfg"])
+def test_rejected_load_changes_nothing(kind, name):
+    """load_state_dict checks the whole checkpoint before it changes anything: a checkpoint of the other optimiser kind, or
+    one whose last network's U-Net tensors carry different Adam step counts, leaves cur_itrs, the Philox offsets, every
+    optimiser buffer and every step count as they were."""
+    st, _ = _driver(kind, optimizer=name)
+    _fill_any(st, kind, 7)
+    other, _ = _driver(kind, optimizer="adamw" if name == "sgd" else "sgd")
+    _fill_any(other, kind, 9)
+    bad = [(other.state_dict(), "Adam" if name == "sgd" else "SGD")]
+    if name == "adamw":
+        same, _ = _driver(kind, optimizer=name)
+        _fill_any(same, kind, 9)
+        sd = same.state_dict()
+        sd["optimizers"][-1]["state"][5]["step"] = torch.tensor(6.0)
+        bad.append((sd, "step count"))
+    before = _snapshot(st)
+    for sd, match in bad:
+        with pytest.raises(ValueError, match=match):
+            st.load_state_dict(sd)
+        after = _snapshot(st)
+        assert after[0] == before[0] and len(after[1]) == len(before[1])
+        assert all(torch.equal(a, b) for a, b in zip(after[1], before[1]))

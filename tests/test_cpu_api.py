@@ -11,6 +11,7 @@ import torch
 import oracle
 import hpfg_b200 as hb
 from hpfg_b200 import _lib as L
+from hpfg_b200.optim import OptState
 
 ROOT = os.path.dirname(os.path.dirname(os.path.abspath(__file__)))
 
@@ -166,7 +167,7 @@ CHECKPOINT_LAYOUT = {
 
 
 @pytest.mark.parametrize("kind", sorted(CHECKPOINT_LAYOUT))
-def test_step_driver_checkpoint_layout_and_roundtrip(kind):
+def test_step_driver_sgd_checkpoint_layout_and_roundtrip(kind):
     """state_dict() of every step driver: Philox offsets of its networks in a fixed order, one torch.optim.SGD-style entry per
     trained network (lr of the next iteration, per-parameter momentum in parameters() order), and it round-trips."""
     philox_of, opts = CHECKPOINT_LAYOUT[kind]
@@ -179,7 +180,7 @@ def test_step_driver_checkpoint_layout_and_roundtrip(kind):
         getattr(st, name).uniform_(-1, 1)
     if kind == "hpfg":
         for p in st._neck_params(nets[1]):
-            st._neck_mom[id(p)] = torch.randn_like(p)
+            st._neck_states[id(p)] = OptState([torch.randn_like(p)], 7)
     sd = st.state_dict()
     assert sd["cur_itrs"] == 7 and sd["philox"] == [8 * (i + 1) for i in philox_of]
     assert len(sd["optimizers"]) == len(opts)
@@ -217,7 +218,7 @@ def test_necks_and_dense_loss_have_no_cpu_path():
         hb.Dense_Loss(batch_size=5)(x, y)                  # the reference's mask is built for the constructor's batch size
 
 
-def test_hpfg_step_checkpoint_carries_neck_momentum():
+def test_hpfg_step_checkpoint_carries_neck_state():
     """HPFGStep.state_dict(): torch.optim.SGD layout over all 98 parameters of each UNet_Plus -- the flat U-Net momentum at
     indices 0..81, the neck tensors' buffers at 82..97 (only for tensors that have seen a gradient) -- and it round-trips."""
     torch.manual_seed(9)
@@ -229,7 +230,7 @@ def test_hpfg_step_checkpoint_carries_neck_momentum():
     necks2 = st._neck_params(m2)
     assert len(necks2) == 16 and [tuple(p.shape) for p in necks2] == [s for _, s in oracle.unet_plus_neck_spec(4)]
     for p in necks2:
-        st._neck_mom[id(p)] = torch.randn_like(p)
+        st._neck_states[id(p)] = OptState([torch.randn_like(p)], 7)
     sd = st.state_dict()
     assert sd["cur_itrs"] == 7 and len(sd["optimizers"]) == 2
     o1, o2 = sd["optimizers"]
@@ -242,8 +243,8 @@ def test_hpfg_step_checkpoint_carries_neck_momentum():
     st2.load_state_dict(sd)
     assert st2.cur_itrs == 7 and torch.equal(st2.b1, st.b1) and torch.equal(st2.b2, st.b2)
     for p, q in zip(necks2, st2._neck_params(n2)):
-        assert torch.equal(st2._neck_mom[id(q)], st._neck_mom[id(p)])
-    assert not any(id(q) in st2._neck_mom for q in st2._neck_params(n1))
+        assert torch.equal(st2._neck_states[id(q)].bufs[0], st._neck_states[id(p)].bufs[0])
+    assert not any(id(q) in st2._neck_states for q in st2._neck_params(n1))
 
 
 def test_oracle_is_test_infrastructure_only():
