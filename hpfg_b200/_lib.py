@@ -59,6 +59,8 @@ SIGNATURES = {
     "hpfg_ict_loss": (c_int, [c_vp, c_vp, c_vp, c_vp, c_int, c_int, c_int, c_int, c_int, c_f, c_vp, ctypes.POINTER(c_f),
                               c_f, c_f, c_vp, c_vp, c_vp, c_vp]),
     "hpfg_ict_mix": (c_int, [c_vp, c_vp, c_vp, c_int, c_i64, c_vp, c_vp]),
+    "hpfg_cutmix_loss": (c_int, [c_vp] * 5 + [c_int] * 6 + [c_f, c_vp, ctypes.POINTER(c_f), c_f, c_f] + [c_vp] * 5),
+    "hpfg_cutmix_mix": (c_int, [c_vp] * 3 + [c_int] * 5 + [c_vp, c_vp]),
     "hpfg_s4cv_loss": (c_int, [c_vp, c_vp, c_vp, c_vp, c_int, c_int, c_int, c_int, c_int, c_f, c_f, c_vp,
                                ctypes.POINTER(c_f), c_f, c_f, c_vp, c_vp, c_vp, c_vp, c_vp, c_vp, c_vp]),
     "hpfg_softmax_mse": (c_int, [c_vp, c_vp, c_vp, c_int, c_int, c_int, c_int, c_int, c_vp, c_vp]),
@@ -70,7 +72,9 @@ SIGNATURES = {
                                                                c_vp]),
     "hpfg_dense_contrastive_workspace_floats": (c_i64, [c_int, c_int, c_int]),
     "hpfg_dense_contrastive": (c_int, [c_vp, c_vp, c_int, c_int, c_int, c_f, c_vp, c_vp, c_vp, c_vp]),
+    "hpfg_dense_contrastive_scaled": (c_int, [c_vp, c_vp, c_int, c_int, c_int, c_f, c_f, c_vp, c_vp, c_vp, c_vp, c_vp]),
     "hpfg_ema_update": (c_int, [c_vp, c_vp, c_i64, c_f, c_vp]),
+    "hpfg_ema_update_dv": (c_int, [c_vp, c_vp, c_i64, c_vp, c_vp]),
     "hpfg_sgd_momentum": (c_int, [c_vp, c_vp, c_vp, c_i64, c_f, c_f, c_f, c_f, c_int, c_vp]),
     "hpfg_sgd_momentum_ema": (c_int, [c_vp, c_vp, c_vp, c_vp, c_i64, c_f, c_f, c_f, c_f, c_int, c_f, c_vp]),
     "hpfg_sgd_momentum_ema_dv": (c_int, [c_vp, c_vp, c_vp, c_vp, c_i64, c_f, c_f, c_f, c_int, c_vp, c_vp]),
@@ -80,7 +84,7 @@ SIGNATURES = {
 }
 
 PREC_FP32, PREC_BF16 = 0, 1
-LOSS_SUP, LOSS_MT, LOSS_CPS, LOSS_UAMT, LOSS_ICT, LOSS_S4CV = 0, 1, 2, 3, 4, 5
+LOSS_SUP, LOSS_MT, LOSS_CPS, LOSS_UAMT, LOSS_ICT, LOSS_S4CV, LOSS_CUTMIX = 0, 1, 2, 3, 4, 5, 6
 NUM_BN, NUM_DROPOUT, NUM_PARAMS = 18, 5, 82
 
 _lib = None

@@ -4,7 +4,8 @@
 //   2017_03_NIPS_Mean-Teacher_ACDC.py:97-106, 2021_06_CVPR_CPS_ACDC.py:99-111,
 //   2019_07_MICCAI_Uncertainty_Aware_ACDC.py:145-162,
 //   2022_02_ISBI_ICT-MedSeg_ACDC.py:111-137 (ICT: consistency against a per-sample mix of two teacher softmaxes),
-//   2022_08_CVPR_S4CVNet_ACDC.py:124-156 (two students, Dice-only cross pseudo supervision + Mean-Teacher MSE).
+//   2022_08_CVPR_S4CVNet_ACDC.py:124-156 (two students, Dice-only cross pseudo supervision + Mean-Teacher MSE),
+//   main.py:125-134,143 (HPFG model1: supervised + Dice against the teacher's argmax pasted into a second labeled draw by CutMix).
 // Dice is a ratio of batch-wide sums, so the gradient needs those sums first: phase 1 (reduce kernel) streams the logits that
 // carry batch-wide sums and reduces with warp shuffles -> one double atomic per block per quantity; phase 2 (grad kernel)
 // streams all logits (L2-resident: they are << 126 MB) and writes dlogits.  Only the LABELED images carry such sums in the
@@ -39,6 +40,9 @@ struct LossArgs {
     const float *student, *other, *mc;
     const float *mix;               // ICT: per-sample mix factor lambda[n_u] (device)
     const int64_t *labels;
+    const int64_t *labels1;         // CutMix: labels of the second labeled draw [n_l1,H,W], image u reads u % n_l1
+    const float *cutmix_mask;       // CutMix: [n_u,H,W] mask (1: the teacher's argmax, 0: labels1)
+    int n_l1;
     float cons_weight, uamt_threshold, ce_coef, dice_coef;
     float cons_weight2;             // S4CV: weight of the Mean-Teacher MSE terms (cons_weight = weight of the pseudo Dice terms)
     const float *cons_weight_dev;   // optional device scalar overriding cons_weight (CUDA-graph replays)
@@ -48,7 +52,7 @@ struct LossArgs {
     float *dstudent, *dother, *scalars;
     int64_t *pseudo1, *pseudo2;
     double *acc;
-    uint8_t *aux;   // CPS: pl1 | pl2 (n_u*hw each); UAMT: mask (n_u*hw)
+    uint8_t *aux;   // CPS: pl1 | pl2 (n_u*hw each); UAMT: mask (n_u*hw); CutMix: pseudo-labels (n_u*hw, 255 = no class)
     int world;         // exact-global mode: number of ranks whose sums were all-reduced into acc (1 otherwise)
     int reduce_imgs;   // images the reduce kernel streams: n_l for SUP / MT / ICT (their global sums only involve labeled pixels)
     FastDiv qdiv;   // division by hw/4 without the 64-bit integer divide (quad index -> image, quad in image)
@@ -189,6 +193,11 @@ __global__ void __launch_bounds__(256, MODE == HPFG_LOSS_S4CV ? 1 : 2) loss_redu
         if (MODE != HPFG_LOSS_SUP && (TWO || !labeled))
             load4<C>(TWO ? A.other + (img * C) * hw + pix : A.other + (u * C) * hw + pix, hw, z2);
         if (MODE == HPFG_LOSS_ICT && !labeled) load4<C>(A.other + ((u + A.n_u) * C) * hw + pix, hw, z3);
+        float4 cm;
+        if (MODE == HPFG_LOSS_CUTMIX && !labeled) {
+            load_labels4(A.labels1 + (u % A.n_l1) * hw + pix, lab);
+            cm = __ldg(reinterpret_cast<const float4 *>(A.cutmix_mask + u * hw + pix));
+        }
         softmax4<C>(z, p, lse);
         if (labeled) {
             acc_sup<C>(z, p, lse, lab, sl[0]);
@@ -218,6 +227,26 @@ __global__ void __launch_bounds__(256, MODE == HPFG_LOSS_S4CV ? 1 : 2) loss_redu
                         const float d = p[c][j] - (p2[c][j] * oml + p3[c][j] * lam);
                         misc[0] += d * d;
                     }
+            } else if (MODE == HPFG_LOSS_CUTMIX) {
+                // main.py:132-134: pseudo = target1*(1-m) + argmax(softmax(t))*m in fp32, rounded as torch rounds it; a pixel is
+                // class c for the Dice term iff that float equals c (the reference's one-hot), else it belongs to no class
+                const float m[4] = {cm.x, cm.y, cm.z, cm.w};
+                int pl[4];
+#pragma unroll
+                for (int j = 0; j < 4; ++j) {
+                    const float v = __fadd_rn(__fmul_rn((float)lab[j], __fsub_rn(1.f, m[j])), __fmul_rn((float)argmax_first<C>(p2, j), m[j]));
+                    pl[j] = 255;
+#pragma unroll
+                    for (int c = 0; c < C; ++c)
+                        if (v == (float)c) pl[j] = c;
+                }
+                acc_sup<C>(z, p, lse, pl, su[0]);
+                const int64_t o = u * hw + pix;
+                *reinterpret_cast<uchar4 *>(A.aux + o) = make_uchar4(pl[0], pl[1], pl[2], pl[3]);
+                if (A.pseudo1) {
+                    *reinterpret_cast<longlong2 *>(A.pseudo1 + o) = make_longlong2(pl[0], pl[1]);
+                    *reinterpret_cast<longlong2 *>(A.pseudo1 + o + 2) = make_longlong2(pl[2], pl[3]);
+                }
             } else if (TWO) {
                 int pl1[4], pl2[4];
 #pragma unroll
@@ -291,6 +320,7 @@ __global__ void __launch_bounds__(256, MODE == HPFG_LOSS_S4CV ? 1 : 2) loss_redu
         flush<NS>(su[0], A.acc + 1 * kAccPerSet, slots, smem);
         flush<NS>(su[NSETS - 1], A.acc + 3 * kAccPerSet, slots, smem);
     }
+    if (MODE == HPFG_LOSS_CUTMIX) flush<NS>(su[0], A.acc + 1 * kAccPerSet, slots, smem);
     if (MODE == HPFG_LOSS_MT || MODE == HPFG_LOSS_UAMT || MODE == HPFG_LOSS_ICT || MODE == HPFG_LOSS_S4CV) {
         if (threadIdx.x < 3) slots[threadIdx.x] = threadIdx.x;
         __syncthreads();
@@ -381,6 +411,7 @@ __global__ void __launch_bounds__(256, MODE == HPFG_LOSS_MT ? HPFG_LOSS_MT_MINBL
     __shared__ float s_cons;      // per-element consistency coefficient
     const bool s4cv = A.mode == HPFG_LOSS_S4CV;
     const bool cps = A.mode == HPFG_LOSS_CPS || s4cv;   // two student networks
+    constexpr bool cutmix = MODE == HPFG_LOSS_CUTMIX;     // (its own instantiation: the generic kernel is unchanged)
     // Mean-Teacher / ICT: the consistency VALUE is accumulated here, next to its gradient, so the reduce kernel only has to
     // stream the labeled images (the Dice / CE sums); the last CTA to finish writes loss and consistency term
     const bool late_mse = A.mode == HPFG_LOSS_MT || A.mode == HPFG_LOSS_ICT;
@@ -394,6 +425,7 @@ __global__ void __launch_bounds__(256, MODE == HPFG_LOSS_MT ? HPFG_LOSS_MT_MINBL
             make_coef<C>(A.acc + 2 * kAccPerSet, A.class_w, coef[2]);
             make_coef<C>(A.acc + 3 * kAccPerSet, A.class_w, coef[3]);
         }
+        if (cutmix) make_coef<C>(A.acc + 1 * kAccPerSet, A.class_w, coef[1]);
         float cons = 0.f, cons_val = 0.f;
         const double M = (double)A.n_u * C * (double)A.hw * (double)A.world;      // elements of the consistency mean (all ranks)
         if (late_mse) {   // the squared distance is summed by THIS kernel (below); its gradient needs no global sum
@@ -414,6 +446,7 @@ __global__ void __launch_bounds__(256, MODE == HPFG_LOSS_MT ? HPFG_LOSS_MT_MINBL
                 sup = sup0 + A.ce_coef * coef[2].ce + A.dice_coef * coef[2].dice;
                 aux = ps_ce * coef[1].ce + ps_dice * coef[1].dice + ps_ce * coef[3].ce + ps_dice * coef[3].dice;
             }
+            if (cutmix) aux = coef[1].dice;      // scalars[2]: the unweighted pseudo-label Dice
             float loss = (A.mode == HPFG_LOSS_SUP) ? sup : sup + A.cons_weight * aux;
             float s6 = (float)A.acc[kAccMaskSum], s7 = 0.f;
             if (s4cv) {   // loss_semi = w_cps*(ps1+ps2) + w_mt*(cl1+cl2); scalars: [2] loss_semi, [6] ps1+ps2, [7] cl1+cl2
@@ -460,6 +493,15 @@ __global__ void __launch_bounds__(256, MODE == HPFG_LOSS_MT ? HPFG_LOSS_MT_MINBL
             continue;
         }
         const int64_t u = img - A.n_l;
+        if (cutmix) {       // Dice only against the reduce kernel's pseudo-labels, weighted by pseudo_weight
+            load4<C>(A.student + so, hw, z);
+            const uchar4 a = *reinterpret_cast<const uchar4 *>(A.aux + u * hw + pix);
+            const int pl[4] = {a.x, a.y, a.z, a.w};
+            softmax4g<C>(z, p);
+            grad_sup<C>(p, pl, coef[1], 0.f, 1.f, A.cons_weight, g);
+            store4<C>(A.dstudent + so, hw, g);
+            continue;
+        }
         if (A.mode == HPFG_LOSS_SUP) {
 #pragma unroll
             for (int c = 0; c < C; ++c)
@@ -831,13 +873,15 @@ static int launch_loss(const LossArgs &A, cudaStream_t st) {
         case HPFG_LOSS_ICT: HPFG_CUDA_CHECK(launch_pdl(loss_reduce_kernel<C, HPFG_LOSS_SUP>, rgrid, 256, 0, st, A)); break;
         case HPFG_LOSS_CPS: HPFG_CUDA_CHECK(launch_pdl(loss_reduce_kernel<C, HPFG_LOSS_CPS>, rgrid, 256, 0, st, A)); break;
         case HPFG_LOSS_S4CV: HPFG_CUDA_CHECK(launch_pdl(loss_reduce_kernel<C, HPFG_LOSS_S4CV>, rgrid, 256, 0, st, A)); break;
+        case HPFG_LOSS_CUTMIX: HPFG_CUDA_CHECK(launch_pdl(loss_reduce_kernel<C, HPFG_LOSS_CUTMIX>, rgrid, 256, 0, st, A)); break;
         default: HPFG_CUDA_CHECK(launch_pdl(loss_reduce_kernel<C, HPFG_LOSS_UAMT>, rgrid, 256, 0, st, A)); break;
     }
     HPFG_LAUNCH_CHECK();
     // exact-global mode: Dice / CE / pseudo-label / mask sums over the batch of ALL ranks before any coefficient is formed
     // (the last slot is the gradient kernel's block counter: still zero everywhere, so it may take part)
     const bool mt = A.mode == HPFG_LOSS_MT;
-    auto grad = mt ? loss_grad_kernel<C, HPFG_LOSS_MT> : loss_grad_kernel<C, -1>;
+    auto grad = mt ? loss_grad_kernel<C, HPFG_LOSS_MT>
+                   : A.mode == HPFG_LOSS_CUTMIX ? loss_grad_kernel<C, HPFG_LOSS_CUTMIX> : loss_grad_kernel<C, -1>;
     const int ggrid = mt ? loss_grid((int64_t)(A.n_l + A.n_u) * (A.hw >> 2), loss_mt_ctas_per_sm()) : grid;
     if (A.world > 1) {
         HPFG_RETURN_IF(sync_allreduce(A.acc, kAccTotal, true, st));
@@ -868,7 +912,7 @@ extern "C" int64_t hpfg_ssl_loss_workspace_bytes(int mode, int n_l, int n_u, int
     (void)n_l; (void)num_classes;
     int64_t aux = 0;
     if (mode == HPFG_LOSS_CPS || mode == HPFG_LOSS_S4CV) aux = 2LL * n_u * height * width;
-    if (mode == HPFG_LOSS_UAMT) aux = 1LL * n_u * height * width;
+    if (mode == HPFG_LOSS_UAMT || mode == HPFG_LOSS_CUTMIX) aux = 1LL * n_u * height * width;
     return kAccTotal * (int64_t)sizeof(double) + ((aux + 255) / 256) * 256;
 }
 
@@ -878,8 +922,9 @@ static int ssl_loss_impl(int mode, const float *student, const float *other, con
                          const float *class_weights_host, float ce_coef, float dice_coef, float *dstudent, float *dother,
                          float *scalars_out, int64_t *pseudo1, int64_t *pseudo2, void *workspace, void *stream,
                          const float *mix = nullptr, float cons_weight2 = 0.f, const float *cons_weight2_dev = nullptr,
-                         const float *uamt_threshold_dev = nullptr) {
-    HPFG_REQUIRE(mode >= HPFG_LOSS_SUP && mode <= HPFG_LOSS_S4CV, "hpfg_ssl_loss: unknown mode");
+                         const float *uamt_threshold_dev = nullptr, const int64_t *labels1 = nullptr,
+                         const float *cutmix_mask = nullptr, int n_l1 = 0) {
+    HPFG_REQUIRE(mode >= HPFG_LOSS_SUP && mode <= HPFG_LOSS_CUTMIX, "hpfg_ssl_loss: unknown mode");
     HPFG_REQUIRE(student && dstudent && scalars_out && workspace, "hpfg_ssl_loss: null buffer");
     HPFG_REQUIRE(n_l >= 0 && n_u >= 0 && n_l + n_u > 0, "hpfg_ssl_loss: empty batch");
     HPFG_REQUIRE(n_l == 0 || labels, "hpfg_ssl_loss: labels required");
@@ -890,6 +935,11 @@ static int ssl_loss_impl(int mode, const float *student, const float *other, con
         HPFG_REQUIRE(dother && other, "hpfg_ssl_loss: CPS / S4CV need peer logits and dother");
     if (mode == HPFG_LOSS_ICT && n_u > 0) HPFG_REQUIRE(mix, "hpfg_ict_loss: mix_factors required");
     if (mode == HPFG_LOSS_UAMT) HPFG_REQUIRE(mc_logits && mc_passes > 0, "hpfg_ssl_loss: UAMT needs mc_logits");
+    if (mode == HPFG_LOSS_CUTMIX && n_u > 0) {
+        HPFG_REQUIRE(labels1 && cutmix_mask, "hpfg_cutmix_loss: labels1 and cutmix_mask required");
+        HPFG_REQUIRE(n_l1 > 0 && n_u % n_l1 == 0, "hpfg_cutmix_loss: n_u must be a positive multiple of n_l1 (main.py:139-140 repeats "
+                                                  "the second labeled draw to the unlabeled batch)");
+    }
     cudaStream_t st = (cudaStream_t)stream;
     LossArgs A{};
     HPFG_REQUIRE((int64_t)(n_l + n_u) * height * width / 4 < (1LL << 31), "hpfg_ssl_loss: batch too large for 32-bit quad indexing");
@@ -900,6 +950,7 @@ static int ssl_loss_impl(int mode, const float *student, const float *other, con
     A.student = student; A.other = other; A.mc = mc_logits; A.labels = labels;
     A.mix = mix; A.cons_weight2 = cons_weight2; A.cons_weight2_dev = cons_weight2_dev;
     A.uamt_threshold_dev = uamt_threshold_dev;
+    A.labels1 = labels1; A.cutmix_mask = cutmix_mask; A.n_l1 = n_l1;
     A.cons_weight = cons_weight; A.cons_weight_dev = cons_weight_dev; A.uamt_threshold = uamt_threshold; A.ce_coef = ce_coef; A.dice_coef = dice_coef;
     for (int c = 0; c < kMaxC; ++c) A.class_w[c] = (class_weights_host && c < num_classes) ? class_weights_host[c] : 1.f;
     A.dstudent = dstudent; A.dother = dother; A.scalars = scalars_out; A.pseudo1 = pseudo1; A.pseudo2 = pseudo2;
@@ -990,6 +1041,18 @@ extern "C" int hpfg_s4cv_loss(const float *logits1, const float *logits2, const 
                          weights_dev ? weights_dev + 1 : nullptr);
 }
 
+// ---- HPFG model1 (main.py:125-134,143) -----------------------------------------------------------------------------
+extern "C" int hpfg_cutmix_loss(const float *student, const float *teacher_u, const int64_t *labels, const int64_t *labels1,
+                                const float *cutmix_mask, int n_l, int n_u, int n_l1, int num_classes, int height, int width,
+                                float pseudo_weight, const float *pseudo_weight_dev, const float *class_weights, float ce_coef,
+                                float dice_coef, float *dstudent, float *scalars_out, int64_t *pseudo_out, void *workspace,
+                                void *stream) {
+    return ssl_loss_impl(HPFG_LOSS_CUTMIX, student, teacher_u, nullptr, 0, labels, n_l, n_u, num_classes, height, width,
+                         pseudo_weight, pseudo_weight_dev, 0.f, class_weights, ce_coef, dice_coef, dstudent, nullptr,
+                         scalars_out, pseudo_out, nullptr, workspace, stream, nullptr, 0.f, nullptr, nullptr, labels1,
+                         cutmix_mask, n_l1);
+}
+
 namespace hpfg {
 // out[u] = a[u]*(1-lambda_u) + b[u]*lambda_u over whole images (the ICT input mix, 2022_02...:115-117); 128-bit accesses.
 __global__ void __launch_bounds__(256) ict_mix_kernel(const float4 *__restrict__ a, const float4 *__restrict__ b,
@@ -1002,6 +1065,24 @@ __global__ void __launch_bounds__(256) ict_mix_kernel(const float4 *__restrict__
         // separate roundings (no FMA contraction): bit-identical to torch's a*(1-l) + b*l
         out[q] = make_float4(__fadd_rn(__fmul_rn(x.x, o), __fmul_rn(y.x, l)), __fadd_rn(__fmul_rn(x.y, o), __fmul_rn(y.y, l)),
                              __fadd_rn(__fmul_rn(x.z, o), __fmul_rn(y.z, l)), __fadd_rn(__fmul_rn(x.w, o), __fmul_rn(y.w, l)));
+    }
+}
+
+// out[u,ch] = a[u % n_a, ch]*(1-m[u]) + b[u,ch]*m[u] (the CutMix input mix, main.py:145), the [n,1,H,W] mask broadcast over the
+// channels; separate roundings, as ict_mix_kernel: bit-identical to torch's expression on the repeated second labeled draw.
+__global__ void __launch_bounds__(256) cutmix_mix_kernel(const float4 *__restrict__ a, const float4 *__restrict__ b,
+                                                         const float4 *__restrict__ mask, float4 *__restrict__ out, int n_a,
+                                                         int channels, int64_t quads_per_plane, int64_t total_quads) {
+    pdl_prologue();
+    for (int64_t q = (int64_t)blockIdx.x * blockDim.x + threadIdx.x; q < total_quads; q += (int64_t)gridDim.x * blockDim.x) {
+        const int64_t plane = q / quads_per_plane, r = q - plane * quads_per_plane;
+        const int64_t u = plane / channels, ch = plane - u * channels;
+        const float4 m = __ldg(mask + u * quads_per_plane + r);
+        const float4 x = __ldg(a + ((u % n_a) * channels + ch) * quads_per_plane + r), y = __ldg(b + q);
+        out[q] = make_float4(__fadd_rn(__fmul_rn(x.x, __fsub_rn(1.f, m.x)), __fmul_rn(y.x, m.x)),
+                             __fadd_rn(__fmul_rn(x.y, __fsub_rn(1.f, m.y)), __fmul_rn(y.y, m.y)),
+                             __fadd_rn(__fmul_rn(x.z, __fsub_rn(1.f, m.z)), __fmul_rn(y.z, m.z)),
+                             __fadd_rn(__fmul_rn(x.w, __fsub_rn(1.f, m.w)), __fmul_rn(y.w, m.w)));
     }
 }
 
@@ -1110,6 +1191,23 @@ extern "C" int hpfg_ict_mix(const float *a, const float *b, const float *mix_fac
     ProfScope _prof(PROF_LOSS, st);
     HPFG_CUDA_CHECK(launch_pdl(ict_mix_kernel, loss_grid(total, 6), 256, 0, st, reinterpret_cast<const float4 *>(a),
                                reinterpret_cast<const float4 *>(b), mix_factors, reinterpret_cast<float4 *>(out), qpi, total));
+    HPFG_LAUNCH_CHECK();
+    return HPFG_OK;
+}
+
+extern "C" int hpfg_cutmix_mix(const float *a, const float *b, const float *cutmix_mask, int n, int n_a, int channels,
+                               int height, int width, float *out, void *stream) {
+    HPFG_REQUIRE(a && b && cutmix_mask && out, "hpfg_cutmix_mix: null buffer");
+    HPFG_REQUIRE(n > 0 && n_a > 0 && channels > 0, "hpfg_cutmix_mix: empty batch");
+    HPFG_REQUIRE(n % n_a == 0, "hpfg_cutmix_mix: n must be a multiple of n_a (main.py:139 repeats the second labeled draw)");
+    const int64_t hw = (int64_t)height * width;
+    HPFG_REQUIRE(hw > 0 && hw % 4 == 0, "hpfg_cutmix_mix: H*W must be a positive multiple of 4");
+    cudaStream_t st = (cudaStream_t)stream;
+    const int64_t qpp = hw / 4, total = qpp * channels * n;
+    ProfScope _prof(PROF_LOSS, st);
+    HPFG_CUDA_CHECK(launch_pdl(cutmix_mix_kernel, loss_grid(total, 6), 256, 0, st, reinterpret_cast<const float4 *>(a),
+                               reinterpret_cast<const float4 *>(b), reinterpret_cast<const float4 *>(cutmix_mask),
+                               reinterpret_cast<float4 *>(out), n_a, channels, qpp, total));
     HPFG_LAUNCH_CHECK();
     return HPFG_OK;
 }

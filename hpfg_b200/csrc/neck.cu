@@ -283,10 +283,11 @@ __global__ void contrast_rows_kernel(const float *__restrict__ z, int B, int V, 
 
 // CTA 0 writes loss = mean(rowloss).  With d_out1 != NULL, CTA k (< B): dL/dz_k = ((P_k. + P_.k) z - 2 z_pair) / (2B t) with the
 // pair's coefficient P_k,pair + P_pair,k - 2 taken as -(miss_k + miss_pair), pulled back through the normalisation of out_1[k]:
-// dx = (g - a <a,g>) / |x| per spatial position (g / eps where |x| < eps).
+// dx = (g - a <a,g>) / |x| per spatial position (g / eps where |x| < eps), times `out_scale` (from scale_dev when given) as a separate
+// rounding, so that d_out1 is bit-identical to out_scale * (the unscaled gradient).
 __global__ void contrast_grad_kernel(const float *__restrict__ z, const float *__restrict__ norms, const float *__restrict__ P,
                                      const float *__restrict__ miss, const float *__restrict__ rowloss, int B, int D, int S, float inv_t,
-                                     float *__restrict__ loss, float *__restrict__ d_out1) {
+                                     float out_scale, const float *__restrict__ scale_dev, float *__restrict__ loss, float *__restrict__ d_out1) {
     extern __shared__ float sm[];                   // g [V] | coef [2B]
     const int k = blockIdx.x, rows = 2 * B, V = D * S;
     float *g = sm, *coef = sm + V;
@@ -298,6 +299,7 @@ __global__ void contrast_grad_kernel(const float *__restrict__ z, const float *_
         *loss = v / (float)rows;
     }
     if (d_out1 == nullptr) return;
+    if (scale_dev) out_scale = *scale_dev;
     for (int j = threadIdx.x; j < rows; j += blockDim.x)
         coef[j] = (j == k + B) ? -(miss[k] + miss[k + B]) : P[(int64_t)k * rows + j] + P[(int64_t)j * rows + k];
     __syncthreads();
@@ -318,7 +320,7 @@ __global__ void contrast_grad_kernel(const float *__restrict__ z, const float *_
         const float inv = 1.f / fmaxf(nrm, kNormEps);
         for (int d = lane; d < D; d += 32) {
             const float gv = g[d * S + s];
-            d_out1[(int64_t)k * V + d * S + s] = (clamped ? gv : gv - zk[d * S + s] * dot) * inv;
+            d_out1[(int64_t)k * V + d * S + s] = __fmul_rn(out_scale, (clamped ? gv : gv - zk[d * S + s] * dot) * inv);
         }
     }
 }
@@ -420,8 +422,9 @@ extern "C" int64_t hpfg_dense_contrastive_workspace_floats(int batch, int dim, i
     return rows * dim * positions + rows * positions + rows * rows + 2 * rows;
 }
 
-extern "C" int hpfg_dense_contrastive(const float *out1, const float *out2, int batch, int dim, int positions, float temperature,
-                                      float *loss, float *d_out1, float *workspace, void *stream) {
+extern "C" int hpfg_dense_contrastive_scaled(const float *out1, const float *out2, int batch, int dim, int positions, float temperature,
+                                             float scale, const float *scale_dev, float *loss, float *d_out1, float *workspace,
+                                             void *stream) {
     HPFG_REQUIRE(out1 && out2 && loss && workspace, "hpfg_dense_contrastive: null buffer");
     HPFG_REQUIRE(batch > 0 && dim > 0 && positions > 0, "hpfg_dense_contrastive: empty problem");
     HPFG_REQUIRE(temperature > 0.f, "hpfg_dense_contrastive: temperature must be positive");
@@ -441,7 +444,13 @@ extern "C" int hpfg_dense_contrastive(const float *out1, const float *out2, int 
     HPFG_CUDA_CHECK(launch_pdl(contrast_rows_kernel, dim3((unsigned)rows), dim3(256), smem, st, (const float *)z, batch, (int)V, inv_t, P, miss, rowloss));
     HPFG_LAUNCH_CHECK();
     HPFG_CUDA_CHECK(launch_pdl(contrast_grad_kernel, dim3(d_out1 ? batch : 1), dim3(256), smem, st, (const float *)z, (const float *)norms,
-                               (const float *)P, (const float *)miss, (const float *)rowloss, batch, dim, positions, inv_t, loss, d_out1));
+                               (const float *)P, (const float *)miss, (const float *)rowloss, batch, dim, positions, inv_t, scale, scale_dev,
+                               loss, d_out1));
     HPFG_LAUNCH_CHECK();
     return HPFG_OK;
+}
+
+extern "C" int hpfg_dense_contrastive(const float *out1, const float *out2, int batch, int dim, int positions, float temperature,
+                                      float *loss, float *d_out1, float *workspace, void *stream) {
+    return hpfg_dense_contrastive_scaled(out1, out2, batch, dim, positions, temperature, 1.f, nullptr, loss, d_out1, workspace, stream);
 }

@@ -16,8 +16,12 @@ __device__ __forceinline__ float ema1(float e, float p, float alpha, float one_m
 }
 
 __global__ void __launch_bounds__(256) ema_kernel(float *__restrict__ ema, const float *__restrict__ param,
-                                                  int64_t n, float alpha, float one_minus) {
+                                                  int64_t n, float alpha, float one_minus, const float *__restrict__ dyn) {
     pdl_prologue();
+    if (dyn) {          // device block {alpha, 1 - alpha} (CUDA-graph replays)
+        alpha = dyn[0];
+        one_minus = dyn[1];
+    }
     const int64_t n4 = n >> 2;
     const int64_t stride = (int64_t)gridDim.x * blockDim.x;
     for (int64_t i = (int64_t)blockIdx.x * blockDim.x + threadIdx.x; i < n4; i += stride) {
@@ -175,7 +179,18 @@ extern "C" int hpfg_ema_update(float *ema, const float *param, int64_t n, float 
     HPFG_REQUIRE(aligned16(ema) && aligned16(param), "hpfg_ema_update: buffers must be 16-byte aligned");
     if (n == 0) return HPFG_OK;
     ProfScope _prof(PROF_OPTIM, (cudaStream_t)stream);
-    HPFG_CUDA_CHECK(launch_pdl(ema_kernel, flat_grid(n), 256, 0, (cudaStream_t)stream, ema, param, n, alpha, 1.0f - alpha));
+    HPFG_CUDA_CHECK(launch_pdl(ema_kernel, flat_grid(n), 256, 0, (cudaStream_t)stream, ema, param, n, alpha, 1.0f - alpha,
+                               (const float *)nullptr));
+    HPFG_LAUNCH_CHECK();
+    return HPFG_OK;
+}
+
+extern "C" int hpfg_ema_update_dv(float *ema, const float *param, int64_t n, const float *alpha_dev, void *stream) {
+    HPFG_REQUIRE(ema && param && alpha_dev && n >= 0, "hpfg_ema_update_dv: null buffer");
+    HPFG_REQUIRE(aligned16(ema) && aligned16(param), "hpfg_ema_update_dv: buffers must be 16-byte aligned");
+    if (n == 0) return HPFG_OK;
+    ProfScope _prof(PROF_OPTIM, (cudaStream_t)stream);
+    HPFG_CUDA_CHECK(launch_pdl(ema_kernel, flat_grid(n), 256, 0, (cudaStream_t)stream, ema, param, n, 0.f, 0.f, alpha_dev));
     HPFG_LAUNCH_CHECK();
     return HPFG_OK;
 }

@@ -293,6 +293,75 @@ def s4cvnet_loss(logits1, logits2, teacher_logits_u, labels, cps_weight, mt_weig
         a, b, t, labels, n_l, cps_weight=cps_weight, mt_weight=mt_weight, ce_coef=ce, dice_coef=dice))
 
 
+# ---- HPFG (main.py:125-145): model1's loss on the CutMix batch and the CutMix input mix ------------------------------------
+def check_cutmix_batch(n_u, n_l1):
+    """main.py's broadcast of the second labeled draw over the unlabeled batch needs n_u to be a multiple of its size."""
+    if n_l1 <= 0 or n_u % n_l1:
+        raise ValueError("CutMix: the unlabeled batch (%d) must be a multiple of the second labeled draw (%d), as main.py:139-140 "
+                         "repeats it" % (n_u, n_l1))
+
+
+def cutmix_loss_raw(student, teacher_u, labels, labels1, cutmix_mask, n_l, *, pseudo_weight, pseudo_weight_dev=None,
+                    class_weights=None, ce_coef=0.5, dice_coef=0.5, want_pseudo=False):
+    """Thin wrapper of hpfg_cutmix_loss.  student [n_l+n_u,C,H,W] logits of the CutMix batch; teacher_u [n_u,C,H,W] teacher
+    logits of the plain unlabeled images; labels [n_l,H,W]; labels1 [n_l1,H,W] (the second labeled draw, not repeated);
+    cutmix_mask [n_u,(1,)H,W].  Returns dict(scalars[8], dstudent, dother=None, pseudo=[n_u,H,W] int64 or None)."""
+    L.require_cuda(student, "logits")
+    student = student.contiguous().float()
+    n, c, h, w = student.shape
+    n_u = n - n_l
+    dev = student.device
+    teacher_u = teacher_u.contiguous().float()
+    assert teacher_u.shape == (n_u, c, h, w), "teacher logits must cover the unlabeled images"
+    labels = labels.contiguous().to(torch.int64)
+    assert labels.shape == (n_l, h, w), "labels must be [n_l,H,W]"
+    labels1 = labels1.contiguous().to(torch.int64)
+    assert labels1.dim() == 3 and tuple(labels1.shape[1:]) == (h, w), "labels1 must be [n_l1,H,W]"
+    check_cutmix_batch(n_u, labels1.shape[0])
+    mask = cutmix_mask.contiguous().float()
+    assert mask.numel() == n_u * h * w, "cutmix_mask must be [n_u,1,H,W]"
+    dstudent = torch.empty_like(student)
+    scalars = torch.empty(8, device=dev, dtype=torch.float32)
+    ws = _workspace(L.LOSS_CUTMIX, n_l, n_u, c, h, w, dev)
+    pseudo = torch.empty((n_u, h, w), device=dev, dtype=torch.int64) if want_pseudo else None
+    L.check(L.lib().hpfg_cutmix_loss(L.ptr(student), L.ptr(teacher_u), L.ptr(labels), L.ptr(labels1), L.ptr(mask), n_l, n_u,
+                                     labels1.shape[0], c, h, w, float(pseudo_weight), L.ptr(pseudo_weight_dev),
+                                     _weights_arg(class_weights, c), float(ce_coef), float(dice_coef), L.ptr(dstudent),
+                                     L.ptr(scalars), L.ptr(pseudo), L.ptr(ws), L.stream_ptr(dev)), "hpfg_cutmix_loss")
+    return dict(scalars=scalars, dstudent=dstudent, dother=None, pseudo=pseudo)
+
+
+def cutmix_pseudo_loss(outputs1, ema_logits_u, target_label, target_label1, cutmix_mask, pseudo_weight, ce=0.5, dice=0.5):
+    """model1's terms of main.py:125-134,143 in one call: ce*CE + dice*Dice of outputs1[:n_l] against target_label, plus
+    pseudo_weight * Dice(softmax(outputs1[n_l:]), target_label1*(1-m) + argmax(softmax(ema_logits_u))*m).  It replaces
+    ``loss1`` and the ``7*w*pseudo_supervision1`` term (pass pseudo_weight = 7*w); target_label1 is the second labeled draw
+    before main.py's repeat (image u reads u % n_l1).  Gradients flow to outputs1 only."""
+    n_l = target_label.shape[0]
+    t = ema_logits_u.detach()
+    return _RawLossFn.apply(outputs1, None, lambda s, _: cutmix_loss_raw(
+        s, t, target_label, target_label1, cutmix_mask, n_l, pseudo_weight=pseudo_weight, ce_coef=ce, dice_coef=dice))
+
+
+def cutmix_mix_inputs(label_img1, img_unlabel, cutmix_mask, out=None):
+    """batch_un_mix = label_img1*(1-m) + img_unlabel*m (main.py:139,145) with label_img1 [n_l1,C,H,W] the second labeled
+    draw, not repeated (image u reads u % n_l1), img_unlabel [n_u,C,H,W], cutmix_mask [n_u,1,H,W]: bit-identical to torch's
+    expression on the repeated draw.  ``out``: an [n_u,C,H,W] fp32 contiguous tensor to write into (e.g. the mixed half of a
+    persistent batch buffer)."""
+    L.require_cuda(img_unlabel, "CutMix inputs")
+    a, b = label_img1.contiguous().float(), img_unlabel.contiguous().float()
+    n_u, ch, h, w = b.shape
+    assert a.dim() == 4 and tuple(a.shape[1:]) == (ch, h, w), "label_img1 must be [n_l1,C,H,W]"
+    check_cutmix_batch(n_u, a.shape[0])
+    mask = cutmix_mask.contiguous().float()
+    assert mask.numel() == n_u * h * w, "cutmix_mask must be [n_u,1,H,W]"
+    if out is None:
+        out = torch.empty_like(b)
+    assert out.shape == b.shape and out.dtype == torch.float32 and out.is_contiguous()
+    L.check(L.lib().hpfg_cutmix_mix(L.ptr(a), L.ptr(b), L.ptr(mask), n_u, a.shape[0], ch, h, w, L.ptr(out),
+                                    L.stream_ptr(b.device)), "hpfg_cutmix_mix")
+    return out
+
+
 def argmax_labels(logits, dtype=torch.int64):
     """torch.argmax(torch.softmax(logits, dim=1), dim=1) in one launch (val.py:275); int64 (default) or uint8 labels."""
     L.require_cuda(logits, "logits")

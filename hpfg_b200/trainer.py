@@ -14,13 +14,15 @@ SGD-momentum or Adam / AdamW (+EMA) pass over the flat parameter buffers.  Nothi
 a device scalar.  Host-side schedules (Medical_LR, consistency ramp-up, EMA alpha) are python floats exactly as
 in the reference (utils/scheduler/medical_lr.py:13-17, utils/utils.py:67-86)."""
 import contextlib
+import ctypes
 import math
 
 import torch
 
 from . import _lib as L
 from .optim import SGD, Adam
-from .losses import ssl_loss_raw, ict_loss_raw, ict_mix_inputs, s4cv_loss_raw
+from .losses import ssl_loss_raw, ict_loss_raw, ict_mix_inputs, s4cv_loss_raw, cutmix_loss_raw, cutmix_mix_inputs, check_cutmix_batch
+from .unet import FT_CHNS
 from .utils import sigmoid_rampup, linear_rampup
 
 
@@ -146,8 +148,10 @@ class _StepBase:
         fused loss, backward with its side-stream weight gradients, fused SGD(+EMA)).  The scalars that change per
         iteration -- learning rate, EMA alpha, consistency weight, UAMT threshold, dropout Philox offsets -- live in a
         small device block that is refreshed before every replay (the `_dv` entry points read them at run time).
-        data_parallel=True also captures the bucketed NCCL all-reduces of a multi-process run; by default a data-parallel
-        step stays eager, and so does the exact-global mode.  S4CVStep and HPFGStep always launch eagerly."""
+        data_parallel=True also captures the bucketed NCCL all-reduces of a multi-process run (HPFGStep: the all-reduces of
+        its flat and neck gradients); by default a data-parallel step stays eager, and so does the exact-global mode.
+        HPFGStep captures once every optimiser state, flat and neck, has taken its first update (see its _use_graph).
+        S4CVStep always launches eagerly."""
         self._graph_enabled = bool(enabled)
         self._graph_dp = bool(data_parallel)      # also capture the NCCL bucket all-reduces (torch >= 2.x captures NCCL work)
         if not enabled:
@@ -206,6 +210,7 @@ class _StepBase:
             m.ensure_flat(quick=True)
         ptrs = tuple((m.flat_params.data_ptr(), m.bn_running.data_ptr(), m.bn_counters.data_ptr(), id(m._plans)) for m in models)
         ptrs += tuple(t.data_ptr() for _, g, s in self._trained for t in (g,) + s.bufs if t is not None)
+        ptrs += self._graph_ptrs()
         # (the dropout seed is a by-value launch argument: a re-seeded generator needs a new capture)
         ptrs += (torch.cuda.default_generators[dev.index if dev.index is not None else torch.cuda.current_device()].initial_seed(),)
         sig = tuple((tuple(t.shape), t.dtype) for t in inputs) + (len(dyn_f), len(fwd_models), ptrs)
@@ -255,6 +260,11 @@ class _StepBase:
         return self._gout
 
     _RING = 8
+
+    def _graph_ptrs(self):
+        """Further raw pointers a captured step bakes in (part of the graph signature); none beyond the networks' and the
+        flat optimiser buffers for the drivers without tensors outside the flat buffers."""
+        return ()
 
     def _body_on_device_block(self, body, fwd_models):
         """Enqueue body with every per-iteration scalar read from the device block; _forward takes the Philox slots of
@@ -346,9 +356,10 @@ class _StepBase:
     # (UAMT: one student forward next to five teacher forwards; S4CVNet) the longer stream would finish on half a machine.
     SHARED_FORWARD_CTAS = 74
     share_forward = True
+    sync_bn_exact_global = True     # exact-global mode: the plans' BatchNorm statistics are all-reduced (SyncBN)
 
     def _set_forward_share(self, plan, shared):
-        if self.exact_global and not getattr(plan, "sync_bn", False):
+        if self.exact_global and self.sync_bn_exact_global and not getattr(plan, "sync_bn", False):
             L.check(L.lib().hpfg_unet_plan_set_sync_bn(plan.handle, 1), "hpfg_unet_plan_set_sync_bn")
             plan.sync_bn = True
         want = self.SHARED_FORWARD_CTAS if shared else 0
@@ -362,13 +373,13 @@ class _StepBase:
     def _dyn_scalars(self, ema_decay=None, *extra):
         """The device block: [lr, ema_alpha, 1 - ema_alpha (fp32 subtraction, as the by-value entry point), consistency
         weight, *extra (UAMT: its threshold)], then the optimiser's group of each trained network in the order of ``_trained``
-        (SGD: none; Adam / AdamW: [step_size, bc2_sqrt, decay_factor, ema_alpha, 1 - ema_alpha]), whose offset its state
-        records."""
+        and of each state of a tensor outside the flat buffers (HPFGStep's neck tensors; SGD: none; Adam / AdamW: [step_size,
+        bc2_sqrt, decay_factor, ema_alpha, 1 - ema_alpha]), whose offset its state records."""
         alpha = min(1 - 1 / (self.cur_itrs + 1), ema_decay) if ema_decay is not None else 0.0
         one_minus = float(1.0 - torch.tensor(alpha, dtype=torch.float32))
         lr = self._lr()
         out = [lr, alpha, one_minus, self._consistency_weight(), *extra]
-        for _, _, state in self._trained:
+        for state in [s for _, _, s in self._trained] + list(self._neck_states.values()):
             state.dv_offset = len(out)
             out += self._opt.device_group(state.step, lr, alpha, one_minus)
         return out
@@ -699,102 +710,208 @@ class S4CVStep(_StepBase):
 
 
 class HPFGStep(_StepBase):
-    """The HPFG iteration of main.py:128-207 on three ``UNet_Plus`` networks (model1 sees the CutMix batch, model2 and the EMA
-    teacher the plain batch).  U-Net bodies, projection necks and ``Dense_Loss`` run on the library's kernels behind autograd
-    Functions; the pixel losses do not go through autograd at all: model2's supervised + Mean-Teacher terms are the MT mode of the
-    fused loss kernels, model1's supervised term the SUP mode, its Dice against the CutMix-pasted pseudo-labels ``hpfg_dice_loss``,
-    and their logits gradients are fed to ONE ``torch.autograd.backward`` together with the contrastive term.  The optimiser side is
-    fused: flat SGD over the 82 U-Net tensors of each student, one launch per neck tensor, the backbone EMA model2 <- model1
-    (main.py:68-76) and the teacher EMA (utils/utils.py:82-86) as flat passes.
+    """The HPFG iteration of main.py:128-207 on three ``UNet_Plus`` networks: model1 sees the CutMix batch, model2 and the EMA
+    teacher the plain batch.  One step body (``_body``) runs eagerly or is captured and replayed as one CUDA graph
+    (``enable_graph``): the CutMix input mix (``hpfg_cutmix_mix``); the three U-Net forwards; the projection necks of model2
+    and of the teacher (model1's neck outputs are dropped by main.py:148, so they do not run); model2's supervised + Mean-Teacher
+    terms as the MT mode of the fused loss kernels, model1's supervised + pseudo-label Dice as the CUTMIX mode, the four
+    ``Dense_Loss`` terms with their gradients scaled by 0.5*w; the neck backwards (the head neck's input gradient joins model2's
+    logits gradient, the high neck's the bottleneck); both U-Net backwards into flat gradient buffers; the optimiser over both
+    flat buffers and each of model2's 16 neck tensors; the backbone EMA model2 <- model1 (main.py:68-76) and the teacher EMA
+    (utils/utils.py:82-86) over the flat buffer and the neck tensors.  No autograd runs.
 
-    step(label_img, target_label, label_img1, target_label1, img_unlabel, cutmix_mask): the tensors main.py:128-150 builds
-    (label_img1 / target_label1: the second labeled draw, repeated to the unlabeled batch size here as at :139-140;
-    cutmix_mask [n_u,1,H,W] from BoxMaskGenerator)."""
+    After a step, ``p.grad`` of every parameter of model1 and model2 holds that step's gradient as a view into the driver's
+    buffers (model1's neck tensors: None).  The exact-global data-parallel mode is not implemented by this step: with
+    ``exact_global=True`` gradients are summed over the ranks and nothing else changes.
+
+    step(label_img, target_label, label_img1, target_label1, img_unlabel, cutmix_mask): the tensors main.py:128-143 draws
+    (label_img1 / target_label1: the second labeled draw, n_l1 images, never repeated: unlabeled image u reads u % n_l1 as
+    main.py:139-140's repeat does; cutmix_mask [n_u,1,H,W] from BoxMaskGenerator)."""
+    share_forward = False           # (the step runs on one stream: each forward has the whole machine)
+    sync_bn_exact_global = False
 
     def __init__(self, model1, model2, ema_model, *, ema_decay=0.99, mt_start=1000, temperature=0.7, **kw):
         super().__init__(**kw)
-        from .losses import Dense_Loss
         self.m1, self.m2, self.ema_model, self.ema_decay, self.mt_start = model1, model2, ema_model, ema_decay, mt_start
-        # the gradients come from autograd (model.last_flat_grad): optimiser state only
-        (_, self.b1), (_, self.b2) = self._setup([model1, model2], [model1, model2, ema_model], grads=False)
+        (self.g1, self.b1), (self.g2, self.b2) = self._setup([model1, model2], [model1, model2, ema_model])
         for p in ema_model.parameters():
             p.requires_grad = False
         self.temperature = temperature
-        self._dense = None
-        self._DenseLoss = Dense_Loss
+        self._step_lr = None
+        self._stepped = False           # this driver has run a step (plans, neck states and buffers exist)
 
     def _consistency_weight(self):
         return self.consistency * linear_rampup(self.cur_itrs // 150, self.consistency_rampup)
 
-    def _sgd_model(self, trained, lr):
-        """torch.optim.SGD (or Adam / AdamW) semantics over all parameters of a UNet_Plus: the flat U-Net buffer in one pass +
-        one launch per neck tensor that has a gradient (model1's necks never have one: main.py:148 drops their outputs)."""
-        model, _, state = trained
-        st = L.stream_ptr(model.flat_params.device)
-        self._opt.launch(model.flat_params, model.last_flat_grad, state, None, lr, 0.0, None, st)
-        for p in self._neck_params(model):
-            if p.grad is None:
-                continue
-            # torch.optim: a tensor's state is created the first time it has a gradient, and each tensor counts its own steps
-            neck = self._neck_states.get(id(p))
-            if neck is None:
-                neck = self._neck_states[id(p)] = self._opt.new_state(p.data)
-            neck.step += 1
-            self._opt.launch(p.data, p.grad.contiguous(), neck, None, lr, 0.0, None, st)
+    def _mt_weight(self):
+        """Weight of model2's Mean-Teacher term: w from mt_start on, 0 before (main.py:137-142)."""
+        return self._consistency_weight() if self.cur_itrs >= self.mt_start else 0.0
+
+    def _lr(self):
+        return medical_lr(self.cur_itrs, self.base_lr, self.total_itrs) if self._step_lr is None else self._step_lr
+
+    def _use_graph(self):
+        """Replay once this driver has run a step and every optimiser state, flat and neck, has taken its first update: the SGD
+        launch bakes in whether it initialises the momentum buffer, and the neck states are created at their first gradient."""
+        states = [s for _, _, s in self._trained] + [self._neck_states.get(id(p)) for p in self._neck_params(self.m2)]
+        return (self._graph_enabled and self._stepped and (self.world == 1 or self._graph_dp) and not self.exact_global
+                and all(s is not None and s.step >= 2 for s in states))
+
+    def _graph_ptrs(self):
+        necks2 = self._neck_params(self.m2)
+        ptrs = tuple(p.data_ptr() for p in necks2 + self._neck_params(self.ema_model))
+        ptrs += tuple(b.data_ptr() for p in necks2 for b in self._neck_states[id(p)].bufs)
+        return ptrs + tuple(t.data_ptr() for t in self._bufs.values())      # neck gradients, neck / loss scratch, batches
 
     def step(self, label_img, target_label, label_img1, target_label1, img_unlabel, cutmix_mask, lr=None):
         """lr: override of the Medical_LR value of this iteration (resuming with a fresh scheduler; parity harness).
-        cutmix_mask: the 0/1 box masks of BoxMaskGenerator (main.py:141-143)."""
-        from .utils import update_ema_variables, ema_update_flat
-        from .losses import ssl_loss_raw, dice_loss_raw, argmax_labels
+        cutmix_mask: the box masks of BoxMaskGenerator (main.py:141-143).  Returns the loss (device scalar)."""
+        check_cutmix_batch(img_unlabel.shape[0], label_img1.shape[0])
         self._next_iteration()
-        m1, m2, ema = self.m1, self.m2, self.ema_model
-        label_bs, unlabel_bs = label_img.shape[0], img_unlabel.shape[0]
-        rep = int(unlabel_bs // label_bs)
-        label_img1 = label_img1.repeat(rep, 1, 1, 1).float()
-        target_label1 = target_label1.repeat(rep, 1, 1).long()
-        cutmix_mask = cutmix_mask.float()
-        batch_un_mix = label_img1 * (1.0 - cutmix_mask) + img_unlabel * cutmix_mask          # main.py:145
-        batch_mix = torch.cat([label_img, batch_un_mix], dim=0).float()
-        volume_batch = torch.cat([label_img, img_unlabel], dim=0).float()
-        if self._dense is None or self._dense.batch_size != label_bs + unlabel_bs:
-            self._dense = self._DenseLoss(label_bs + unlabel_bs, volume_batch.device, self.temperature)
-        for m in (m1, m2):
-            for p in m.parameters():
-                p.grad = None
-        outputs1, _, _ = m1(batch_mix)
-        outputs2, h1, h2 = m2(volume_batch)
-        with torch.no_grad():
-            ema_output, ema_h1, ema_h2 = ema(volume_batch)
-        tl = target_label.long()
+        necks2 = self._neck_params(self.m2)
+        for p in necks2:        # torch.optim: a tensor's state appears at its first gradient, and it counts its own steps
+            s = self._neck_states.get(id(p))
+            if s is None:
+                s = self._neck_states[id(p)] = self._opt.new_state(p.data)
+                self.__dict__.setdefault("_neck_owners", {})[id(p)] = p     # (keeps the id of a replaced tensor from being reused)
+            s.step += 1
+        self._step_lr = lr
         w = self._consistency_weight()
-        # model2 (main.py:157-158,183,186): supervised + w * mean((softmax2_u - softmax_ema_u)^2) = the Mean-Teacher mode of the fused
-        # loss kernels (value, loss_sup, consistency value and d/d outputs2 in one launch); the MSE term is 0 before mt_start
-        r2 = ssl_loss_raw(L.LOSS_MT, outputs2.detach(), ema_output[label_bs:], tl, label_bs,
-                          cons_weight=w if self.cur_itrs >= self.mt_start else 0.0)
-        # model1 (main.py:154-155,170-175,185): supervised (SUP mode: zero gradient on the unlabeled images) + 7w * Dice of
-        # softmax1_u against the teacher's argmax pasted into the second labeled draw's labels by the CutMix mask
-        r1 = ssl_loss_raw(L.LOSS_SUP, outputs1.detach(), None, tl, label_bs)
-        pseudo = torch.where(cutmix_mask.squeeze(1) > 0.5, argmax_labels(ema_output[label_bs:]), target_label1)      # main.py:171-172
-        ps, d_ps = dice_loss_raw(outputs1.detach()[label_bs:], pseudo, softmax=True)
-        dlogits1 = r1["dstudent"]
-        dlogits1[label_bs:].add_(d_ps, alpha=7.0 * w)
-        loss_contrast = self._dense(h1, ema_h1) + self._dense(h2, ema_h2)                     # main.py:166 (autograd: the necks)
-        loss_sup = r1["scalars"][1] + r2["scalars"][1]
-        loss = r1["scalars"][0] + 7 * w * ps[0] + r2["scalars"][0] + w * loss_contrast
-        # one backward pass: the loss kernels' gradients enter at the logits, the contrastive term through the necks of model2
-        torch.autograd.backward([outputs1, outputs2, w * loss_contrast], [dlogits1, r2["dstudent"], None])
-        if self.world > 1:      # data parallel (main.py itself is single-process): gradients summed here, scaled by 1/world in the SGD pass
+        ins = [label_img, target_label, label_img1, target_label1, img_unlabel, cutmix_mask]
+        if self._use_graph():
+            out = self._graph_replay(ins, self._dyn_scalars(self.ema_decay, self._mt_weight(), 7.0 * w, 0.5 * w),
+                                     [self.m1, self.m2, self.ema_model], self._body)
+        else:
+            out = self._body(ins, None)
+        self._stepped = True
+        self._publish_grads(necks2)
+        self.last = dict(out, lr=self._lr(), w=w)
+        return out["loss"]
+
+    def _publish_grads(self, necks2):
+        """p.grad of model1 / model2: views into the flat gradient buffers and model2's neck gradient buffers."""
+        views = self.__dict__.setdefault("_grad_views", {})
+        for model, g, _ in self._trained:
+            for p, (o, n, shape) in zip(model._flat_params_list, model._layout):
+                v = views.get(id(p), (None, None))[1]
+                if v is None:
+                    v = g[o:o + n].view(shape)
+                    views[id(p)] = (p, v)
+                if p.grad is not v:
+                    p.grad = v
+        for p in self._neck_params(self.m1):
+            p.grad = None
+        for j, p in enumerate(necks2):
+            g = self._bufs["neck_grad%d" % j]
+            if p.grad is not g:
+                p.grad = g
+
+    def _neck_forward(self, neck, x, key):
+        """projection_conv.forward of ``neck`` on x into step-persistent buffers: (pooled, hidden, out_global, out_dense)."""
+        n, c, h, w = x.shape
+        s, hid, dim = neck.is_s, neck.mlp[0].out_features, neck.mlp[2].out_features
+        rows, dev = n * (1 + s * s), x.device
+        bufs = (self._persistent(key + ".pooled", (rows, c), dev), self._persistent(key + ".hidden", (rows, hid), dev),
+                self._persistent(key + ".global", (n, dim), dev), self._persistent(key + ".dense", (n, dim, s * s), dev))
+        params = (ctypes.c_void_p * 8)(*[p.data_ptr() for p in neck._param_list()])
+        L.check(L.lib().hpfg_neck_forward(L.ptr(x), n, c, h, w, s, hid, dim, params, *[L.ptr(b) for b in bufs],
+                                          L.stream_ptr(dev)), "hpfg_neck_forward")
+        return bufs
+
+    def _neck_backward(self, neck, x, key, fwd, d_global, d_dense, grads, dx):
+        n, c, h, w = x.shape
+        s, hid, dim = neck.is_s, neck.mlp[0].out_features, neck.mlp[2].out_features
+        scratch = self._persistent(key + ".scratch", (n * s * s * dim + n * (1 + s * s) * (hid + c),), x.device)
+        params = (ctypes.c_void_p * 8)(*[p.data_ptr() for p in neck._param_list()])
+        L.check(L.lib().hpfg_neck_backward(L.ptr(d_global), L.ptr(d_dense), n, c, h, w, s, hid, dim, params, L.ptr(fwd[0]),
+                                           L.ptr(fwd[1]), (ctypes.c_void_p * 8)(*[g.data_ptr() for g in grads]), L.ptr(dx),
+                                           L.ptr(scratch), L.stream_ptr(x.device)), "hpfg_neck_backward")
+
+    def _ema(self, ema, param, alpha, dv):
+        """ema <- alpha*ema + (1 - alpha)*param; captures read {alpha, 1 - alpha} from the device block."""
+        if dv is None:
+            L.check(L.lib().hpfg_ema_update(L.ptr(ema), L.ptr(param), ema.numel(), float(alpha), L.stream_ptr(ema.device)),
+                    "hpfg_ema_update")
+        else:
+            L.check(L.lib().hpfg_ema_update_dv(L.ptr(ema), L.ptr(param), ema.numel(), L.ptr(dv[0][1:3]),
+                                               L.stream_ptr(ema.device)), "hpfg_ema_update_dv")
+
+    def _body(self, ins, dv):
+        label_img, target_label, label_img1, target_label1, img_unlabel, cutmix_mask = ins
+        m1, m2, ema = self.m1, self.m2, self.ema_model
+        n_l, n_u = label_img.shape[0], img_unlabel.shape[0]
+        n, dev = n_l + n_u, label_img.device
+        img_shape, hh, ww = tuple(label_img.shape[1:]), label_img.shape[2], label_img.shape[3]
+        lib = L.lib()
+        # main.py:137-150: model1 sees cat(label_img, CutMix(label_img1, img_unlabel)), model2 and the teacher cat(label_img, img_unlabel)
+        batch_mix = self._persistent("batch_mix", (n,) + img_shape, dev)
+        volume = self._persistent("volume", (n,) + img_shape, dev)
+        batch_mix[:n_l].copy_(label_img)
+        cutmix_mix_inputs(label_img1, img_unlabel, cutmix_mask, out=batch_mix[n_l:])
+        volume[:n_l].copy_(label_img)
+        volume[n_l:].copy_(img_unlabel)
+        shape = (n, self.num_classes, hh, ww)
+        p1, o1 = self._forward(m1, batch_mix, True, self._persistent("o1", shape, dev), dv)
+        p2, o2 = self._forward(m2, volume, True, self._persistent("o2", shape, dev), dv)
+        pt, t_out = self._forward(ema, volume, False, self._persistent("t_out", shape, dev), dv)
+        feat_shape = (n, FT_CHNS[-1], hh // 16, ww // 16)
+        feats = []
+        for plan, key in ((p2, "feat2"), (pt, "feat_t")):     # feature[-1] (model/unet.py:199-201)
+            f = self._persistent(key, feat_shape, dev)
+            L.check(lib.hpfg_unet_bottleneck(plan.handle, L.ptr(f), L.stream_ptr(dev)), "hpfg_unet_bottleneck")
+            feats.append(f)
+        necks = [(m2.dense_projection_high, ema.dense_projection_high, feats[0], feats[1], "high"),
+                 (m2.dense_projection_head, ema.dense_projection_head, o2, t_out, "head")]
+        fwd2 = [self._neck_forward(nk, x, key + "2") for nk, _, x, _, key in necks]
+        fwd_t = [self._neck_forward(nk, x, key + "_t") for _, nk, _, x, key in necks]
+        # main.py:144,166: w * (Dense_Loss(h1, ema_h1) + Dense_Loss(h2, ema_h2)), Dense_Loss = 0.5 * (global term + dense term):
+        # four contrastive calls, each writing 0.5*w * its gradient wrt model2's neck output
+        w = self._consistency_weight()
+        contrast = self._persistent("contrast", (4,), dev)
+        ws = self._persistent("contrast_ws", (lib.hpfg_dense_contrastive_workspace_floats(n, fwd2[0][3].shape[1],
+                                                                                          fwd2[0][3].shape[2]),), dev)
+        d_out = []
+        for k, (a, b) in enumerate((a, b) for f2, ft in zip(fwd2, fwd_t) for a, b in ((f2[2], ft[2]), (f2[3], ft[3]))):
+            d = self._persistent("d_contrast%d" % k, tuple(a.shape), dev)
+            L.check(lib.hpfg_dense_contrastive_scaled(L.ptr(a), L.ptr(b), n, a.shape[1], a[0, 0].numel(), float(self.temperature),
+                                                      float(0.5 * w), L.ptr(self._dv_scalar(dv, 6)), L.ptr(contrast[k:k + 1]),
+                                                      L.ptr(d), L.ptr(ws), L.stream_ptr(dev)), "hpfg_dense_contrastive_scaled")
+            d_out.append(d)
+        # model2 (main.py:127,142,144): supervised + Mean-Teacher MSE from mt_start on; model1 (:125,131-134,143): supervised + 7w *
+        # Dice against the teacher's argmax pasted into the second labeled draw's labels
+        r2 = ssl_loss_raw(L.LOSS_MT, o2, t_out[n_l:], target_label, n_l, cons_weight=self._mt_weight(),
+                          cons_weight_dev=self._dv_scalar(dv, 4))
+        r1 = cutmix_loss_raw(o1, t_out[n_l:], target_label, target_label1, cutmix_mask, n_l, pseudo_weight=7.0 * w,
+                             pseudo_weight_dev=self._dv_scalar(dv, 5))
+        # neck backwards: the high neck's input gradient enters model2 at the bottleneck, the head neck's at the logits
+        necks2 = self._neck_params(m2)
+        ngrads = [self._persistent("neck_grad%d" % j, tuple(p.shape), dev) for j, p in enumerate(necks2)]
+        dfeat = self._persistent("dfeat", feat_shape, dev)
+        dx_head = self._persistent("dx_head", shape, dev)
+        for i, ((nk, _, x, _, key), dx) in enumerate(zip(necks, (dfeat, dx_head))):
+            self._neck_backward(nk, x, key + "2", fwd2[i], d_out[2 * i], d_out[2 * i + 1], ngrads[8 * i:8 * i + 8], dx)
+        dl2 = r2["dstudent"]
+        dl2.add_(dx_head)
+        L.check(lib.hpfg_unet_backward(p1.handle, L.ptr(m1.flat_params), L.ptr(r1["dstudent"]), L.ptr(self.g1), 0,
+                                       L.stream_ptr(dev)), "hpfg_unet_backward")
+        L.check(lib.hpfg_unet_backward_ex(p2.handle, L.ptr(m2.flat_params), L.ptr(dl2), L.ptr(dfeat), L.ptr(self.g2), 0,
+                                          L.stream_ptr(dev)), "hpfg_unet_backward_ex")
+        if self.world > 1:      # data parallel (main.py itself is single-process): gradients summed here, scaled in the optimiser
             import torch.distributed as dist
-            for m in (m1, m2):
-                dist.all_reduce(m.last_flat_grad, group=self.pg)
-                allreduce_tensor_list([p.grad for p in self._neck_params(m)], group=self.pg)
-        lr = medical_lr(self.cur_itrs, self.base_lr, self.total_itrs) if lr is None else lr
-        self._sgd_model(self._trained[0], lr)
-        self._sgd_model(self._trained[1], lr)
+            dist.all_reduce(self.g1, group=self.pg)
+            dist.all_reduce(self.g2, group=self.pg)
+            allreduce_tensor_list(ngrads, group=self.pg)
+        self._opt_step(self._trained[0], dv)
+        self._opt_step(self._trained[1], dv)
+        block = None if dv is None else dv[0]
+        for p, g in zip(necks2, ngrads):
+            self._opt.launch(p.data, g, self._neck_states[id(p)], None, self._lr(), 0.0, block, L.stream_ptr(dev))
         alpha = min(1 - 1 / (self.cur_itrs + 1), self.ema_decay)
-        ema_update_flat(m2.ensure_flat(), m1.ensure_flat(), alpha)          # update_ema_variables_backbone: encoder + decoder = the flat buffer
-        update_ema_variables(m2, ema, self.ema_decay, self.cur_itrs)
-        self.last = dict(loss=loss.detach(), loss_sup=loss_sup, contrast=loss_contrast.detach(), pseudo=ps[0], cons2=r2["scalars"][2],
-                         lr=lr, w=w, outputs1=outputs1.detach(), outputs2=outputs2.detach(), ema_output=ema_output)
-        return loss.detach()
+        self._ema(m2.flat_params, m1.flat_params, alpha, dv)        # update_ema_variables_backbone: encoder + decoder = the flat buffer
+        self._ema(ema.flat_params, m2.flat_params, alpha, dv)
+        for e, p in zip(self._neck_params(ema), necks2):
+            self._ema(e.data, p.data, alpha, dv)
+        lc = 0.5 * (contrast[0] + contrast[1]) + 0.5 * (contrast[2] + contrast[3])
+        loss = r1["scalars"][0] + r2["scalars"][0] + (w if dv is None else dv[0][3]) * lc
+        return dict(loss=loss, loss_sup=r1["scalars"][1] + r2["scalars"][1], contrast=lc, pseudo=r1["scalars"][2],
+                    cons2=r2["scalars"][2], outputs1=o1, outputs2=o2, ema_output=t_out)

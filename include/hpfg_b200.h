@@ -41,6 +41,7 @@ extern "C" {
 #define HPFG_LOSS_UAMT 3 /* + w * uncertainty-masked softmax-MSE              (UAMT)                   */
 #define HPFG_LOSS_ICT 4  /* + w * MSE against a per-sample mix of two teacher softmaxes (hpfg_ict_loss)  */
 #define HPFG_LOSS_S4CV 5 /* two nets: Dice-only cross pseudo supervision + teacher MSE (hpfg_s4cv_loss)  */
+#define HPFG_LOSS_CUTMIX 6 /* + w * Dice against CutMix-pasted teacher pseudo-labels (HPFG model1, hpfg_cutmix_loss) */
 
 #define HPFG_NUM_BN 18
 #define HPFG_NUM_DROPOUT 5
@@ -241,6 +242,26 @@ int hpfg_s4cv_loss(const float *logits1, const float *logits2, const float *teac
                    float *dlogits1, float *dlogits2, float *scalars_out, int64_t *pseudo1, int64_t *pseudo2,
                    void *workspace, void *stream);
 
+/* ---- HPFG model1 (main.py:125-134,143; replaces Med_Sup_Loss on outputs1[:n_l] plus the pseudo_supervision1 DiceLoss):
+ *   loss = ce_coef*CE(s[:n_l], labels) + dice_coef*Dice(softmax(s[:n_l]), labels) + pseudo_weight*Dice(softmax(s[n_l:]), pseudo)
+ *   pseudo[u,p] = labels1[u % n_l1, p]*(1 - m[u,p]) + argmax_c softmax(teacher_u[u])[c,p]*m[u,p]   in fp32 as torch rounds it;
+ * a pixel is class c for the Dice term iff that float equals c (the reference's one-hot; for a 0/1 mask: a torch.where).  The
+ * argmax is the first maximum of the accurate softmax, the labels of hpfg_argmax_labels.  student [n_l+n_u,C,H,W], teacher_u
+ * [n_u,C,H,W] fp32; labels [n_l,H,W], labels1 [n_l1,H,W] int64 (never repeated: image u reads u % n_l1, main.py:139-140);
+ * cutmix_mask [n_u,1,H,W] fp32.  n_u must be a multiple of n_l1 (HPFG_ERR_INVALID otherwise).  pseudo_weight_dev (optional
+ * device scalar) overrides pseudo_weight (graph replay).  dstudent: the gradient for all n_l+n_u images.  scalars_out: {loss,
+ * loss_sup, pseudo Dice (unweighted), ce, dice, n_valid, 0, 0}.  pseudo_out (optional): int64 [n_u,H,W], the class each pixel
+ * took in the Dice term (255: none).  Workspace: hpfg_ssl_loss_workspace_bytes(HPFG_LOSS_CUTMIX, n_l, n_u, ...). */
+int hpfg_cutmix_loss(const float *student, const float *teacher_u, const int64_t *labels, const int64_t *labels1,
+                     const float *cutmix_mask, int n_l, int n_u, int n_l1, int num_classes, int height, int width,
+                     float pseudo_weight, const float *pseudo_weight_dev, const float *class_weights, float ce_coef,
+                     float dice_coef, float *dstudent, float *scalars_out, int64_t *pseudo_out, void *workspace, void *stream);
+/* The CutMix input mix (main.py:139,145): out[u] = a[u % n_a]*(1 - m[u]) + b[u]*m[u] over n images of `channels` planes of
+ * H*W floats, the [n,1,H,W] mask broadcast over the channels; separate fp32 roundings (bit-identical to torch's expression on
+ * the repeated draw).  n must be a multiple of n_a. */
+int hpfg_cutmix_mix(const float *a, const float *b, const float *cutmix_mask, int n, int n_a, int channels, int height,
+                    int width, float *out, void *stream);
+
 /* ---- inference side (SURVEY 8f.3; val.py:268-281 test_single_volume): argmax(softmax(logits), dim=1), first maximum
  * wins, for a whole batch of eval-mode logits in one launch.  Either output may be NULL. */
 int hpfg_argmax_labels(const float *logits, int n, int num_classes, int height, int width, int64_t *labels_i64,
@@ -282,10 +303,21 @@ int hpfg_neck_backward(const float *d_global, const float *d_dense, int n, int c
 int64_t hpfg_dense_contrastive_workspace_floats(int batch, int dim, int positions);
 int hpfg_dense_contrastive(const float *out1, const float *out2, int batch, int dim, int positions, float temperature,
                            float *loss, float *d_out1, float *workspace, void *stream);
+/* The same with d_out1 = scale * d loss / d out1 (a separate fp32 rounding: bit-identical to scaling the unscaled gradient);
+ * the loss stays unscaled.  scale_dev (optional device scalar) overrides scale (graph replay).  HPFGStep passes the 0.5*w
+ * that main.py:144,166 (w * (0.5*(contrast_global + contrast_dense)) per neck) puts in front of each term, which autograd
+ * used to apply. */
+int hpfg_dense_contrastive_scaled(const float *out1, const float *out2, int batch, int dim, int positions, float temperature,
+                                  float scale, const float *scale_dev, float *loss, float *d_out1, float *workspace,
+                                  void *stream);
 
 /* ---- optimiser-side passes over the flat buffers --------------------------------------------------- */
 /* update_ema_variables (utils/utils.py:82-86): ema <- alpha*ema + (1-alpha)*param, alpha already clamped. */
 int hpfg_ema_update(float *ema, const float *param, int64_t n, float alpha, void *stream);
+/* The same with alpha_dev: device float[2] = {alpha, 1 - alpha} (graph replay; the same arithmetic as hpfg_ema_update, whose
+ * 1 - alpha is an fp32 subtraction).  HPFGStep: the backbone EMA model2 <- model1 (main.py:68-76) and the teacher EMA over the
+ * flat buffer and each neck tensor (utils/utils.py:82-86). */
+int hpfg_ema_update_dv(float *ema, const float *param, int64_t n, const float *alpha_dev, void *stream);
 /* torch.optim.SGD step (momentum, weight decay, no nesterov/dampening): first_step != 0 initialises the
  * momentum buffer with the decayed gradient.  grad_scale multiplies the gradient first (1/world for DP). */
 int hpfg_sgd_momentum(float *param, const float *grad, float *momentum_buf, int64_t n, float lr, float momentum,
