@@ -91,11 +91,15 @@ class Med_Sup_Loss(nn.Module):
 
 def dice_loss_raw(inputs, target, softmax=False, weight=None, want_grad=True):
     """Thin wrapper of hpfg_dice_loss: (scalars[1+C] = {loss, per-class dice}, d loss / d inputs or None).  inputs [n,C,H,W]
-    probabilities (or logits with softmax=True), target any [n,(1,)H,W] tensor of class ids."""
+    probabilities (or logits with softmax=True), target any [n,(1,)H,W] tensor of class ids.  A float target follows the
+    reference's one-hot (``target == c``): a value that is not an integer in [0, 255] is in no class (255), not truncated."""
     L.require_cuda(inputs, "DiceLoss inputs")
     x = inputs.contiguous().float()
     n, c, h, w = x.shape
-    t = target.reshape(n, h, w).contiguous().to(torch.int64)
+    t = target.reshape(n, h, w)
+    if t.is_floating_point():
+        t = torch.where((t == t.round()) & (t >= 0) & (t <= 255), t, 255)
+    t = t.contiguous().to(torch.int64)
     dx = torch.empty_like(x) if want_grad else None
     scalars = torch.empty(1 + c, device=x.device, dtype=torch.float32)
     ws = torch.empty(2048, dtype=torch.uint8, device=x.device)

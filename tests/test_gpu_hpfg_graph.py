@@ -63,7 +63,7 @@ def _inputs(n_cls, n_l, n_u, n_l1, h, w, seed, fractional):
     return [x.to(DEV) for x in (s, t, y, y1, m)]
 
 
-@pytest.mark.parametrize("n_cls,fractional", [(2, False), (4, False), (4, True)])
+@pytest.mark.parametrize("n_cls,fractional", [(c, False) for c in range(2, 9)] + [(3, True), (4, True), (8, True)])
 def test_cutmix_loss_mode_matches_main_py(n_cls, fractional):
     n_l, n_u, n_l1, h, w, pw = 2, 6, 2, 32, 48, 0.35
     s, t, y, y1, m = _inputs(n_cls, n_l, n_u, n_l1, h, w, 40 + n_cls, fractional)

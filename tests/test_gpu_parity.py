@@ -133,7 +133,11 @@ def test_fused_losses_vs_reference_golden(tag):
     l = hb.DiceLoss(C)(probs, y.unsqueeze(1))
     assert abs(l.item() - g["dice"]) / abs(g["dice"]) < 1e-5
     (gr,) = torch.autograd.grad(l, s)                                  # grad through torch's softmax
-    lo = oracle.dice_loss(torch.softmax(g["student"].clone().requires_grad_(True), 1)[:n_l], g["y"].unsqueeze(1), C)
+    s64 = g["student"].double().requires_grad_(True)
+    lo = oracle.dice_loss(torch.softmax(s64, 1)[:n_l], g["y"].unsqueeze(1), C)
+    (go,) = torch.autograd.grad(lo, s64)
+    assert abs(l.item() - lo.item()) / abs(lo.item()) < 1e-5
+    assert rel_l2(gr, go) < 1e-5
     mt = g["mt"]
     l = hb.mean_teacher_loss(s, t[n_l:], y, mt["w"])
     (gr,) = torch.autograd.grad(l, s)
