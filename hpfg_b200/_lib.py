@@ -65,6 +65,9 @@ SIGNATURES = {
                                ctypes.POINTER(c_f), c_f, c_f, c_vp, c_vp, c_vp, c_vp, c_vp, c_vp, c_vp]),
     "hpfg_softmax_mse": (c_int, [c_vp, c_vp, c_vp, c_int, c_int, c_int, c_int, c_int, c_vp, c_vp]),
     "hpfg_argmax_labels": (c_int, [c_vp, c_int, c_int, c_int, c_int, c_vp, c_vp, c_vp]),
+    "hpfg_zoom_nearest": (c_int, [c_vp, c_i64, c_int, c_int, c_int, c_int, c_int, c_vp, c_vp]),
+    "hpfg_volume_metrics_workspace_bytes": (c_i64, [c_int] * 4),
+    "hpfg_volume_metrics": (c_int, [c_vp, c_vp, c_int, c_int, c_int, c_int, c_vp, c_vp, c_vp]),
     "hpfg_dice_loss": (c_int, [c_vp, c_vp, c_int, c_int, c_int, c_int, c_int, ctypes.POINTER(c_f), c_vp, c_vp, c_vp,
                                c_vp]),
     "hpfg_neck_forward": (c_int, [c_vp] + [c_int] * 7 + [ctypes.POINTER(c_vp)] + [c_vp] * 5),

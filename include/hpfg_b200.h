@@ -267,6 +267,23 @@ int hpfg_cutmix_mix(const float *a, const float *b, const float *cutmix_mask, in
 int hpfg_argmax_labels(const float *logits, int n, int num_classes, int height, int width, int64_t *labels_i64,
                        uint8_t *labels_u8, void *stream);
 
+/* ---- validation (val.py:268-281 test_single_volume, val.py:255-265 calculate_metric_percase; csrc/val.cu) -------------
+ * hpfg_zoom_nearest: scipy.ndimage.zoom(plane, (out_h/in_h, out_w/in_w), order=0) for each of n planes of elem_bytes-byte
+ * elements (1, 4 or 8: uint8 / int64 labels, fp32 images), as val.py:272 resamples each slice to the patch size and :277 the
+ * predicted labels back.  scipy's rule per axis: f = (in-1)/(out-1) in fp64, c = k*f; c > in-1 gives 0, else in[floor(c+0.5)].
+ * hpfg_volume_metrics: medpy 0.4.0's dc and hd95 (no voxel spacing) of pred == c vs label == c for every class c = 1..C-1 of one
+ * [depth,height,width] volume of uint8 labels, all classes in one launch per phase and no host synchronisation.  out: device
+ * int64[(C-1)*6], per class {|P|, |G|, |P n G|, n, d2_lo, d2_hi}: n = the number of surface distances (border voxels of both
+ * sets, 6-neighbourhood, border_value 0), d2_lo / d2_hi the exact squared distances at ranks floor((n-1)*0.95) and the next
+ * (numpy.percentile's linear method); 0 for a class absent from either volume.  The caller finishes
+ * dc = 2|P n G| / (|P| + |G|) and the lerp of the square roots.  workspace: hpfg_volume_metrics_workspace_bytes() bytes of
+ * device scratch (-1 and HPFG_ERR_UNSUPPORTED from the call itself: more than 2^31 voxels, or a squared diameter over int32). */
+int hpfg_zoom_nearest(const void *in, int64_t n, int in_h, int in_w, int out_h, int out_w, int elem_bytes, void *out,
+                      void *stream);
+int64_t hpfg_volume_metrics_workspace_bytes(int depth, int height, int width, int num_classes);
+int hpfg_volume_metrics(const uint8_t *pred_u8, const uint8_t *label_u8, int depth, int height, int width, int num_classes,
+                        int64_t *out, void *workspace, void *stream);
+
 /* softmax_mse_loss (utils/loss/diceloss.py:64-81): the UNREDUCED map (softmax(input) - softmax(target))^2 over dim 1
  * (sigmoid != 0: element-wise sigmoids instead), all tensors fp32 NCHW [n,C,H,W].  grad_out == NULL: out = the map;
  * grad_out != NULL: out = d(sum(grad_out * map)) / d input_logits (the target carries no gradient, as in the trainers,
